@@ -1,7 +1,8 @@
 #!/usr/bin/env python
-"""bench.py -- headline benchmark of the B200 MINCO trajectory optimizer (contract: see the task prompt / DESIGN.md §6).
+"""bench.py -- headline benchmark of the B200 MINCO trajectory optimizer (see DESIGN.md §6).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload c4|c2|c5] [--no-extras]
+                    [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P bench.py --gpus N ...
 
 One "step" = one pass of the hot path (warm_start_plan semantics: straight-line expert guess, up to 5 L-BFGS-B
@@ -16,6 +17,8 @@ At N = 1 the line also carries, under "extras", the other configurations measure
 cost+gradient evaluation rate (k_eval, the second half of BASELINE.json's metric) and the latency of ONE plan through the
 drop-in MinJerkPlanner.plan (the reference node's call, NODE:490-525), each with its own roofline / CPU figure.
 Prints ONE JSON line (rank 0).
+--dump-outputs DIR writes the result records of the last timed step as DIR/<field>.npy (see dump_outputs), so that two
+builds can be compared output for output on the same seeded inputs.
 """
 from __future__ import annotations
 
@@ -300,6 +303,30 @@ def timed_steps(torch, dist, run, K, W, flush, distributed, all_bytes):
     return [a.elapsed_time(b) for a, b in evs]
 
 
+DUMP_BUDGET = 64_000_000
+NPY_HEADER = 128
+
+
+def dump_outputs(path, raw, B, M):
+    """Writes what a caller of the timed path receives -- x, ts, coeffs, costs and the int32 fields status, ok, attempt,
+    nit, runs, nfev -- from the packed record buffer(s) `raw` (one block of B problems per rank, global order) as
+    path/<field>.npy in float64 (exact for the int32 fields). Above DUMP_BUDGET bytes in all, a fixed seeded sample of
+    problems is written instead, with its problem indices as path/problem_index.npy."""
+    from neo_planner_b200 import sharding
+    f = sharding.split_packed_records(raw.reshape(-1, sharding.packed_record_bytes(B, M)), B, M)
+    f = {k: v.reshape((-1,) + v.shape[2:]) for k, v in f.items()}
+    total = f['x'].shape[0]
+    per_problem = 8 * sum(v[0].size for v in f.values())
+    keep = np.arange(total)
+    if total * per_problem + NPY_HEADER * len(f) > DUMP_BUDGET:
+        rows = (DUMP_BUDGET - NPY_HEADER * (len(f) + 1)) // (per_problem + 8)
+        keep = np.sort(np.random.default_rng(0).choice(total, rows, replace=False))
+        f['problem_index'] = keep
+    os.makedirs(path, exist_ok=True)
+    for k, v in f.items():
+        np.save(os.path.join(path, k + '.npy'), np.asarray(v if k == 'problem_index' else v[keep], dtype=np.float64))
+
+
 def roofline_of(acc, M, step_ms, fp64_peak, hbm_peak, peaks_found, hbm_bytes, name):
     ach = acc['flops'] / (step_ms * 1e-3) / 1e12
     return {'bound': 'fp64', 'kernel': 'k_optimize', 'achieved': ach, 'peak': fp64_peak, 'unit': 'TFLOP/s', 'frac': ach / fp64_peak,
@@ -427,7 +454,12 @@ def main():
     ap.add_argument('--workload', default='c4', choices=['c2', 'c4', 'c5'])
     ap.add_argument('--no-cpu-baseline', action='store_true')
     ap.add_argument('--no-extras', action='store_true')
+    ap.add_argument('--dump-outputs', metavar='DIR', help='write the result records of the last timed step as DIR/<field>.npy')
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error('--steps must be at least 1')
+    if args.dump_outputs and args.impl != 'ours':
+        ap.error('--dump-outputs needs --impl ours')
     rank = int(os.environ.get('RANK', '0'))
     world_size = int(os.environ.get('WORLD_SIZE', '1'))
     local_rank = int(os.environ.get('LOCAL_RANK', '0'))
@@ -497,6 +529,8 @@ def main():
     t_wall0 = time.perf_counter()
     step_ms_list = timed_steps(torch, dist, run, K, W, flush, distributed, all_bytes)
     t_wall = time.perf_counter() - t_wall0
+    # the clock-sampling launches below rewrite run.out: keep the records of the last timed step
+    last_step = (all_bytes if distributed else run.out).clone() if args.dump_outputs and rank == 0 else None
     launches = (run.h.launch_count() - launches0) * K // (K + W)        # kernels of this library inside the timed region
     # keep the GPU under the same load a little longer if the timed region was too short to sample clocks.
     # Kernel launches only: the number of extra iterations differs per rank, so no collective may run here.
@@ -582,6 +616,8 @@ def main():
             line['cpu_baseline'] = cpu_base
         if extras is not None:
             line['extras'] = extras
+        if last_step is not None:
+            dump_outputs(args.dump_outputs, last_step.cpu().numpy(), B, wl['M'])
         print(json.dumps(line))
     if distributed:
         dist.barrier()

@@ -10,6 +10,7 @@ import subprocess
 import numpy as np
 import pytest
 
+from neo_planner_b200.build import nvcc_path
 from neo_planner_b200.worlds import make_world
 from oracle import minco_ref
 
@@ -22,9 +23,10 @@ SO = os.path.join(ROOT, 'devtools', '_astar_host.so')
 def sim():
     deps = [SRC, os.path.join(ROOT, 'neo_planner_b200', 'csrc', 'astar_warp.cuh')]
     if not os.path.exists(SO) or any(os.path.getmtime(d) > os.path.getmtime(SO) for d in deps):
-        if shutil.which('nvcc') is None:
+        nvcc = shutil.which(nvcc_path())
+        if nvcc is None:
             pytest.skip('nvcc not available to build the host simulation')
-        subprocess.run(['nvcc', '-gencode', 'arch=compute_100a,code=sm_100a', '-O2', '-std=c++17', '-shared', '-Xcompiler',
+        subprocess.run([nvcc, '-gencode', 'arch=compute_100a,code=sm_100a', '-O2', '-std=c++17', '-shared', '-Xcompiler',
                         '-fPIC', '-o', SO, SRC], check=True, cwd=ROOT)
     lib = ctypes.CDLL(SO)
     dp, ip = ctypes.POINTER(ctypes.c_double), ctypes.POINTER(ctypes.c_int32)
