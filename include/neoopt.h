@@ -216,6 +216,11 @@ int neo_launch_count(neo_handle *h, int64_t *count);
 /* test hooks: the double-double exp used for tau -> T, on the device and as compiled for the host */
 int neo_test_exp_dev(neo_handle *h, int n, const double *x, double *y);
 int neo_test_exp_host(int n, const double *x, double *y);
+/* test hooks: the optimizer's vector primitives (lbfgsb_tile.cuh) compiled for the device with the library's flags, one
+ * vector per thread. v, a, b: (count, n) row-major. nrm: dnrm2 (x87_nrm2.h); blas: the ddot kernel's summation order (n < 32);
+ * loop: scipy's own mul + add loop. */
+int neo_test_nrm2_dev(neo_handle *h, int count, int n, const double *v, double *nrm);
+int neo_test_ddot_dev(neo_handle *h, int count, int n, const double *a, const double *b, double *blas, double *loop);
 /* test hook (no GPU needed): `calls` runs of the host worker pool that neo_optimize uses, over [0, count); returns the number
  * of indices not visited exactly once per run. */
 int neo_test_host_pool(long long count, int calls);

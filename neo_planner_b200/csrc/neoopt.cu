@@ -426,6 +426,10 @@ __global__ void k_exp_dd(int n, const double *x, double *y)
     if (i < n) { bool o; y[i] = exp_dd(x[i], &o); }
 }
 
+// test_prims.cu: the optimizer's vector primitives on the device, in a translation unit of their own so that a second
+// caller does not change how k_optimize is compiled
+void launch_blas_prims(int count, int n, const double *a, const double *b, double *out, cudaStream_t stream);
+
 // ---------------------------------------------------------------------------------------------------------
 // handle
 // ---------------------------------------------------------------------------------------------------------
@@ -1701,6 +1705,46 @@ extern "C" int neo_test_exp_dev(neo_handle *h, int n, const double *x, double *y
     CK(cudaGetLastError());
     CK(cudaMemcpyAsync(y, d + n, sizeof(double) * n, cudaMemcpyDeviceToHost, h->stream));
     CK(cudaStreamSynchronize(h->stream));
+    return NEO_OK;
+}
+
+// test hooks: the optimizer's dnrm2 (x87_nrm2.h) and its two inner products as the device build computes them
+static int test_blas_prims(neo_handle *h, int count, int n, const double *a, const double *b, double *out)
+{
+    std::lock_guard<std::mutex> g(h->mu);
+    if (count == 0 || n == 0) { for (size_t i = 0; i < 3 * (size_t)count; i++) out[i] = 0.0; return NEO_OK; }
+    CK(cudaSetDevice(h->device));
+    double *d;
+    const size_t len = (size_t)count * n;
+    int rc = dev_buf(h, 5, sizeof(double) * (2 * len + 3 * (size_t)count), (void **)&d);
+    if (rc) return rc;
+    CK(cudaMemcpyAsync(d, a, sizeof(double) * len, cudaMemcpyHostToDevice, h->stream));
+    CK(cudaMemcpyAsync(d + len, b ? b : a, sizeof(double) * len, cudaMemcpyHostToDevice, h->stream));
+    launch_blas_prims(count, n, d, d + len, d + 2 * len, h->stream);
+    h->launches++;
+    CK(cudaGetLastError());
+    CK(cudaMemcpyAsync(out, d + 2 * len, sizeof(double) * 3 * count, cudaMemcpyDeviceToHost, h->stream));
+    CK(cudaStreamSynchronize(h->stream));
+    return NEO_OK;
+}
+
+extern "C" int neo_test_nrm2_dev(neo_handle *h, int count, int n, const double *v, double *nrm)
+{
+    if (!h || count < 0 || n < 0 || !v || !nrm) return NEO_ERR_INVALID;
+    std::vector<double> out(3 * (size_t)count);
+    const int rc = test_blas_prims(h, count, n, v, nullptr, out.data());
+    if (rc) return rc;
+    for (int i = 0; i < count; i++) nrm[i] = out[3 * (size_t)i];
+    return NEO_OK;
+}
+
+extern "C" int neo_test_ddot_dev(neo_handle *h, int count, int n, const double *a, const double *b, double *blas, double *loop)
+{
+    if (!h || count < 0 || n < 0 || !a || !b || !blas || !loop) return NEO_ERR_INVALID;
+    std::vector<double> out(3 * (size_t)count);
+    const int rc = test_blas_prims(h, count, n, a, b, out.data());
+    if (rc) return rc;
+    for (int i = 0; i < count; i++) { blas[i] = out[3 * (size_t)i + 1]; loop[i] = out[3 * (size_t)i + 2]; }
     return NEO_OK;
 }
 

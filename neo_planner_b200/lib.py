@@ -46,7 +46,7 @@ class Result(C.Structure):
 EXPORTS = ['neo_create', 'neo_destroy', 'neo_set_config', 'neo_last_error', 'neo_device_info', 'neo_set_map_esdf',
            'neo_set_map_occupancy', 'neo_set_maps_occupancy', 'neo_set_map_points', 'neo_get_occupancy', 'neo_get_map', 'neo_query_map', 'neo_eval', 'neo_eval_dev', 'neo_optimize',
            'neo_optimize_dev', 'neo_optimize_trace', 'neo_T2tau', 'neo_get_coeffs', 'neo_sample', 'neo_last_kernel_ms', 'neo_fp64_peak',
-           'neo_launch_count', 'neo_test_exp_dev', 'neo_test_exp_host', 'neo_test_host_pool', 'neo_astar', 'neo_astar_dev']
+           'neo_launch_count', 'neo_test_exp_dev', 'neo_test_exp_host', 'neo_test_nrm2_dev', 'neo_test_ddot_dev', 'neo_test_host_pool', 'neo_astar', 'neo_astar_dev']
 
 _lib = None
 
@@ -86,6 +86,8 @@ def load():
         lib.neo_launch_count.argtypes = [V, V]
         lib.neo_test_exp_dev.argtypes = [V, I, V, V]
         lib.neo_test_exp_host.argtypes = [I, V, V]
+        lib.neo_test_nrm2_dev.argtypes = [V, I, I, V, V]
+        lib.neo_test_ddot_dev.argtypes = [V, I, I, V, V, V, V]
         lib.neo_astar.argtypes = [V, I, V, V, V, I, I, V, V, V, V, V]
         lib.neo_astar_dev.argtypes = [V, I, V, V, V, I, I, V, V, V, V, V, V]
         _lib = lib
@@ -319,6 +321,19 @@ class Handle:
         x = f64(x).reshape(-1); y = np.empty_like(x)
         self._ck(self.lib.neo_test_exp_dev(self.h, x.size, ptr(x), ptr(y)))
         return y
+
+    def nrm2_dev(self, v):
+        """dnrm2 of each row of v (count, n) by the optimizer's nrm2_x87 on the device"""
+        v = f64(v); count, n = v.shape; out = np.empty(count)
+        self._ck(self.lib.neo_test_nrm2_dev(self.h, count, n, ptr(v), ptr(out)))
+        return out
+
+    def ddot_dev(self, a, b):
+        """row-wise a . b (count, n) by the optimizer's two inner products on the device: (blas_ddot, loop_dot)"""
+        a = f64(a); count, n = a.shape; b = f64(b, (count, n))
+        blas = np.empty(count); loop = np.empty(count)
+        self._ck(self.lib.neo_test_ddot_dev(self.h, count, n, ptr(a), ptr(b), ptr(blas), ptr(loop)))
+        return blas, loop
 
 
 def exp_host(x):

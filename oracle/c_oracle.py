@@ -57,6 +57,8 @@ def lib():
         _lib.orc_sample.argtypes = [C.c_int, C.c_void_p, C.c_void_p, C.c_double, C.c_int, C.c_void_p]
         _lib.orc_esdf_build.argtypes = [C.c_void_p, C.c_int, C.c_int, C.c_double, C.c_void_p, C.c_void_p, C.c_void_p]
         _lib.orc_esdf_brute.argtypes = [C.c_void_p, C.c_int, C.c_int, C.c_double, C.c_void_p]
+        _lib.orc_count_into.argtypes = [C.c_void_p]
+        _lib.orc_count_size.restype = C.c_int
     return _lib
 
 
@@ -163,8 +165,51 @@ def dnrm2(a):
     return float(f(a.size, a.ctypes.data_as(C.POINTER(C.c_double))))
 
 
-def lbfgsb_cb(fg, x0):
-    """The C restatement of scipy's L-BFGS-B around a Python evaluator fg(x) -> (f, g). Returns (x, nit, nfev, status)."""
+# the optimizer's branch counters (minco_oracle.c, enum OC_*), in order
+BRANCHES = ([f'dir_col{c}' for c in range(11)] +
+            ['factor_fail1', 'factor_fail2', 'nondescent_col0', 'nondescent_col', 'maxls', 'abnormal', 'reset_failed_search',
+             'skip_update', 'wrap', 'reset_after_wrap', 'accept_stp1', 'accept_stp', 'cache_hit'] +
+            [f'dcstep{k}_{"brackt" if b else "open"}' for k in range(1, 5) for b in (0, 1)] +
+            ['exit_conv', 'exit_bound', 'exit_xtol', 'exit_stpmax', 'exit_stpmin', 'stx_fallback',
+             'pg_x0', 'pg', 'ftol', 'maxiter', 'eval_overflow', 'eval_domain', 'eval_nan'])
+
+
+def new_counts():
+    """A zeroed counter array for the `counts=` argument of lbfgsb_cb / lbfgsb_replay (counts are added to it)."""
+    assert lib().orc_count_size() == len(BRANCHES)
+    return np.zeros(len(BRANCHES), np.int64)
+
+
+def counts_dict(c):
+    return {k: int(v) for k, v in zip(BRANCHES, c)}
+
+
+def _counted(counts, call):
+    if counts is None:
+        return call()
+    assert counts.dtype == np.int64 and counts.shape == (len(BRANCHES),) and counts.flags.c_contiguous
+    lib().orc_count_into(_p(counts))
+    try:
+        return call()
+    finally:
+        lib().orc_count_into(None)
+
+
+def ddot(a, b):
+    """The restated inner products on one pair of vectors: (the BLAS ddot kernel's order, scipy's own mul + add loop)."""
+    a = np.ascontiguousarray(a, dtype=np.float64); b = np.ascontiguousarray(b, dtype=np.float64)
+    assert a.shape == b.shape and a.ndim == 1
+    out = []
+    for f in (lib().orc_ddot, lib().orc_loop_dot):
+        f.restype = C.c_double
+        f.argtypes = [C.c_int, C.c_void_p, C.c_void_p]
+        out.append(float(f(a.size, _p(a), _p(b))))
+    return tuple(out)
+
+
+def lbfgsb_cb(fg, x0, counts=None):
+    """The C restatement of scipy's L-BFGS-B around a Python evaluator fg(x) -> (f, g). Returns (x, nit, nfev, status).
+    counts: an array from new_counts() to which the run's branch counters are added."""
     x0 = f64(x0); n = x0.size
 
     def tramp(_ctx, n_, xp, fp, gp, cp):
@@ -183,7 +228,7 @@ def lbfgsb_cb(fg, x0):
         return 0
     res = Result()
     cb = FG_FN(tramp)
-    st = lib().orc_lbfgsb_cb(C.c_int(n), _p(x0), cb, None, C.byref(res))
+    st = _counted(counts, lambda: lib().orc_lbfgsb_cb(C.c_int(n), _p(x0), cb, None, C.byref(res)))
     return np.array(res.x[:n]), res.nit, res.nfev, st
 
 
@@ -199,17 +244,19 @@ def lbfgsb_traced(params, omap, M, head, tail, x0, cap=4096):
                 xs=xs[:k], fs=fs[:k], gs=gs[:k])
 
 
-def lbfgsb_replay(x0, xs, fs, gs, costs=None, status=None):
+def lbfgsb_replay(x0, xs, fs, gs, costs=None, status=None, counts=None):
     """Feeds recorded evaluations (the device's) to the checker's optimizer. Returns dict(x, nit, nfev, status,
-    first_bad (-1: every requested point was bit-identical to the recorded one), used)."""
+    first_bad (-1: every requested point was bit-identical to the recorded one), used). counts: as for lbfgsb_cb; for a
+    replay that matched to the end they are the branches the recorded run took."""
     x0 = f64(x0); n = x0.size
     xs = f64(xs).reshape(-1, n); gs = f64(gs).reshape(-1, n); fs = f64(fs)
     k = xs.shape[0]
     costs = np.zeros((k, 4)) if costs is None else f64(costs)
     st = None if status is None else np.ascontiguousarray(status, dtype=np.int32)
     res = Result(); bad = C.c_int(-1); used = C.c_int(0)
-    rc = lib().orc_lbfgsb_replay(C.c_int(n), _p(x0), C.c_int(k), _p(xs), _p(fs), _p(gs), _p(costs),
-                                 None if st is None else _p(st), C.byref(res), C.byref(bad), C.byref(used))
+    rc = _counted(counts, lambda: lib().orc_lbfgsb_replay(C.c_int(n), _p(x0), C.c_int(k), _p(xs), _p(fs), _p(gs), _p(costs),
+                                                          None if st is None else _p(st), C.byref(res), C.byref(bad),
+                                                          C.byref(used)))
     return dict(x=np.array(res.x[:n]), nit=res.nit, nfev=res.nfev, status=rc, first_bad=bad.value, used=used.value,
                 costs=np.array(res.costs[:]))
 

@@ -514,11 +514,52 @@ typedef struct {
     double finit, ginit, gtest, width, width1, stx, fx, gx, sty, fy, gy, stmin, stmax;
 } dcs_state;
 
+/* Optional branch counters of the optimizer (tests: which L-BFGS-B branches a run went through). Integer increments only:
+ * the arithmetic is the same with and without them. The order is oracle/c_oracle.py's BRANCHES. */
+enum {
+    OC_DIR = 0,                       /* [0..10]: search directions computed with memory length col */
+    OC_FACTOR_FAIL1 = 11,             /* formk: first Cholesky factorisation failed (memory dropped) */
+    OC_FACTOR_FAIL2,                  /* formk: second Cholesky factorisation failed */
+    OC_NONDESCENT_COL0,               /* g'd >= 0 with an empty memory */
+    OC_NONDESCENT_COL,                /* g'd >= 0 with col > 0 */
+    OC_MAXLS,                         /* a 21st evaluation request: the search failed */
+    OC_ABNORMAL,                      /* failed search with an empty memory: ABNORMAL */
+    OC_RESET_FAILED,                  /* failed search with col > 0: memory dropped, search restarted */
+    OC_SKIP_UPDATE,                   /* s'y <= eps * (-g_old's): pair not stored */
+    OC_WRAP,                          /* a pair stored with a full memory (iupdat > 10): the oldest is overwritten */
+    OC_RESET_AFTER_WRAP,              /* a memory drop (either cause) after at least one wrap */
+    OC_ACCEPT_STP1,                   /* search accepted with stp == 1 */
+    OC_ACCEPT_STP,                    /* search accepted with stp != 1 */
+    OC_CACHE_HIT,                     /* trial point equal to the last evaluated one: not evaluated again */
+    OC_DCSTEP,                        /* [24..32): dcstep case 1..4 (2 * (case - 1)) x brackt at entry (+1) */
+    OC_EXIT_CONV = OC_DCSTEP + 8,     /* dcsrch: CONVERGENCE */
+    OC_EXIT_BOUND,                    /* dcsrch WARNING: brackt and stp outside (stmin, stmax) */
+    OC_EXIT_XTOL,                     /* dcsrch WARNING: interval width <= xtol * stmax */
+    OC_EXIT_STPMAX,                   /* dcsrch WARNING: stp == stpmax */
+    OC_EXIT_STPMIN,                   /* dcsrch WARNING: stp == stpmin */
+    OC_STX_FALLBACK,                  /* dcsrch: the new stp fell outside the bracket, stp = stx */
+    OC_PG_X0,                         /* projected gradient <= pgtol at x0 */
+    OC_PG,                            /* projected gradient <= pgtol after an iteration */
+    OC_FTOL,                          /* relative reduction of f <= factr * eps */
+    OC_MAXITER,                       /* iteration or evaluation limit */
+    OC_EVAL_OVERFLOW,                 /* the run ended on an evaluation status: overflow */
+    OC_EVAL_DOMAIN,                   /* ... domain error */
+    OC_EVAL_NAN,                      /* ... NaN */
+    OC_COUNT
+};
+static __thread int64_t *orc_count_cur = 0;
+#define OC(i) do { if (orc_count_cur) orc_count_cur[i]++; } while (0)
+
+/* counters go to c[0..OC_COUNT) (added to) for the calls this thread makes until it passes NULL */
+void orc_count_into(int64_t *c) { orc_count_cur = c; }
+int orc_count_size(void) { return OC_COUNT; }
+
 static void dcstep(double *stx, double *fx, double *dx, double *sty, double *fy, double *dy, double *stp,
                    double fp, double dp, int *brackt, double stpmin, double stpmax)
 {
     double sgnd = dp * (*dx / fabs(*dx));
     double stpf, stpc, stpq, theta, s, gamma, p, q, r;
+    OC(OC_DCSTEP + 2 * (fp > *fx ? 0 : sgnd < 0.0 ? 1 : fabs(dp) < fabs(*dx) ? 2 : 3) + (*brackt ? 1 : 0));
     if (fp > *fx) {
         theta = 3.0 * (*fx - fp) / (*stp - *stx) + *dx + dp;
         s = fmax(fabs(theta), fmax(fabs(*dx), fabs(dp)));
@@ -602,6 +643,13 @@ static int dcsrch_step(dcs_state *S, double *stp, double f, double g)
     if (*stp == LS_STPMAX && f <= ftest && g <= S->gtest) task = 2;
     if (*stp == LS_STPMIN && (f > ftest || g >= S->gtest)) task = 2;
     if (f <= ftest && fabs(g) <= LS_GTOL * (-S->ginit)) task = 1;
+    if (task == 1) OC(OC_EXIT_CONV);
+    else if (task == 2) {
+        if (S->brackt && (*stp <= S->stmin || *stp >= S->stmax)) OC(OC_EXIT_BOUND);
+        if (S->brackt && S->stmax - S->stmin <= LS_XTOL * S->stmax) OC(OC_EXIT_XTOL);
+        if (*stp == LS_STPMAX && f <= ftest && g <= S->gtest) OC(OC_EXIT_STPMAX);
+        if (*stp == LS_STPMIN && (f > ftest || g >= S->gtest)) OC(OC_EXIT_STPMIN);
+    }
     if (task) return task;
     if (S->stage == 1 && f <= S->fx && f > ftest) {
         double fm = f - *stp * S->gtest, fxm = S->fx - S->stx * S->gtest, fym = S->fy - S->sty * S->gtest;
@@ -620,7 +668,7 @@ static int dcsrch_step(dcs_state *S, double *stp, double f, double g)
     else { S->stmin = *stp + 1.1 * (*stp - S->stx); S->stmax = *stp + 4.0 * (*stp - S->stx); }
     *stp = fmax(*stp, LS_STPMIN); *stp = fmin(*stp, LS_STPMAX);
     if ((S->brackt && (*stp <= S->stmin || *stp >= S->stmax)) ||
-        (S->brackt && S->stmax - S->stmin <= LS_XTOL * S->stmax)) *stp = S->stx;
+        (S->brackt && S->stmax - S->stmin <= LS_XTOL * S->stmax)) { *stp = S->stx; OC(OC_STX_FALLBACK); }
     return 0;
 }
 
@@ -768,6 +816,7 @@ static void lb_update(lb_mem *C, const double *s, const double *y, double rr, do
     C->iupdat++;
     if (C->iupdat <= LB_M) C->col = C->iupdat;
     else {
+        OC(OC_WRAP);
         memmove(C->ws[0], C->ws[1], sizeof(double) * (LB_M - 1) * ORC_MAXN);
         memmove(C->wy[0], C->wy[1], sizeof(double) * (LB_M - 1) * ORC_MAXN);
         for (int j = 0; j < LB_M - 1; j++) {
@@ -797,13 +846,14 @@ static int lb_factor(lb_mem *C)
         for (int jy = iy; jy < col; jy++) wn[jy][is] = C->rz[iy][jy];
         wn[iy][iy] = wn[iy][iy] + C->dr[iy];
     }
-    if (!lapack_potf2(wn, 0, col)) return 0;
+    if (!lapack_potf2(wn, 0, col)) { OC(OC_FACTOR_FAIL1); return 0; }
     if (col == 1) wn[0][1] = wn[0][1] / wn[0][0];        /* one right-hand side: trsv */
     else blas_trsm_LT(wn, col, col, col);
     for (int is = col; is < 2 * col; is++)
         for (int js = is; js < 2 * col; js++)
             wn[is][js] = wn[is][js] + blas_ddot(col, &wn[0][is], LB_W, &wn[0][js], LB_W);
-    return lapack_potf2(wn, col, col);
+    if (!lapack_potf2(wn, col, col)) { OC(OC_FACTOR_FAIL2); return 0; }
+    return 1;
 }
 
 /* subsm with r = -g: the subspace step (added to x by the caller) */
@@ -853,7 +903,10 @@ static int lbfgsb_run(int n, const double *x0, orc_fg_fn fg, void *ctx, orc_resu
 #define LB_EVAL()                                                                                              \
     do {                                                                                                       \
         st = fg(ctx, n, x, &f, g, costs);                                                                      \
-        if (st) { out->status = st; out->nit = nit; out->nfev = nfev; memcpy(out->x, x, sizeof(double) * n); return st; } \
+        if (st) {                                                                                              \
+            if (st >= ORC_OVERFLOW && st <= ORC_NAN) OC(OC_EVAL_OVERFLOW + st - ORC_OVERFLOW);                  \
+            out->status = st; out->nit = nit; out->nfev = nfev; memcpy(out->x, x, sizeof(double) * n); return st; \
+        }                                                                                                      \
         nfev++; memcpy(xl, x, sizeof(double) * n); memcpy(out->costs, costs, sizeof(costs));                    \
         if (orc_trace_cur && orc_trace_cur->len < orc_trace_cur->cap) {                                        \
             orc_trace *T = orc_trace_cur;                                                                      \
@@ -863,56 +916,61 @@ static int lbfgsb_run(int n, const double *x0, orc_fg_fn fg, void *ctx, orc_resu
     } while (0)
     LB_EVAL();
     double sbg = 0.0; for (int i = 0; i < n; i++) sbg = fmax(sbg, fabs(g[i]));
-    if (sbg <= pgtol) { st = ORC_CONV_PG; goto done; }
+    if (sbg <= pgtol) { st = ORC_CONV_PG; OC(OC_PG_X0); goto done; }
     for (;;) {
         /* search direction: Cauchy point x - g with an empty memory (theta = 1), else the subspace step; d = z - x */
         if (C.col == 0) for (int i = 0; i < n; i++) z[i] = x[i] - g[i];
         else {
-            if (!lb_factor(&C)) { lb_reset(&C, n); continue; }
+            if (!lb_factor(&C)) { if (C.iupdat > LB_M) OC(OC_RESET_AFTER_WRAP); lb_reset(&C, n); continue; }
             lb_step(&C, g, d);
             for (int i = 0; i < n; i++) z[i] = x[i] + d[i];
         }
         for (int i = 0; i < n; i++) d[i] = z[i] - x[i];
+        OC(OC_DIR + C.col);
         /* lnsrlb */
         const double dnorm = blas_dnrm2(n, d);
         double stp = (nit == 0) ? fmin(1.0 / dnorm, LS_STPMAX) : 1.0;
         memcpy(t, x, sizeof(double) * n); memcpy(r, g, sizeof(double) * n); fold = f;
         double gd = blas_ddot(n, g, 1, d, 1), gdold = gd;
         int fail = 0;
-        if (gd >= 0.0) fail = 1;
+        if (gd >= 0.0) { fail = 1; OC(C.col == 0 ? OC_NONDESCENT_COL0 : OC_NONDESCENT_COL); }
         else {
             dcs_state ls; dcsrch_start(&ls, stp, f, gd);
             int ifun = 0;
             for (;;) {
                 ifun++;
-                if (ifun - 1 >= maxls) { fail = 1; break; }
+                if (ifun - 1 >= maxls) { fail = 1; OC(OC_MAXLS); break; }
                 if (stp == 1.0) memcpy(xn, z, sizeof(double) * n);
                 else for (int i = 0; i < n; i++) xn[i] = stp * d[i] + t[i];
                 int same = 1; for (int i = 0; i < n; i++) if (xn[i] != xl[i]) { same = 0; break; }
                 memcpy(x, xn, sizeof(double) * n);
                 if (!same) LB_EVAL();          /* scipy's ScalarFunction does not re-evaluate an unchanged x */
+                else OC(OC_CACHE_HIT);
                 gd = blas_ddot(n, g, 1, d, 1);
                 if (dcsrch_step(&ls, &stp, f, gd)) break;
             }
         }
         if (fail) {
             memcpy(x, t, sizeof(double) * n); memcpy(g, r, sizeof(double) * n); f = fold;
-            if (C.col == 0) { st = ORC_ABNORMAL; goto done; }
+            if (C.col == 0) { st = ORC_ABNORMAL; OC(OC_ABNORMAL); goto done; }
+            OC(OC_RESET_FAILED);
+            if (C.iupdat > LB_M) OC(OC_RESET_AFTER_WRAP);
             lb_reset(&C, n);
             continue;
         }
         nit++;
+        OC(stp == 1.0 ? OC_ACCEPT_STP1 : OC_ACCEPT_STP);
         sbg = 0.0; for (int i = 0; i < n; i++) sbg = fmax(sbg, fabs(g[i]));
-        if (sbg <= pgtol) { st = ORC_CONV_PG; goto done; }
-        { const double dd = fmax(fmax(fabs(fold), fabs(f)), 1.0); if (fold - f <= tol * dd) { st = ORC_CONV_FTOL; goto done; } }
-        if (nit >= maxiter || nfev > maxfun) { st = ORC_MAXITER; goto done; }
+        if (sbg <= pgtol) { st = ORC_CONV_PG; OC(OC_PG); goto done; }
+        { const double dd = fmax(fmax(fabs(fold), fabs(f)), 1.0); if (fold - f <= tol * dd) { st = ORC_CONV_FTOL; OC(OC_FTOL); goto done; } }
+        if (nit >= maxiter || nfev > maxfun) { st = ORC_MAXITER; OC(OC_MAXITER); goto done; }
         /* BFGS update (matupd) */
         double rr, dr, ddum;
         for (int i = 0; i < n; i++) r[i] = g[i] - r[i];
         { const double nr = blas_dnrm2(n, r); rr = nr * nr; }
         if (stp == 1.0) { dr = gd - gdold; ddum = -gdold; }
         else { dr = (gd - gdold) * stp; for (int i = 0; i < n; i++) d[i] = d[i] * stp; ddum = -gdold * stp; }
-        if (dr <= epsmch * ddum) continue;   /* skip the update */
+        if (dr <= epsmch * ddum) { OC(OC_SKIP_UPDATE); continue; }   /* skip the update */
         lb_update(&C, d, r, rr, dr);
     }
 done:
@@ -945,6 +1003,9 @@ int orc_lbfgsb(const orc_params *p, const orc_map *map, int M, const double *hea
 int orc_lbfgsb_cb(int n, const double *x0, orc_fg_fn fg, void *ctx, orc_result *out) { return lbfgsb_run(n, x0, fg, ctx, out); }
 /* the restated BLAS norm alone (tests/test_x87_nrm2.py pins it to scipy's bundled kernel) */
 double orc_dnrm2(int n, const double *a) { return blas_dnrm2(n, a); }
+/* ... and the two inner products (the BLAS kernel's order, and scipy's own loops) */
+double orc_ddot(int n, const double *a, const double *b) { return blas_ddot(n, a, 1, b, 1); }
+double orc_loop_dot(int n, const double *a, const double *b) { return loop_dot(n, a, b); }
 
 /* ... with every evaluation recorded: x (cap, n), f (cap), g (cap, n); returns the number of evaluations recorded */
 int orc_lbfgsb_traced(const orc_params *p, const orc_map *map, int M, const double *head, const double *tail,

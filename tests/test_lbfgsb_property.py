@@ -27,13 +27,7 @@ def openblas_core():
     return b'?'
 
 
-@settings(max_examples=120, deadline=None, suppress_health_check=[HealthCheck.too_slow], derandomize=True, database=None)
-@given(n=st.integers(2, 28), seed=st.integers(0, 2**31 - 1), cond=st.floats(0.0, 4.0), quartic=st.floats(0.0, 2.0),
-       skew=st.floats(0.0, 0.3))
-# found by this test in round 2: the last trial point differed in one component by one ulp because the restated norm
-# added the squares sequentially; OpenBLAS's x87 kernel uses four accumulators for n >= 8 (tests/test_x87_nrm2.py)
-@example(n=25, seed=25, cond=1.582789709559926, quartic=1.582789709559926, skew=0.0)
-def test_restated_lbfgsb_walks_scipys_iterates(n, seed, cond, quartic, skew):
+def random_objective(n, seed, cond, quartic, skew):
     rng = np.random.default_rng(seed)
     Q = np.linalg.qr(rng.normal(size=(n, n)))[0]
     H = Q @ np.diag(10.0 ** rng.uniform(-cond / 2, cond / 2, n)) @ Q.T
@@ -45,7 +39,17 @@ def test_restated_lbfgsb_walks_scipys_iterates(n, seed, cond, quartic, skew):
 
     def g(x):       # skew > 0: not the gradient of f (a rotation is mixed in), as in the reference
         return H @ x + 4.0 * quartic * (x - c) ** 3 - np.sin(x) + S @ np.sin(x)
+    return f, g, x0
 
+
+@settings(max_examples=120, deadline=None, suppress_health_check=[HealthCheck.too_slow], derandomize=True, database=None)
+@given(n=st.integers(2, 28), seed=st.integers(0, 2**31 - 1), cond=st.floats(0.0, 4.0), quartic=st.floats(0.0, 2.0),
+       skew=st.floats(0.0, 0.3))
+# found by this test in round 2: the last trial point differed in one component by one ulp because the restated norm
+# added the squares sequentially; OpenBLAS's x87 kernel uses four accumulators for n >= 8 (tests/test_x87_nrm2.py)
+@example(n=25, seed=25, cond=1.582789709559926, quartic=1.582789709559926, skew=0.0)
+def test_restated_lbfgsb_walks_scipys_iterates(n, seed, cond, quartic, skew):
+    f, g, x0 = random_objective(n, seed, cond, quartic, skew)
     res = sopt.minimize(f, x0, method='L-BFGS-B', jac=g, bounds=None, tol=1e-4,
                         options={'maxcor': 10, 'maxfun': 15000, 'maxiter': 15000, 'maxls': 20})
     x, nit, nfev, status = c_oracle.lbfgsb_cb(lambda v: (f(v), g(v)), x0)

@@ -14,6 +14,7 @@ import pytest
 from scipy.linalg import blas
 
 from oracle import c_oracle
+from test_lbfgsb_property import openblas_core
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 SRC = os.path.join(ROOT, 'devtools', 'x87_host.cpp')
@@ -77,3 +78,66 @@ def test_edge_magnitudes(sim):
     fast, exact = sim(v)
     real = np.array([blas.dnrm2(row) for row in v])
     assert np.array_equal(fast, real) and np.array_equal(exact, real)
+
+
+def dot_vectors(rng, count, n):
+    """Pairs whose products span twelve decades and whose sum cancels to a small fraction of its largest term, so that the
+    summation order and which products are fused decide the last bits."""
+    a = rng.normal(size=(count, n)) * 10.0 ** rng.uniform(-6, 6, size=(count, 1)) * 10.0 ** rng.uniform(-3, 3, size=(count, n))
+    b = rng.normal(size=(count, n)) * 10.0 ** rng.uniform(-3, 3, size=(count, n))
+    if n >= 2:
+        k = count // 2
+        p = a[:k, :-1] * b[:k, :-1]
+        a[:k, -1] = -p.sum(axis=1) / b[:k, -1] * (1.0 + rng.normal(size=k) * 1e-9)
+    return a, b
+
+
+@pytest.fixture(scope='module')
+def dev():
+    from neo_planner_b200 import lib
+    from neo_planner_b200.worlds import YamlConfig
+    h = lib.Handle(YamlConfig(), 0, 1)
+    yield h
+    h.close()
+
+
+@pytest.mark.gpu
+@pytest.mark.parametrize('n', list(range(1, 33)) + [40, 63])
+def test_device_build_nrm2_equals_the_real_kernel(dev, n):
+    """nrm2_x87 of lbfgsb_tile.cuh compiled by nvcc with the library's flags (--fmad=true: its two-sum is written with
+    plain operators that nvcc may contract) on the adversarial vectors above."""
+    rng = np.random.default_rng(1000 + n)
+    v = vectors(rng, 4000 if n < 8 else 16000, n)
+    got = dev.nrm2_dev(v)
+    checker = np.array([c_oracle.dnrm2(row) for row in v])
+    assert np.array_equal(got, checker), (n, int((got != checker).sum()))
+    real = np.array([blas.dnrm2(row) for row in v])
+    assert np.array_equal(got, real), (n, int((got != real).sum()))
+
+
+@pytest.mark.gpu
+def test_device_build_nrm2_edge_magnitudes(dev):
+    v = np.array([[0.0, 0.0, 0.0], [1e-200, 2e-200, 0.0], [1e150, 1e150, 1e150], [3.0, 4.0, 0.0], [1.0, 0.0, 0.0],
+                  [2.0 ** -600, 2.0 ** -600, 2.0 ** -600], [1e-310, 0.0, 5e-324], [1e300, -1e300, 1e-300],
+                  [2.0 ** 511, 2.0 ** 511, 0.0], [-7.0, 0.0, -24.0]])
+    got = dev.nrm2_dev(v)
+    assert np.array_equal(got, np.array([blas.dnrm2(row) for row in v]))
+    assert np.array_equal(got, np.array([c_oracle.dnrm2(row) for row in v]))
+
+
+@pytest.mark.gpu
+@pytest.mark.parametrize('n', list(range(1, 32)))
+def test_device_build_ddot_equals_the_checker(dev, n):
+    """blas_ddot (fused chain; the four-lane prefix from n = 16) and loop_dot (multiply, then add) of lbfgsb_tile.cuh as
+    nvcc compiles them for the device, against the checker's restatement and, for the BLAS order, scipy's own ddot."""
+    rng = np.random.default_rng(2000 + n)
+    a, b = dot_vectors(rng, 4000, n)
+    blas_d, loop_d = dev.ddot_dev(a, b)
+    ref = np.array([c_oracle.ddot(x, y) for x, y in zip(a, b)])
+    assert np.array_equal(blas_d, ref[:, 0]), (n, int((blas_d != ref[:, 0]).sum()))
+    assert np.array_equal(loop_d, ref[:, 1]), (n, int((loop_d != ref[:, 1]).sum()))
+    if n >= 2:
+        assert (ref[:, 0] != ref[:, 1]).sum() >= 100        # the vectors tell the two orders apart
+    if openblas_core() in (b'SkylakeX', b'?'):
+        real = np.array([blas.ddot(x, y) for x, y in zip(a, b)])
+        assert np.array_equal(blas_d, real), (n, int((blas_d != real).sum()))
