@@ -15,6 +15,7 @@
 #include <mutex>
 #include <thread>
 #include <string>
+#include <type_traits>
 #include <vector>
 
 #include "../../include/neoopt.h"
@@ -531,8 +532,13 @@ struct neo_handle {
     std::vector<MapView> views;      // host copies of the published views (sources of the async uploads)
     MapView *d_maps = nullptr;
     unsigned int *d_counter = nullptr;
-    std::vector<DevBuf> bufs;        // reusable device staging buffers for the host-pointer entry points
-    DevBuf pinned;                   // reusable pinned host staging buffer (neo_optimize)
+    // Grow-only buffers. Every host-pointer entry point synchronises before it returns and runs under mu, so all of
+    // them lay out their device arrays in `stage`. The two scratch areas a device-pointer launch still reads after its
+    // call has returned have buffers of their own.
+    DevBuf stage;
+    DevBuf opt_scratch;              // launch_optimize: per-task records and per-problem state words
+    DevBuf astar_overflow;           // astar_launch: overflow list of the first pass
+    DevBuf pinned;                   // pinned host staging buffer (neo_optimize)
     DevBuf astar;                    // per-warp search scratch of neo_astar (node records all-zero between launches)
     size_t astar_cap = 0;            // cells per warp the scratch is laid out for
     int astar_warps = 0;             // worker warps the scratch is laid out for
@@ -562,7 +568,7 @@ static std::string g_create_err;
         }                                                                                                 \
     } while (0)
 
-static int fail(neo_handle *h, const char *msg)
+static int fail(neo_handle *h, const std::string &msg)
 {
     h->err = msg;
     return NEO_ERR_INVALID;
@@ -578,36 +584,32 @@ static DevParams dev_params(const neo_config &c)
     return P;
 }
 
-// grow-only device staging buffer #i
-static int dev_buf(neo_handle *h, size_t i, size_t bytes, void **out)
+// makes b hold at least `bytes`: device memory, or mapped pinned host memory for h->pinned (the optimizer writes its
+// results straight into it). A call must not grow a buffer it has already enqueued copies into.
+static int grow(neo_handle *h, DevBuf &b, size_t bytes, char **out)
 {
-    if (h->bufs.size() <= i) h->bufs.resize(i + 1);
-    DevBuf &b = h->bufs[i];
+    const bool pinned = &b == &h->pinned;
     if (b.cap < bytes) {
-        if (b.p) CK(cudaFree(b.p));
+        if (b.p) CK(pinned ? cudaFreeHost(b.p) : cudaFree(b.p));
         b.p = nullptr; b.cap = 0;
-        size_t cap = bytes + bytes / 4 + 256;
-        CK(cudaMalloc(&b.p, cap));
+        const size_t cap = bytes + bytes / 4 + 256;
+        CK(pinned ? cudaHostAlloc(&b.p, cap, cudaHostAllocMapped) : cudaMalloc(&b.p, cap));
         b.cap = cap;
     }
-    *out = b.p;
+    *out = (char *)b.p;
     return NEO_OK;
 }
 
-// grow-only pinned host staging buffer
-static int pin_buf(neo_handle *h, size_t bytes, void **out)
-{
-    DevBuf &b = h->pinned;
-    if (b.cap < bytes) {
-        if (b.p) CK(cudaFreeHost(b.p));
-        b.p = nullptr; b.cap = 0;
-        const size_t cap = bytes + bytes / 4 + 256;
-        CK(cudaHostAlloc(&b.p, cap, cudaHostAllocMapped));      // mapped: the optimizer writes its results straight into it
-        b.cap = cap;
+// byte offsets of arrays laid out one after another in one buffer, each 256-byte aligned; end is the total size
+struct Layout {
+    size_t end = 0;
+    size_t add(size_t bytes)
+    {
+        const size_t at = (end + 255) & ~(size_t)255;
+        end = at + bytes;
+        return at;
     }
-    *out = b.p;
-    return NEO_OK;
-}
+};
 
 static int cfg_check(const neo_config *c)
 {
@@ -660,9 +662,8 @@ extern "C" int neo_destroy(neo_handle *h)
     cudaSetDevice(h->device);
     cudaStreamSynchronize(h->stream);
     for (auto &s : h->slots) { if (s.cells) cudaFree(s.cells); if (s.occ) cudaFree(s.occ); if (s.blocked) cudaFree(s.blocked); }
-    for (auto &b : h->bufs) if (b.p) cudaFree(b.p);
+    for (DevBuf *b : {&h->stage, &h->opt_scratch, &h->astar_overflow, &h->astar}) if (b->p) cudaFree(b->p);
     if (h->pinned.p) cudaFreeHost(h->pinned.p);
-    if (h->astar.p) cudaFree(h->astar.p);
     cudaFree(h->d_maps); cudaFree(h->d_counter);
     cudaEventDestroy(h->ev0); cudaEventDestroy(h->ev1);
     cudaStreamDestroy(h->stream);
@@ -705,12 +706,17 @@ static int slot_prepare(neo_handle *h, int slot, int H, int W, double res, doubl
     return NEO_OK;
 }
 
+static MapView map_view(const MapSlot &s)
+{
+    MapView v;
+    v.cells = s.cells; v.H = s.H; v.W = s.W; v.res = s.res; v.ox = s.ox; v.oy = s.oy; v.inv_res = 1.0 / s.res;
+    v.blocked = s.blocked;
+    return v;
+}
+
 static int slot_publish(neo_handle *h, int slot, bool sync = true)
 {
     MapSlot &s = h->slots[slot];
-    MapView v;
-    v.cells = s.cells; v.H = s.H; v.W = s.W; v.res = s.res; v.ox = s.ox; v.oy = s.oy; v.inv_res = 1.0 / s.res;
-    v.blocked = nullptr;
     // node-blocked grid of the geometric initializer (AP:130-141), one byte per node of the enlarged grid
     const size_t nodes = astar_grid_cells(s.H, s.W, s.res);
     if (s.blocked_cap < nodes) {
@@ -718,12 +724,12 @@ static int slot_publish(neo_handle *h, int slot, bool sync = true)
         CK(cudaMalloc(&s.blocked, nodes));
         s.blocked_cap = nodes;
     }
+    const MapView v = map_view(s);
     const int pad = (int)(10.0 / s.res);
     dim3 grid((s.W + pad + 127) / 128, s.H + pad);
     k_astar_blocked<<<grid, 128, 0, h->stream>>>(v, s.blocked);
     h->launches++;
     CK(cudaGetLastError());
-    v.blocked = s.blocked;
     h->views[slot] = v;                 // pageable source of an async copy: must outlive the call
     CK(cudaMemcpyAsync(h->d_maps + slot, &h->views[slot], sizeof(v), cudaMemcpyHostToDevice, h->stream));
     if (sync) CK(cudaStreamSynchronize(h->stream));
@@ -740,25 +746,34 @@ extern "C" int neo_set_map_esdf(neo_handle *h, int slot, int H, int W, double re
     int rc = slot_prepare(h, slot, H, W, res, ox, oy);
     if (rc) return rc;
     const size_t n = (size_t)H * W;
-    double *d;
-    if ((rc = dev_buf(h, 0, sizeof(double) * 3 * n, (void **)&d))) return rc;
-    CK(cudaMemcpyAsync(d, esdf, sizeof(double) * n, cudaMemcpyHostToDevice, h->stream));
-    CK(cudaMemcpyAsync(d + n, gx, sizeof(double) * n, cudaMemcpyHostToDevice, h->stream));
-    CK(cudaMemcpyAsync(d + 2 * n, gy, sizeof(double) * n, cudaMemcpyHostToDevice, h->stream));
+    Layout L;
+    const size_t o_e = L.add(sizeof(double) * n), o_gx = L.add(sizeof(double) * n), o_gy = L.add(sizeof(double) * n);
+    char *d;
+    if ((rc = grow(h, h->stage, L.end, &d))) return rc;
+    CK(cudaMemcpyAsync(d + o_e, esdf, sizeof(double) * n, cudaMemcpyHostToDevice, h->stream));
+    CK(cudaMemcpyAsync(d + o_gx, gx, sizeof(double) * n, cudaMemcpyHostToDevice, h->stream));
+    CK(cudaMemcpyAsync(d + o_gy, gy, sizeof(double) * n, cudaMemcpyHostToDevice, h->stream));
     dim3 grid((W + 127) / 128, H);
-    k_pack_cells<<<grid, 128, 0, h->stream>>>(d, d + n, d + 2 * n, H, W, h->slots[slot].cells, nullptr, nullptr);
+    k_pack_cells<<<grid, 128, 0, h->stream>>>((double *)(d + o_e), (double *)(d + o_gx), (double *)(d + o_gy), H, W,
+                                              h->slots[slot].cells, nullptr, nullptr);
     h->launches++;
     CK(cudaGetLastError());
     return slot_publish(h, slot);
 }
 
-// occupancy (device, int8) -> exact EDT -> cells; d_occ lives in staging buffer 0 (offset 0)
-static int build_from_occ(neo_handle *h, int slot, int H, int W, double res, char *base, size_t off_g, size_t off_any, size_t off_e,
-                          bool sync = true)
+// device arrays of one occupancy -> EDT -> cells build: the binarised grid, the EDT's row pass, its flag, the distances
+struct OccArrays { size_t occ, g, any, e; };
+static OccArrays occ_arrays(Layout &L, size_t n)
 {
-    const int8_t *d_occ = (const int8_t *)base;
-    int *d_g = (int *)(base + off_g), *d_any = (int *)(base + off_any);
-    double *d_e = (double *)(base + off_e);
+    return {L.add(n), L.add(sizeof(int) * n), L.add(sizeof(int)), L.add(sizeof(double) * n)};
+}
+
+// occupancy (device, int8, in the staging buffer at base) -> exact EDT -> cells
+static int build_from_occ(neo_handle *h, int slot, int H, int W, double res, char *base, const OccArrays &o, bool sync = true)
+{
+    const int8_t *d_occ = (const int8_t *)(base + o.occ);
+    int *d_g = (int *)(base + o.g), *d_any = (int *)(base + o.any);
+    double *d_e = (double *)(base + o.e);
     MapSlot &s = h->slots[slot];
     const size_t n = (size_t)H * W;
     if (s.occ && s.occ_cap < n) { CK(cudaFree(s.occ)); s.occ = nullptr; }
@@ -774,17 +789,6 @@ static int build_from_occ(neo_handle *h, int slot, int H, int W, double res, cha
     return slot_publish(h, slot, sync);
 }
 
-struct OccLayout { size_t off_g, off_any, off_e, total; };
-static OccLayout occ_layout(size_t n)
-{
-    OccLayout L;
-    L.off_g = (n + 255) & ~(size_t)255;
-    L.off_any = L.off_g + sizeof(int) * n;
-    L.off_e = (L.off_any + 256 + 255) & ~(size_t)255;
-    L.total = L.off_e + sizeof(double) * n;
-    return L;
-}
-
 extern "C" int neo_set_map_occupancy(neo_handle *h, int slot, int H, int W, double res, double ox, double oy,
                                      const int8_t *occ)
 {
@@ -796,11 +800,12 @@ extern "C" int neo_set_map_occupancy(neo_handle *h, int slot, int H, int W, doub
     int rc = slot_prepare(h, slot, H, W, res, ox, oy);
     if (rc) return rc;
     const size_t n = (size_t)H * W;
-    const OccLayout L = occ_layout(n);
-    char *base;
-    if ((rc = dev_buf(h, 0, L.total, (void **)&base))) return rc;
-    CK(cudaMemcpyAsync(base, occ, n, cudaMemcpyHostToDevice, h->stream));
-    return build_from_occ(h, slot, H, W, res, base, L.off_g, L.off_any, L.off_e);
+    Layout L;
+    const OccArrays o = occ_arrays(L, n);
+    char *d;
+    if ((rc = grow(h, h->stage, L.end, &d))) return rc;
+    CK(cudaMemcpyAsync(d + o.occ, occ, n, cudaMemcpyHostToDevice, h->stream));
+    return build_from_occ(h, slot, H, W, res, d, o);
 }
 
 // K maps of one shape in one call (the 256 generated worlds of the data-generation sweep): one H2D copy per group of
@@ -819,21 +824,22 @@ extern "C" int neo_set_maps_occupancy(neo_handle *h, int K, const int32_t *slots
     if (K == 0) return NEO_OK;
     CK(cudaSetDevice(h->device));
     const size_t n = (size_t)H * W;
-    const OccLayout L = occ_layout(n);
-    const size_t stride = (L.total + 255) & ~(size_t)255;
     const int group = K < 32 ? K : 32;                        // staging for 32 maps at a time
-    char *base;
-    int rc = dev_buf(h, 0, stride * group, (void **)&base);
+    Layout L;
+    std::vector<OccArrays> o(group);
+    for (auto &a : o) a = occ_arrays(L, n);
+    char *d;
+    int rc = grow(h, h->stage, L.end, &d);
     if (rc) return rc;
     for (int k0 = 0; k0 < K; k0 += group) {
         const int kn = K - k0 < group ? K - k0 : group;
         if (k0) CK(cudaStreamSynchronize(h->stream));          // the staging block is reused by the next group
         for (int k = 0; k < kn; k++) {
             if ((rc = slot_prepare(h, slots[k0 + k], H, W, res, ox[k0 + k], oy[k0 + k]))) return rc;
-            CK(cudaMemcpyAsync(base + stride * k, occ + n * (size_t)(k0 + k), n, cudaMemcpyHostToDevice, h->stream));
+            CK(cudaMemcpyAsync(d + o[k].occ, occ + n * (size_t)(k0 + k), n, cudaMemcpyHostToDevice, h->stream));
         }
         for (int k = 0; k < kn; k++)
-            if ((rc = build_from_occ(h, slots[k0 + k], H, W, res, base + stride * k, L.off_g, L.off_any, L.off_e, false))) return rc;
+            if ((rc = build_from_occ(h, slots[k0 + k], H, W, res, d, o[k], false))) return rc;
     }
     CK(cudaStreamSynchronize(h->stream));
     return NEO_OK;
@@ -850,20 +856,20 @@ extern "C" int neo_set_map_points(neo_handle *h, int slot, int n_points, const f
     int rc = slot_prepare(h, slot, H, W, res, ox, oy);
     if (rc) return rc;
     const size_t n = (size_t)H * W;
-    const OccLayout L = occ_layout(n);
-    char *base;
-    float *d_xyz;
-    if ((rc = dev_buf(h, 0, L.total, (void **)&base))) return rc;
-    if ((rc = dev_buf(h, 1, sizeof(float) * 3 * (size_t)(n_points > 0 ? n_points : 1), (void **)&d_xyz))) return rc;
-    CK(cudaMemsetAsync(base, 0, n, h->stream));
+    Layout L;
+    const OccArrays o = occ_arrays(L, n);
+    const size_t o_xyz = L.add(sizeof(float) * 3 * (size_t)n_points);
+    char *d;
+    if ((rc = grow(h, h->stage, L.end, &d))) return rc;
+    CK(cudaMemsetAsync(d + o.occ, 0, n, h->stream));
     if (n_points > 0) {
-        CK(cudaMemcpyAsync(d_xyz, xyz, sizeof(float) * 3 * (size_t)n_points, cudaMemcpyHostToDevice, h->stream));
-        k_points_to_occ<<<(n_points + 255) / 256, 256, 0, h->stream>>>(d_xyz, n_points, z_min, z_max, ox, oy, res, H, W,
-                                                                       (int8_t *)base);
+        CK(cudaMemcpyAsync(d + o_xyz, xyz, sizeof(float) * 3 * (size_t)n_points, cudaMemcpyHostToDevice, h->stream));
+        k_points_to_occ<<<(n_points + 255) / 256, 256, 0, h->stream>>>((const float *)(d + o_xyz), n_points, z_min, z_max,
+                                                                       ox, oy, res, H, W, (int8_t *)(d + o.occ));
         h->launches++;
         CK(cudaGetLastError());
     }
-    return build_from_occ(h, slot, H, W, res, base, L.off_g, L.off_any, L.off_e);
+    return build_from_occ(h, slot, H, W, res, d, o);
 }
 
 extern "C" int neo_get_occupancy(neo_handle *h, int slot, int8_t *occ)
@@ -886,15 +892,18 @@ extern "C" int neo_get_map(neo_handle *h, int slot, double *esdf, double *gx, do
     CK(cudaSetDevice(h->device));
     const MapSlot &s = h->slots[slot];
     const size_t n = (size_t)s.H * s.W;
-    double *d;
-    int rc = dev_buf(h, 0, sizeof(double) * 3 * n, (void **)&d);
+    Layout L;
+    const size_t o_e = L.add(sizeof(double) * n), o_gx = L.add(sizeof(double) * n), o_gy = L.add(sizeof(double) * n);
+    char *d;
+    int rc = grow(h, h->stage, L.end, &d);
     if (rc) return rc;
-    k_unpack_cells<<<(unsigned)((n + 255) / 256), 256, 0, h->stream>>>(s.cells, n, d, d + n, d + 2 * n);
+    k_unpack_cells<<<(unsigned)((n + 255) / 256), 256, 0, h->stream>>>(s.cells, n, (double *)(d + o_e), (double *)(d + o_gx),
+                                                                       (double *)(d + o_gy));
     h->launches++;
     CK(cudaGetLastError());
-    if (esdf) CK(cudaMemcpyAsync(esdf, d, sizeof(double) * n, cudaMemcpyDeviceToHost, h->stream));
-    if (gx) CK(cudaMemcpyAsync(gx, d + n, sizeof(double) * n, cudaMemcpyDeviceToHost, h->stream));
-    if (gy) CK(cudaMemcpyAsync(gy, d + 2 * n, sizeof(double) * n, cudaMemcpyDeviceToHost, h->stream));
+    if (esdf) CK(cudaMemcpyAsync(esdf, d + o_e, sizeof(double) * n, cudaMemcpyDeviceToHost, h->stream));
+    if (gx) CK(cudaMemcpyAsync(gx, d + o_gx, sizeof(double) * n, cudaMemcpyDeviceToHost, h->stream));
+    if (gy) CK(cudaMemcpyAsync(gy, d + o_gy, sizeof(double) * n, cudaMemcpyDeviceToHost, h->stream));
     CK(cudaStreamSynchronize(h->stream));
     return NEO_OK;
 }
@@ -907,23 +916,20 @@ extern "C" int neo_query_map(neo_handle *h, int slot, int n, const double *xy, i
     if (n < 0 || !xy || !idx || !dis || !grad) return fail(h, "neo_query_map: invalid argument");
     if (n == 0) return NEO_OK;
     CK(cudaSetDevice(h->device));
-    const MapSlot &s = h->slots[slot];
-    char *base;
-    const size_t o_xy = 0, o_idx = sizeof(double) * 2 * n, o_dis = o_idx + sizeof(double) * n /* 8n >= 2*4n */,
-                 o_grad = o_dis + sizeof(double) * n;
-    int rc = dev_buf(h, 1, o_grad + sizeof(double) * 2 * n, (void **)&base);
+    Layout L;
+    const size_t o_xy = L.add(sizeof(double) * 2 * n), o_idx = L.add(sizeof(int32_t) * 2 * n),
+                 o_dis = L.add(sizeof(double) * n), o_grad = L.add(sizeof(double) * 2 * n);
+    char *d;
+    int rc = grow(h, h->stage, L.end, &d);
     if (rc) return rc;
-    CK(cudaMemcpyAsync(base + o_xy, xy, sizeof(double) * 2 * n, cudaMemcpyHostToDevice, h->stream));
-    MapView v;
-    v.cells = s.cells; v.H = s.H; v.W = s.W; v.res = s.res; v.ox = s.ox; v.oy = s.oy; v.inv_res = 1.0 / s.res;
-    v.blocked = s.blocked;
-    k_query<<<(n + 127) / 128, 128, 0, h->stream>>>(v, n, (const double *)(base + o_xy), (int32_t *)(base + o_idx),
-                                                    (double *)(base + o_dis), (double *)(base + o_grad));
+    CK(cudaMemcpyAsync(d + o_xy, xy, sizeof(double) * 2 * n, cudaMemcpyHostToDevice, h->stream));
+    k_query<<<(n + 127) / 128, 128, 0, h->stream>>>(map_view(h->slots[slot]), n, (const double *)(d + o_xy),
+                                                    (int32_t *)(d + o_idx), (double *)(d + o_dis), (double *)(d + o_grad));
     h->launches++;
     CK(cudaGetLastError());
-    CK(cudaMemcpyAsync(idx, base + o_idx, sizeof(int32_t) * 2 * n, cudaMemcpyDeviceToHost, h->stream));
-    CK(cudaMemcpyAsync(dis, base + o_dis, sizeof(double) * n, cudaMemcpyDeviceToHost, h->stream));
-    CK(cudaMemcpyAsync(grad, base + o_grad, sizeof(double) * 2 * n, cudaMemcpyDeviceToHost, h->stream));
+    CK(cudaMemcpyAsync(idx, d + o_idx, sizeof(int32_t) * 2 * n, cudaMemcpyDeviceToHost, h->stream));
+    CK(cudaMemcpyAsync(dis, d + o_dis, sizeof(double) * n, cudaMemcpyDeviceToHost, h->stream));
+    CK(cudaMemcpyAsync(grad, d + o_grad, sizeof(double) * 2 * n, cudaMemcpyDeviceToHost, h->stream));
     CK(cudaStreamSynchronize(h->stream));
     return NEO_OK;
 }
@@ -948,14 +954,13 @@ static int check_problem(neo_handle *h, int B, int M)
 static int check_map_ids(neo_handle *h, int B, const int32_t *map_ids, const char *who)
 {
     if (!map_ids) {
-        if (!h->slots[0].cells) { h->err = std::string(who) + ": map_ids is NULL and slot 0 holds no map"; return NEO_ERR_INVALID; }
+        if (!h->slots[0].cells) return fail(h, std::string(who) + ": map_ids is NULL and slot 0 holds no map");
         return NEO_OK;
     }
     for (int i = 0; i < B; i++)
-        if (map_ids[i] < 0 || map_ids[i] >= (int)h->slots.size() || !h->slots[map_ids[i]].cells) {
-            h->err = std::string(who) + ": map id " + std::to_string(map_ids[i]) + " (problem " + std::to_string(i) + ") refers to an empty slot";
-            return NEO_ERR_INVALID;
-        }
+        if (map_ids[i] < 0 || map_ids[i] >= (int)h->slots.size() || !h->slots[map_ids[i]].cells)
+            return fail(h, std::string(who) + ": map id " + std::to_string(map_ids[i]) + " (problem " + std::to_string(i) +
+                               ") refers to an empty slot");
     return NEO_OK;
 }
 
@@ -964,90 +969,110 @@ static size_t smem_bytes(int M, int TL = 32, bool one_block = false, int wpc = W
     return sizeof(double) * (size_t)tile_mem_doubles(M, TL, one_block) * wpc * (32 / TL);
 }
 
+// sets the kernel's dynamic shared memory and returns in *grid the CTAs for `items` work items at per_cta a CTA, no
+// more than are resident on the device at once (the kernels loop over the rest)
 template <typename K>
-static int prep_kernel(neo_handle *h, K kernel, size_t smem, int *ctas_per_sm, int wpc = WARPS_PER_CTA)
+static int launch_grid(neo_handle *h, K kernel, size_t smem, int wpc, size_t items, size_t per_cta, int *grid)
 {
     CK(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     int occ = 0;
     CK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, kernel, wpc * 32, smem));
     if (occ < 1) return fail(h, "kernel does not fit on an SM");
-    *ctas_per_sm = occ;
+    const size_t need = (items + per_cta - 1) / per_cta, resident = (size_t)occ * h->sm_count;
+    *grid = (int)(need < resident ? need : resident);
     return NEO_OK;
 }
+
+// lanes per problem when short trajectories share a warp: n = 3M - 2 <= 8 for M <= 3, <= 16 for M = 4
+constexpr int shared_lanes(int M) { return M <= 3 ? 8 : 16; }
 
 // lanes per problem: M >= 5 needs the warp (n > 16); short trajectories share a warp once the batch is large enough to
 // fill the machine with several problems per warp (below that, one problem per warp has the shorter evaluation)
 static int tile_lanes(const neo_handle *h, int B, int M)
 {
     if (M > 4) return 32;
-    const int small = M <= 3 ? 8 : 16;
-    if (h->tile) return h->tile == 32 ? 32 : small;
-    return B >= NEO_TILE_MIN_PROBLEMS ? small : 32;
+    if (h->tile) return h->tile == 32 ? 32 : shared_lanes(M);
+    return B >= NEO_TILE_MIN_PROBLEMS ? shared_lanes(M) : 32;
 }
 
-typedef void (*OptKernel)(const DevParams, const OptArgs);
-template <int MODE, int MC, int TL, int MINB>
-static OptKernel pick_optimize(bool grouped, int *wpc)
+// The kernels of one piece count and lane count. One instantiation per supported piece count (loops over pieces/nodes
+// unroll: 1.27x); sampling schedule (minco_tile.cuh) by trajectory length. Every k_optimize variant is sized for 12
+// warps per SM (168 registers, no spills: config 5 38.7 -> 33.2 ms against 8 warps) and exists twice: three CTAs of 4
+// warps per SM (small batches: spread over all SMs, nobody waits) and ONE CTA of 12 warps whose warps leave the
+// evaluation site in groups of nine, sharing their instruction fetches (config 4 33.9 -> 26.4 ms, config 5 33.2 -> 30.5
+// ms, neutral at 2,048 problems).
+struct Variant {
+    void (*opt)(const DevParams, const OptArgs) = nullptr;
+    int opt_wpc = WARPS_PER_CTA;     // warps per CTA of opt
+    void (*eval)(const DevParams, const EvalArgs) = nullptr;
+};
+
+template <int MODE, int MC, int TL>
+static Variant kernels(bool grouped)
 {
-    if (grouped) { *wpc = 4 * MINB; return k_optimize<MODE, MC, TL, 1, 4 * MINB>; }
-    return k_optimize<MODE, MC, TL, MINB, WARPS_PER_CTA>;
+    Variant v;
+    v.eval = k_eval<MODE, MC, TL>;
+    if (grouped) { v.opt = k_optimize<MODE, MC, TL, 1, 3 * WARPS_PER_CTA>; v.opt_wpc = 3 * WARPS_PER_CTA; }
+    else v.opt = k_optimize<MODE, MC, TL, 3, WARPS_PER_CTA>;
+    return v;
+}
+
+// TL: tile_lanes; only M <= 4 has shared-tile kernels (one staging block per tile)
+template <int MC>
+static Variant variant(int TL, bool grouped)
+{
+    if constexpr (MC > 4) return kernels<SAMPLE_ALL_PIECES, MC, 32>(grouped);
+    else return TL < 32 ? kernels<SAMPLE_BY_PIECE_STAGED, MC, shared_lanes(MC)>(grouped) : kernels<SAMPLE_BY_PIECE, MC, 32>(grouped);
+}
+
+static Variant pick_variant(int M, int TL, bool grouped)
+{
+    switch (M) {
+#ifndef NEO_FAST_BUILD      // development builds (-DNEO_FAST_BUILD) instantiate M = 3 only
+        case 2: return variant<2>(TL, grouped);
+        case 4: return variant<4>(TL, grouped);
+        case 5: return variant<5>(TL, grouped);
+        case 6: return variant<6>(TL, grouped);
+        case 7: return variant<7>(TL, grouped);
+        case 8: return variant<8>(TL, grouped);
+        case 9: return variant<9>(TL, grouped);
+        case 10: return variant<10>(TL, grouped);
+#endif
+        case 3: return variant<3>(TL, grouped);
+        default: return Variant();
+    }
 }
 
 static int launch_optimize(neo_handle *h, OptArgs a, cudaStream_t st)
 {
-    int occ;
-    // kernel variant: lanes per problem (tile_lanes) and sampling schedule (minco_tile.cuh) by trajectory length; one
-    // instantiation per supported piece count (loops over pieces/nodes unroll: 1.27x). Every variant is sized for 12 warps
-    // per SM (168 registers, no spills: config 5 38.7 -> 33.2 ms against 8 warps) and exists twice: three CTAs of 4 warps
-    // per SM (small batches: spread over all SMs, nobody waits) and ONE CTA of 12 warps whose warps leave the evaluation
-    // site in groups of nine, sharing their instruction fetches (config 4 33.9 -> 26.4 ms, config 5 33.2 -> 30.5 ms,
-    // neutral at 2,048 problems).
-    void (*kern)(const DevParams, const OptArgs) = nullptr;
     const int TL = tile_lanes(h, a.B, a.M);
-    const bool staged = TL < 32;        // shared tiles: one staging block per tile (shared memory is what limits occupancy)
     bool grouped = TL < 32 || a.B >= NEO_GROUPED_MIN_PROBLEMS;
     if (h->grouped >= 0) grouped = h->grouped != 0;
-    int wpc = WARPS_PER_CTA;
-#define NEO_PICK(MODE, MC, TLV, MINB) pick_optimize<MODE, MC, TLV, MINB>(grouped, &wpc)
-#define NEO_KW(MODE, MC) NEO_PICK(MODE, MC, 32, 3)
-    switch (a.M) {
-#ifndef NEO_FAST_BUILD      // development builds (-DNEO_FAST_BUILD) instantiate M = 3 only
-        case 2: kern = TL == 8 ? NEO_PICK(SAMPLE_BY_PIECE_STAGED, 2, 8, 3) : NEO_KW(SAMPLE_BY_PIECE, 2); break;
-        case 4: kern = TL == 16 ? NEO_PICK(SAMPLE_BY_PIECE_STAGED, 4, 16, 3) : NEO_KW(SAMPLE_BY_PIECE, 4); break;
-        case 5: kern = NEO_KW(SAMPLE_ALL_PIECES, 5); break;
-        case 6: kern = NEO_KW(SAMPLE_ALL_PIECES, 6); break;
-        case 7: kern = NEO_KW(SAMPLE_ALL_PIECES, 7); break;
-        case 8: kern = NEO_KW(SAMPLE_ALL_PIECES, 8); break;
-        case 9: kern = NEO_KW(SAMPLE_ALL_PIECES, 9); break;
-        case 10: kern = NEO_KW(SAMPLE_ALL_PIECES, 10); break;
-#endif
-        case 3: kern = TL == 8 ? NEO_PICK(SAMPLE_BY_PIECE_STAGED, 3, 8, 3) : NEO_KW(SAMPLE_BY_PIECE, 3); break;
-        default: return fail(h, "M must be in [2, NEO_MAX_PIECES]");
-    }
-#undef NEO_KW
-#undef NEO_PICK
+    const Variant v = pick_variant(a.M, TL, grouped);
+    if (!v.opt) return fail(h, "M must be in [2, NEO_MAX_PIECES]");
+    const int wpc = v.opt_wpc;
     a.bus_q = h->group_warps > 0 ? h->group_warps : 3 * wpc / 4;        // 12 warps: 9 (26.4 ms; 8: 26.5, 10: 26.9, 6: 27.9, 12: 30.2)
     if (a.bus_q > wpc) a.bus_q = wpc;
-    const size_t smem = smem_bytes(a.M, TL, staged, wpc);
-    int rc = prep_kernel(h, kern, smem, &occ, wpc);
-    if (rc) return rc;
+    // shared tiles: one staging block per tile (shared memory is what limits occupancy)
+    const size_t smem = smem_bytes(a.M, TL, TL < 32, wpc);
     const size_t tasks = (size_t)a.B * a.max_attempts, n = 3 * a.M - 2;
-    const size_t per_cta = (size_t)wpc * (32 / TL);
-    const size_t need = (tasks + per_cta - 1) / per_cta;
-    const int grid = (int)(need < (size_t)occ * h->sm_count ? need : (size_t)occ * h->sm_count);
-    // per-task scratch records + per-problem state word (library-owned, grow-only)
-    char *base;
-    const size_t o_x = 0, o_c = o_x + sizeof(double) * tasks * n, o_w = o_c + sizeof(double) * tasks * 4,
-                 o_i = o_w + sizeof(long long) * tasks * 4, o_p = o_i + sizeof(int32_t) * tasks * 4,
-                 total = o_p + sizeof(unsigned) * a.B;
-    if ((rc = dev_buf(h, 6, total, (void **)&base))) return rc;
-    a.t_x = (double *)(base + o_x); a.t_costs = (double *)(base + o_c); a.t_work = (long long *)(base + o_w);
-    a.t_info = (int32_t *)(base + o_i); a.p_state = (unsigned *)(base + o_p);
+    int grid;
+    int rc = launch_grid(h, v.opt, smem, wpc, tasks, (size_t)wpc * (32 / TL), &grid);
+    if (rc) return rc;
+    // per-task scratch records + per-problem state word
+    Layout L;
+    const size_t o_x = L.add(sizeof(double) * tasks * n), o_c = L.add(sizeof(double) * tasks * 4),
+                 o_w = L.add(sizeof(long long) * tasks * 4), o_i = L.add(sizeof(int32_t) * tasks * 4),
+                 o_p = L.add(sizeof(unsigned) * a.B);
+    char *s;
+    if ((rc = grow(h, h->opt_scratch, L.end, &s))) return rc;
+    a.t_x = (double *)(s + o_x); a.t_costs = (double *)(s + o_c); a.t_work = (long long *)(s + o_w);
+    a.t_info = (int32_t *)(s + o_i); a.p_state = (unsigned *)(s + o_p);
     a.maps = h->d_maps;
     a.counter = h->d_counter;
     CK(cudaMemsetAsync(h->d_counter, 0, sizeof(unsigned int), st));
     CK(cudaMemsetAsync(a.p_state, 0, sizeof(unsigned) * a.B, st));
-    kern<<<grid, wpc * 32, smem, st>>>(dev_params(h->cfg), a);
+    v.opt<<<grid, wpc * 32, smem, st>>>(dev_params(h->cfg), a);
     h->launches++;
     CK(cudaGetLastError());
     return NEO_OK;
@@ -1055,30 +1080,14 @@ static int launch_optimize(neo_handle *h, OptArgs a, cudaStream_t st)
 
 static int launch_eval(neo_handle *h, EvalArgs a, cudaStream_t st)
 {
-    int occ;
-    void (*kern)(const DevParams, const EvalArgs) = nullptr;
     const int TL = tile_lanes(h, a.B, a.M);
-    switch (a.M) {
-#ifndef NEO_FAST_BUILD
-        case 2: kern = TL == 8 ? k_eval<SAMPLE_BY_PIECE_STAGED, 2, 8> : k_eval<SAMPLE_BY_PIECE, 2, 32>; break;
-        case 4: kern = TL == 16 ? k_eval<SAMPLE_BY_PIECE_STAGED, 4, 16> : k_eval<SAMPLE_BY_PIECE, 4, 32>; break;
-        case 5: kern = k_eval<SAMPLE_ALL_PIECES, 5, 32>; break;
-        case 6: kern = k_eval<SAMPLE_ALL_PIECES, 6, 32>; break;
-        case 7: kern = k_eval<SAMPLE_ALL_PIECES, 7, 32>; break;
-        case 8: kern = k_eval<SAMPLE_ALL_PIECES, 8, 32>; break;
-        case 9: kern = k_eval<SAMPLE_ALL_PIECES, 9, 32>; break;
-        case 10: kern = k_eval<SAMPLE_ALL_PIECES, 10, 32>; break;
-#endif
-        case 3: kern = TL == 8 ? k_eval<SAMPLE_BY_PIECE_STAGED, 3, 8> : k_eval<SAMPLE_BY_PIECE, 3, 32>; break;
-        default: return fail(h, "M must be in [2, NEO_MAX_PIECES]");
-    }
+    const auto kern = pick_variant(a.M, TL, false).eval;
+    if (!kern) return fail(h, "M must be in [2, NEO_MAX_PIECES]");
     // evaluator-only shared memory (no optimizer state): half of k_optimize's per tile, so registers decide the occupancy
     const size_t smem = sizeof(double) * (size_t)eval_mem_doubles(a.M, TL, TL < 32) * WARPS_PER_CTA * (32 / TL);
-    int rc = prep_kernel(h, kern, smem, &occ);
+    int grid;
+    int rc = launch_grid(h, kern, smem, WARPS_PER_CTA, a.B, WARPS_PER_CTA * (32 / TL), &grid);
     if (rc) return rc;
-    const int per_cta = WARPS_PER_CTA * (32 / TL);
-    const int need = (a.B + per_cta - 1) / per_cta;
-    const int grid = need < occ * h->sm_count ? need : occ * h->sm_count;
     a.maps = h->d_maps;
     kern<<<grid, WARPS_PER_CTA * 32, smem, st>>>(dev_params(h->cfg), a);
     h->launches++;
@@ -1086,37 +1095,28 @@ static int launch_eval(neo_handle *h, EvalArgs a, cudaStream_t st)
     return NEO_OK;
 }
 
-// byte-offset bump allocator over one staging buffer
-struct Carver {
-    char *base;
-    size_t off = 0;
-    template <typename T>
-    T *take(size_t count)
-    {
-        off = (off + 255) & ~(size_t)255;
-        T *p = base ? (T *)(base + off) : nullptr;
-        off += sizeof(T) * count;
-        return p;
-    }
-};
-
 // ---------------------------------------------------------------------------------------------------------
 // eval
 // ---------------------------------------------------------------------------------------------------------
+// the argument checks of neo_eval and neo_eval_dev; `arrays`: the required arrays are all non-null
+static int eval_check(neo_handle *h, const char *who, int B, int M, bool arrays)
+{
+    const int rc = check_problem(h, B, M);
+    if (rc) return rc;
+    if (!arrays) return fail(h, std::string(who) + ": null pointer");
+    return NEO_OK;
+}
+
 extern "C" int neo_eval_dev(neo_handle *h, int B, int M, const double *x, const double *head, const double *tail,
                             const int32_t *map_ids, double *costs, double *grad, int32_t *status, double *coeffs,
                             double *ts, void *stream)
 {
     if (!h) return NEO_ERR_INVALID;
     std::lock_guard<std::mutex> g(h->mu);
-    int rc = check_problem(h, B, M);
-    if (rc) return rc;
-    if (!x || !head || !tail || !costs || !grad || !status) return fail(h, "neo_eval_dev: null pointer");
-    if (B == 0) return NEO_OK;
+    const int rc = eval_check(h, "neo_eval_dev", B, M, x && head && tail && costs && grad && status);
+    if (rc || B == 0) return rc;
     CK(cudaSetDevice(h->device));
-    EvalArgs a;
-    a.B = B; a.M = M; a.x = x; a.head = head; a.tail = tail; a.map_ids = map_ids;
-    a.costs = costs; a.grad = grad; a.status = status; a.coeffs = coeffs; a.ts = ts; a.maps = nullptr;
+    const EvalArgs a = {B, M, x, head, tail, map_ids, nullptr, costs, grad, coeffs, ts, status};
     return launch_eval(h, a, stream ? (cudaStream_t)stream : h->stream);
 }
 
@@ -1125,45 +1125,38 @@ extern "C" int neo_eval(neo_handle *h, int B, int M, const double *x, const doub
 {
     if (!h) return NEO_ERR_INVALID;
     std::lock_guard<std::mutex> g(h->mu);
-    int rc = check_problem(h, B, M);
-    if (rc) return rc;
-    if (!x || !head || !tail || !costs || !grad || !status) return fail(h, "neo_eval: null pointer");
-    if (B == 0) return NEO_OK;
+    int rc = eval_check(h, "neo_eval", B, M, x && head && tail && costs && grad && status);
+    if (rc || B == 0) return rc;
     if ((rc = check_map_ids(h, B, map_ids, "neo_eval"))) return rc;
     CK(cudaSetDevice(h->device));
     const size_t n = 3 * M - 2, N2 = 12 * M, b = B;
-    for (int pass = 0; pass < 2; pass++) {
-        Carver c{pass ? (char *)h->bufs[2].p : nullptr};
-        double *d_x = c.take<double>(b * n), *d_head = c.take<double>(b * 6), *d_tail = c.take<double>(b * 6);
-        int32_t *d_ids = c.take<int32_t>(b);
-        double *d_costs = c.take<double>(b * 4), *d_grad = c.take<double>(b * n), *d_coeffs = c.take<double>(b * N2),
-               *d_ts = c.take<double>(b * M);
-        int32_t *d_status = c.take<int32_t>(b);
-        if (!pass) {
-            void *p;
-            if ((rc = dev_buf(h, 2, c.off + 256, &p))) return rc;
-            continue;
-        }
-        cudaStream_t st = h->stream;
-        CK(cudaMemcpyAsync(d_x, x, sizeof(double) * b * n, cudaMemcpyHostToDevice, st));
-        CK(cudaMemcpyAsync(d_head, head, sizeof(double) * b * 6, cudaMemcpyHostToDevice, st));
-        CK(cudaMemcpyAsync(d_tail, tail, sizeof(double) * b * 6, cudaMemcpyHostToDevice, st));
-        if (map_ids) CK(cudaMemcpyAsync(d_ids, map_ids, sizeof(int32_t) * b, cudaMemcpyHostToDevice, st));
-        EvalArgs a;
-        a.B = B; a.M = M; a.x = d_x; a.head = d_head; a.tail = d_tail; a.map_ids = map_ids ? d_ids : nullptr;
-        a.costs = d_costs; a.grad = d_grad; a.status = d_status; a.coeffs = coeffs ? d_coeffs : nullptr;
-        a.ts = ts ? d_ts : nullptr; a.maps = nullptr;
-        CK(cudaEventRecord(h->ev0, st));
-        if ((rc = launch_eval(h, a, st))) return rc;
-        CK(cudaEventRecord(h->ev1, st));
-        CK(cudaMemcpyAsync(costs, d_costs, sizeof(double) * b * 4, cudaMemcpyDeviceToHost, st));
-        CK(cudaMemcpyAsync(grad, d_grad, sizeof(double) * b * n, cudaMemcpyDeviceToHost, st));
-        CK(cudaMemcpyAsync(status, d_status, sizeof(int32_t) * b, cudaMemcpyDeviceToHost, st));
-        if (coeffs) CK(cudaMemcpyAsync(coeffs, d_coeffs, sizeof(double) * b * N2, cudaMemcpyDeviceToHost, st));
-        if (ts) CK(cudaMemcpyAsync(ts, d_ts, sizeof(double) * b * M, cudaMemcpyDeviceToHost, st));
-        CK(cudaStreamSynchronize(st));
-        CK(cudaEventElapsedTime(&h->last_ms, h->ev0, h->ev1));
-    }
+    Layout L;
+    const size_t o_x = L.add(sizeof(double) * b * n), o_head = L.add(sizeof(double) * b * 6),
+                 o_tail = L.add(sizeof(double) * b * 6), o_ids = L.add(sizeof(int32_t) * b),
+                 o_costs = L.add(sizeof(double) * b * 4), o_grad = L.add(sizeof(double) * b * n),
+                 o_coeffs = L.add(sizeof(double) * b * N2), o_ts = L.add(sizeof(double) * b * M),
+                 o_status = L.add(sizeof(int32_t) * b);
+    char *d;
+    if ((rc = grow(h, h->stage, L.end, &d))) return rc;
+    cudaStream_t st = h->stream;
+    CK(cudaMemcpyAsync(d + o_x, x, sizeof(double) * b * n, cudaMemcpyHostToDevice, st));
+    CK(cudaMemcpyAsync(d + o_head, head, sizeof(double) * b * 6, cudaMemcpyHostToDevice, st));
+    CK(cudaMemcpyAsync(d + o_tail, tail, sizeof(double) * b * 6, cudaMemcpyHostToDevice, st));
+    if (map_ids) CK(cudaMemcpyAsync(d + o_ids, map_ids, sizeof(int32_t) * b, cudaMemcpyHostToDevice, st));
+    const EvalArgs a = {B, M, (const double *)(d + o_x), (const double *)(d + o_head), (const double *)(d + o_tail),
+                        map_ids ? (const int32_t *)(d + o_ids) : nullptr, nullptr, (double *)(d + o_costs),
+                        (double *)(d + o_grad), coeffs ? (double *)(d + o_coeffs) : nullptr,
+                        ts ? (double *)(d + o_ts) : nullptr, (int32_t *)(d + o_status)};
+    CK(cudaEventRecord(h->ev0, st));
+    if ((rc = launch_eval(h, a, st))) return rc;
+    CK(cudaEventRecord(h->ev1, st));
+    CK(cudaMemcpyAsync(costs, d + o_costs, sizeof(double) * b * 4, cudaMemcpyDeviceToHost, st));
+    CK(cudaMemcpyAsync(grad, d + o_grad, sizeof(double) * b * n, cudaMemcpyDeviceToHost, st));
+    CK(cudaMemcpyAsync(status, d + o_status, sizeof(int32_t) * b, cudaMemcpyDeviceToHost, st));
+    if (coeffs) CK(cudaMemcpyAsync(coeffs, d + o_coeffs, sizeof(double) * b * N2, cudaMemcpyDeviceToHost, st));
+    if (ts) CK(cudaMemcpyAsync(ts, d + o_ts, sizeof(double) * b * M, cudaMemcpyDeviceToHost, st));
+    CK(cudaStreamSynchronize(st));
+    CK(cudaEventElapsedTime(&h->last_ms, h->ev0, h->ev1));
     return NEO_OK;
 }
 
@@ -1194,34 +1187,44 @@ extern "C" int neo_T2tau(const neo_config *cfg, int n, const double *ts, double 
 }
 
 // internal: device pointers, tau-form inputs
-struct TraceDev {
-    int cap = 0;
-    double *x = nullptr, *f = nullptr, *g = nullptr, *costs = nullptr;
-    int32_t *status = nullptr, *len = nullptr;
-};
-
-static int optimize_dev_impl(neo_handle *h, int B, int M, const double *x0, const int32_t *x0_status, const double *head,
-                             const double *tail, const int32_t *map_ids, const double *retry_q, const double *retry_tau,
-                             int retry_status, int max_attempts, const neo_result *out, cudaStream_t st,
-                             const TraceDev *tr = nullptr)
+// the arrays of a neo_result, each with its bytes per problem of M pieces
+template <typename F>
+static void result_fields(neo_result &r, int M, F f)
 {
-    OptArgs a;
-    a.trace_cap = tr ? tr->cap : 0;
-    a.tr_x = tr ? tr->x : nullptr; a.tr_f = tr ? tr->f : nullptr; a.tr_g = tr ? tr->g : nullptr;
-    a.tr_costs = tr ? tr->costs : nullptr; a.tr_status = tr ? tr->status : nullptr; a.tr_len = tr ? tr->len : nullptr;
+    const size_t n = 3 * M - 2;
+    f(r.x, sizeof(double) * n); f(r.ts, sizeof(double) * M); f(r.coeffs, sizeof(double) * 12 * M);
+    f(r.costs, sizeof(double) * 4); f(r.status, sizeof(int32_t)); f(r.ok, sizeof(int32_t)); f(r.attempt, sizeof(int32_t));
+    f(r.nit, sizeof(int32_t)); f(r.runs, sizeof(int32_t)); f(r.nfev, sizeof(int32_t)); f(r.work, sizeof(int64_t) * 4);
+}
+
+// the argument checks of neo_optimize_dev and neo_optimize(_trace); `inputs` / `retry`: the caller's required input
+// arrays / its retry arrays are all non-null
+static int optimize_check(neo_handle *h, const char *who, int B, int M, bool inputs, int max_attempts, bool retry,
+                          const neo_result *o)
+{
+    const int rc = check_problem(h, B, M);
+    if (rc) return rc;
+    if (!inputs || !o || !o->x || !o->ts || !o->coeffs || !o->costs || !o->status || !o->ok || !o->attempt || !o->nit ||
+        !o->runs || !o->nfev)
+        return fail(h, std::string(who) + ": null pointer");
+    if (max_attempts < 1 || max_attempts > NEO_MAX_ATTEMPTS) return fail(h, "max_attempts out of range");
+    if (max_attempts > 1 && !retry) return fail(h, "retry arrays required when max_attempts > 1");
+    return NEO_OK;
+}
+
+// OptArgs of one launch from device pointers and tau-form inputs; launch_optimize adds its scratch, the maps and the queue
+static OptArgs opt_args(int B, int M, const double *x0, const int32_t *x0_status, const double *head, const double *tail,
+                        const int32_t *map_ids, const double *retry_q, const double *retry_tau, int retry_status,
+                        int max_attempts, const neo_result &out)
+{
+    OptArgs a = {};
     a.B = B; a.M = M; a.max_attempts = max_attempts;
     a.x0 = x0; a.x0_status = x0_status; a.head = head; a.tail = tail; a.map_ids = map_ids;
     a.retry_q = retry_q; a.retry_tau = retry_tau; a.retry_status = retry_status;
-    a.maps = nullptr; a.counter = nullptr;
-    a.x = out->x; a.ts = out->ts; a.coeffs = out->coeffs; a.costs = out->costs;
-    a.status = out->status; a.ok = out->ok; a.attempt = out->attempt; a.nit = out->nit; a.runs = out->runs;
-    a.nfev = out->nfev; a.work = (long long *)out->work;
-    return launch_optimize(h, a, st);
-}
-
-static int result_complete(const neo_result *o)
-{
-    return o && o->x && o->ts && o->coeffs && o->costs && o->status && o->ok && o->attempt && o->nit && o->runs && o->nfev;
+    a.x = out.x; a.ts = out.ts; a.coeffs = out.coeffs; a.costs = out.costs;
+    a.status = out.status; a.ok = out.ok; a.attempt = out.attempt; a.nit = out.nit; a.runs = out.runs;
+    a.nfev = out.nfev; a.work = (long long *)out.work;
+    return a;
 }
 
 // Device-pointer entry. Inputs are in tau form (x0 = [q0, map_T2tau(ts0)], retry_tau = map_T2tau(retry_ts))
@@ -1233,15 +1236,12 @@ extern "C" int neo_optimize_dev(neo_handle *h, int B, int M, const double *x0, c
 {
     if (!h) return NEO_ERR_INVALID;
     std::lock_guard<std::mutex> g(h->mu);
-    int rc = check_problem(h, B, M);
-    if (rc) return rc;
-    if (!x0 || !head || !tail || !result_complete(out)) return fail(h, "neo_optimize_dev: null pointer");
-    if (max_attempts < 1 || max_attempts > NEO_MAX_ATTEMPTS) return fail(h, "max_attempts out of range");
-    if (max_attempts > 1 && (!retry_q || !retry_tau)) return fail(h, "retry arrays required when max_attempts > 1");
-    if (B == 0) return NEO_OK;
+    const int rc = optimize_check(h, "neo_optimize_dev", B, M, x0 && head && tail, max_attempts, retry_q && retry_tau, out);
+    if (rc || B == 0) return rc;
     CK(cudaSetDevice(h->device));
-    return optimize_dev_impl(h, B, M, x0, x0_status, head, tail, map_ids, retry_q, retry_tau, retry_status, max_attempts,
-                             out, stream ? (cudaStream_t)stream : h->stream);
+    return launch_optimize(h, opt_args(B, M, x0, x0_status, head, tail, map_ids, retry_q, retry_tau, retry_status,
+                                       max_attempts, *out),
+                           stream ? (cudaStream_t)stream : h->stream);
 }
 
 struct TraceHost {
@@ -1261,36 +1261,37 @@ static int optimize_host(neo_handle *h, int B, int M, const double *q0, const do
 {
     if (!h) return NEO_ERR_INVALID;
     std::lock_guard<std::mutex> g(h->mu);
-    int rc = check_problem(h, B, M);
+    int rc = optimize_check(h, "neo_optimize", B, M, q0 && ts0 && head && tail, max_attempts, retry_q && retry_ts, out);
     if (rc) return rc;
-    if (!q0 || !ts0 || !head || !tail || !result_complete(out)) return fail(h, "neo_optimize: null pointer");
-    if (max_attempts < 1 || max_attempts > NEO_MAX_ATTEMPTS) return fail(h, "max_attempts out of range");
-    if (max_attempts > 1 && (!retry_q || !retry_ts)) return fail(h, "retry arrays required when max_attempts > 1");
     if (trace && (trace->cap < 1 || !trace->x || !trace->f || !trace->g || !trace->costs || !trace->status || !trace->len))
         return fail(h, "neo_optimize_trace: null trace array");
     if (B == 0) return NEO_OK;
     if ((rc = check_map_ids(h, B, map_ids, "neo_optimize"))) return rc;
     CK(cudaSetDevice(h->device));
-    const size_t n = 3 * M - 2, nq = 2 * (M - 1), N2 = 12 * M, b = B, A1 = max_attempts - 1;
+    const size_t n = 3 * M - 2, nq = 2 * (M - 1), b = B, A1 = max_attempts - 1;
 
-    struct Lay {
-        size_t x0, head, tail, st0, ids, rq, rtau, in_end, x, ts, coeffs, costs, status, ok, attempt, nit, runs, nfev, work, end;
-    } L;
-    {
-        size_t o = 0;
-        auto off = [&](size_t bytes) { o = (o + 255) & ~(size_t)255; const size_t at = o; o += bytes; return at; };
-        L.x0 = off(8 * b * n); L.head = off(8 * b * 6); L.tail = off(8 * b * 6); L.st0 = off(4 * b); L.ids = off(4 * b);
-        L.rtau = off(8 * NEO_MAX_PIECES); L.in_end = off(0); L.rq = off(8 * (b * A1 * nq + 1));
-        L.x = off(8 * b * n); L.ts = off(8 * b * M); L.coeffs = off(8 * b * N2); L.costs = off(8 * b * 4);
-        L.status = off(4 * b); L.ok = off(4 * b); L.attempt = off(4 * b); L.nit = off(4 * b); L.runs = off(4 * b);
-        L.nfev = off(4 * b); L.work = off(8 * b * 4); L.end = off(0);
-    }
+    // the inputs sit at the same offsets in the pinned and in the device staging buffer
+    Layout L;
+    const size_t o_x0 = L.add(sizeof(double) * b * n), o_head = L.add(sizeof(double) * b * 6),
+                 o_tail = L.add(sizeof(double) * b * 6), o_st0 = L.add(sizeof(int32_t) * b),
+                 o_ids = L.add(sizeof(int32_t) * b), o_rtau = L.add(sizeof(double) * NEO_MAX_PIECES), in_end = L.end;
+    // device only: the per-task evaluation trace (test path)
+    Layout D = L;
+    const size_t tasks = b * max_attempts, cap = trace ? trace->cap : 0;
+    const size_t o_tx = D.add(sizeof(double) * tasks * cap * n), o_tg = D.add(sizeof(double) * tasks * cap * n),
+                 o_tf = D.add(sizeof(double) * tasks * cap), o_tc = D.add(sizeof(double) * tasks * cap * 4),
+                 o_tst = D.add(sizeof(int32_t) * tasks * cap), o_tl = D.add(sizeof(int32_t) * tasks);
+    // pinned only: the retry guesses, then the results
+    const size_t o_rq = L.add(sizeof(double) * b * A1 * nq);
+    size_t o_res[11];
+    int fi = 0;
+    result_fields(*out, M, [&](auto &, size_t bytes) { o_res[fi++] = L.add(bytes * b); });
     char *dbase, *hbase;
-    if ((rc = dev_buf(h, 3, L.end, (void **)&dbase))) return rc;
-    if ((rc = pin_buf(h, L.end, (void **)&hbase))) return rc;
+    if ((rc = grow(h, h->stage, D.end, &dbase))) return rc;
+    if ((rc = grow(h, h->pinned, L.end, &hbase))) return rc;
 
-    double *hx0 = (double *)(hbase + L.x0);
-    int32_t *hst = (int32_t *)(hbase + L.st0);
+    double *hx0 = (double *)(hbase + o_x0);
+    int32_t *hst = (int32_t *)(hbase + o_st0);
     const bool timing = h->host_timing;
     auto now = [] { return std::chrono::steady_clock::now(); };
     const auto t_begin = now();
@@ -1314,84 +1315,63 @@ static int optimize_host(neo_handle *h, int B, int M, const double *q0, const do
         }
         if (bad) any_bad_flag.store(1);
     });
-    CK(cudaMemcpyAsync(dbase + L.x0, hbase + L.x0, L.head - L.x0, cudaMemcpyHostToDevice, st));
+    CK(cudaMemcpyAsync(dbase + o_x0, hbase + o_x0, o_head - o_x0, cudaMemcpyHostToDevice, st));
     const bool any_bad = any_bad_flag.load() != 0;
     h->pool.run(b, [&](size_t i0, size_t i1) {
-        memcpy(hbase + L.head + 48 * i0, head + i0 * 6, 48 * (i1 - i0));
-        memcpy(hbase + L.tail + 48 * i0, tail + i0 * 6, 48 * (i1 - i0));
-        if (map_ids) memcpy(hbase + L.ids + 4 * i0, map_ids + i0, 4 * (i1 - i0));
+        memcpy(hbase + o_head + 48 * i0, head + i0 * 6, 48 * (i1 - i0));
+        memcpy(hbase + o_tail + 48 * i0, tail + i0 * 6, 48 * (i1 - i0));
+        if (map_ids) memcpy(hbase + o_ids + 4 * i0, map_ids + i0, 4 * (i1 - i0));
     });
-    double *rtau = (double *)(hbase + L.rtau);
+    double *rtau = (double *)(hbase + o_rtau);
     int rstatus = 0;
     if (A1)
         for (int k = 0; k < M; k++) { rtau[k] = 0.0; const int s1 = T2tau_one(&h->cfg, retry_ts[k], &rtau[k]); if (s1) rstatus = s1; }
-    CK(cudaMemcpyAsync(dbase + L.head, hbase + L.head, L.in_end - L.head, cudaMemcpyHostToDevice, st));     // head, tail, st0, ids, retry tau
+    CK(cudaMemcpyAsync(dbase + o_head, hbase + o_head, in_end - o_head, cudaMemcpyHostToDevice, st));     // head, tail, st0, ids, retry tau
     // the retry guesses (the largest input: 4 per problem) stay in the pinned buffer: only the problems that do retry
     // read theirs, through the mapped pointer, when the retry starts
     if (A1)
         h->pool.run(b, [&](size_t i0, size_t i1) {
-            memcpy(hbase + L.rq + 8 * i0 * A1 * nq, retry_q + i0 * A1 * nq, 8 * (i1 - i0) * A1 * nq);
+            memcpy(hbase + o_rq + 8 * i0 * A1 * nq, retry_q + i0 * A1 * nq, 8 * (i1 - i0) * A1 * nq);
         });
     // results: the kernel writes every resolved problem's record straight into the pinned staging buffer (mapped host
     // memory; 0.46 KB per problem, spread over the whole launch), so no device-to-host copy follows the kernel
     char *rbase = nullptr;
     CK(cudaHostGetDevicePointer((void **)&rbase, hbase, 0));
-    neo_result d;
-    d.x = (double *)(rbase + L.x); d.ts = (double *)(rbase + L.ts); d.coeffs = (double *)(rbase + L.coeffs);
-    d.costs = (double *)(rbase + L.costs);
-    d.status = (int32_t *)(rbase + L.status); d.ok = (int32_t *)(rbase + L.ok); d.attempt = (int32_t *)(rbase + L.attempt);
-    d.nit = (int32_t *)(rbase + L.nit); d.runs = (int32_t *)(rbase + L.runs); d.nfev = (int32_t *)(rbase + L.nfev);
-    d.work = out->work ? (int64_t *)(rbase + L.work) : nullptr;
-    TraceDev td;
-    size_t tr_tasks = 0;
-    if (trace) {      // test path: the per-task evaluation trace lives in its own device buffer
-        tr_tasks = b * max_attempts;
-        const size_t cap = trace->cap;
-        Carver c{nullptr};
-        for (int pass = 0; pass < 2; pass++) {
-            c.off = 0;
-            td.cap = trace->cap;
-            td.x = c.take<double>(tr_tasks * cap * n); td.g = c.take<double>(tr_tasks * cap * n);
-            td.f = c.take<double>(tr_tasks * cap); td.costs = c.take<double>(tr_tasks * cap * 4);
-            td.status = c.take<int32_t>(tr_tasks * cap); td.len = c.take<int32_t>(tr_tasks);
-            if (!pass) { void *p; if ((rc = dev_buf(h, 8, c.off + 256, &p))) return rc; c.base = (char *)p; }
-        }
-        CK(cudaMemsetAsync(td.len, 0, sizeof(int32_t) * tr_tasks, st));
+    neo_result d = *out;
+    fi = 0;
+    result_fields(d, M, [&](auto &p, size_t) { if (p) p = (std::decay_t<decltype(p)>)(rbase + o_res[fi]); fi++; });
+    OptArgs a = opt_args(B, M, (const double *)(dbase + o_x0), any_bad ? (const int32_t *)(dbase + o_st0) : nullptr,
+                         (const double *)(dbase + o_head), (const double *)(dbase + o_tail),
+                         map_ids ? (const int32_t *)(dbase + o_ids) : nullptr, A1 ? (const double *)(rbase + o_rq) : nullptr,
+                         A1 ? (const double *)(dbase + o_rtau) : nullptr, rstatus, max_attempts, d);
+    if (trace) {
+        a.trace_cap = trace->cap;
+        a.tr_x = (double *)(dbase + o_tx); a.tr_g = (double *)(dbase + o_tg); a.tr_f = (double *)(dbase + o_tf);
+        a.tr_costs = (double *)(dbase + o_tc); a.tr_status = (int32_t *)(dbase + o_tst); a.tr_len = (int32_t *)(dbase + o_tl);
+        CK(cudaMemsetAsync(a.tr_len, 0, sizeof(int32_t) * tasks, st));
     }
     const auto t_staged = now();
     CK(cudaEventRecord(h->ev0, st));
-    rc = optimize_dev_impl(h, B, M, (const double *)(dbase + L.x0), any_bad ? (const int32_t *)(dbase + L.st0) : nullptr,
-                           (const double *)(dbase + L.head), (const double *)(dbase + L.tail),
-                           map_ids ? (const int32_t *)(dbase + L.ids) : nullptr, A1 ? (const double *)(rbase + L.rq) : nullptr,
-                           A1 ? (const double *)(dbase + L.rtau) : nullptr, rstatus, max_attempts, &d, st, trace ? &td : nullptr);
-    if (rc) return rc;
+    if ((rc = launch_optimize(h, a, st))) return rc;
     CK(cudaEventRecord(h->ev1, st));
     if (trace) {
-        const size_t cap = trace->cap;
-        CK(cudaMemcpyAsync(trace->x, td.x, 8 * tr_tasks * cap * n, cudaMemcpyDeviceToHost, st));
-        CK(cudaMemcpyAsync(trace->g, td.g, 8 * tr_tasks * cap * n, cudaMemcpyDeviceToHost, st));
-        CK(cudaMemcpyAsync(trace->f, td.f, 8 * tr_tasks * cap, cudaMemcpyDeviceToHost, st));
-        CK(cudaMemcpyAsync(trace->costs, td.costs, 8 * tr_tasks * cap * 4, cudaMemcpyDeviceToHost, st));
-        CK(cudaMemcpyAsync(trace->status, td.status, 4 * tr_tasks * cap, cudaMemcpyDeviceToHost, st));
-        CK(cudaMemcpyAsync(trace->len, td.len, 4 * tr_tasks, cudaMemcpyDeviceToHost, st));
+        CK(cudaMemcpyAsync(trace->x, a.tr_x, sizeof(double) * tasks * cap * n, cudaMemcpyDeviceToHost, st));
+        CK(cudaMemcpyAsync(trace->g, a.tr_g, sizeof(double) * tasks * cap * n, cudaMemcpyDeviceToHost, st));
+        CK(cudaMemcpyAsync(trace->f, a.tr_f, sizeof(double) * tasks * cap, cudaMemcpyDeviceToHost, st));
+        CK(cudaMemcpyAsync(trace->costs, a.tr_costs, sizeof(double) * tasks * cap * 4, cudaMemcpyDeviceToHost, st));
+        CK(cudaMemcpyAsync(trace->status, a.tr_status, sizeof(int32_t) * tasks * cap, cudaMemcpyDeviceToHost, st));
+        CK(cudaMemcpyAsync(trace->len, a.tr_len, sizeof(int32_t) * tasks, cudaMemcpyDeviceToHost, st));
     }
     const auto t_launched = now();
     CK(cudaStreamSynchronize(st));
     const auto t_done = now();
     CK(cudaEventElapsedTime(&h->last_ms, h->ev0, h->ev1));
     h->pool.run(b, [&](size_t i0, size_t i1) {
-        const size_t c = i1 - i0;
-        memcpy(out->x + i0 * n, hbase + L.x + 8 * i0 * n, 8 * c * n);
-        memcpy(out->ts + i0 * M, hbase + L.ts + 8 * i0 * M, 8 * c * M);
-        memcpy(out->coeffs + i0 * N2, hbase + L.coeffs + 8 * i0 * N2, 8 * c * N2);
-        memcpy(out->costs + i0 * 4, hbase + L.costs + 32 * i0, 32 * c);
-        memcpy(out->status + i0, hbase + L.status + 4 * i0, 4 * c);
-        memcpy(out->ok + i0, hbase + L.ok + 4 * i0, 4 * c);
-        memcpy(out->attempt + i0, hbase + L.attempt + 4 * i0, 4 * c);
-        memcpy(out->nit + i0, hbase + L.nit + 4 * i0, 4 * c);
-        memcpy(out->runs + i0, hbase + L.runs + 4 * i0, 4 * c);
-        memcpy(out->nfev + i0, hbase + L.nfev + 4 * i0, 4 * c);
-        if (out->work) memcpy(out->work + i0 * 4, hbase + L.work + 32 * i0, 32 * c);
+        int fi = 0;
+        result_fields(*out, M, [&](auto &p, size_t bytes) {
+            if (p) memcpy((char *)p + bytes * i0, hbase + o_res[fi] + bytes * i0, bytes * (i1 - i0));
+            fi++;
+        });
     });
     if (timing) {
         auto ms = [](std::chrono::steady_clock::time_point a, std::chrono::steady_clock::time_point b2) { return std::chrono::duration<double, std::milli>(b2 - a).count(); };
@@ -1430,31 +1410,27 @@ extern "C" int neo_get_coeffs(neo_handle *h, int B, int M, const double *q, cons
     if (B == 0) return NEO_OK;
     CK(cudaSetDevice(h->device));
     const size_t nq = 2 * (M - 1), N2 = 12 * M, b = B;
-    int rc;
-    for (int pass = 0; pass < 2; pass++) {
-        Carver c{pass ? (char *)h->bufs[4].p : nullptr};
-        double *d_q = c.take<double>(b * nq), *d_ts = c.take<double>(b * M), *d_head = c.take<double>(b * 6),
-               *d_tail = c.take<double>(b * 6), *d_c = c.take<double>(b * N2);
-        if (!pass) {
-            void *p;
-            if ((rc = dev_buf(h, 4, c.off + 256, &p))) return rc;
-            continue;
-        }
-        cudaStream_t st = h->stream;
-        CK(cudaMemcpyAsync(d_q, q, sizeof(double) * b * nq, cudaMemcpyHostToDevice, st));
-        CK(cudaMemcpyAsync(d_ts, ts, sizeof(double) * b * M, cudaMemcpyHostToDevice, st));
-        CK(cudaMemcpyAsync(d_head, head, sizeof(double) * b * 6, cudaMemcpyHostToDevice, st));
-        CK(cudaMemcpyAsync(d_tail, tail, sizeof(double) * b * 6, cudaMemcpyHostToDevice, st));
-        int occ;
-        if ((rc = prep_kernel(h, k_coeffs, smem_bytes(M), &occ))) return rc;
-        const int need = (B + WARPS_PER_CTA - 1) / WARPS_PER_CTA;
-        const int grid = need < occ * h->sm_count ? need : occ * h->sm_count;
-        k_coeffs<<<grid, WARPS_PER_CTA * 32, smem_bytes(M), st>>>(B, M, d_q, d_ts, d_head, d_tail, d_c);
-        h->launches++;
-        CK(cudaGetLastError());
-        CK(cudaMemcpyAsync(coeffs, d_c, sizeof(double) * b * N2, cudaMemcpyDeviceToHost, st));
-        CK(cudaStreamSynchronize(st));
-    }
+    Layout L;
+    const size_t o_q = L.add(sizeof(double) * b * nq), o_ts = L.add(sizeof(double) * b * M),
+                 o_head = L.add(sizeof(double) * b * 6), o_tail = L.add(sizeof(double) * b * 6),
+                 o_c = L.add(sizeof(double) * b * N2);
+    char *d;
+    int rc = grow(h, h->stage, L.end, &d);
+    if (rc) return rc;
+    cudaStream_t st = h->stream;
+    CK(cudaMemcpyAsync(d + o_q, q, sizeof(double) * b * nq, cudaMemcpyHostToDevice, st));
+    CK(cudaMemcpyAsync(d + o_ts, ts, sizeof(double) * b * M, cudaMemcpyHostToDevice, st));
+    CK(cudaMemcpyAsync(d + o_head, head, sizeof(double) * b * 6, cudaMemcpyHostToDevice, st));
+    CK(cudaMemcpyAsync(d + o_tail, tail, sizeof(double) * b * 6, cudaMemcpyHostToDevice, st));
+    int grid;
+    if ((rc = launch_grid(h, k_coeffs, smem_bytes(M), WARPS_PER_CTA, b, WARPS_PER_CTA, &grid))) return rc;
+    k_coeffs<<<grid, WARPS_PER_CTA * 32, smem_bytes(M), st>>>(B, M, (const double *)(d + o_q), (const double *)(d + o_ts),
+                                                              (const double *)(d + o_head), (const double *)(d + o_tail),
+                                                              (double *)(d + o_c));
+    h->launches++;
+    CK(cudaGetLastError());
+    CK(cudaMemcpyAsync(coeffs, d + o_c, sizeof(double) * b * N2, cudaMemcpyDeviceToHost, st));
+    CK(cudaStreamSynchronize(st));
     return NEO_OK;
 }
 
@@ -1468,29 +1444,25 @@ extern "C" int neo_sample(neo_handle *h, int B, int M, const double *coeffs, con
     if (B == 0) return NEO_OK;
     CK(cudaSetDevice(h->device));
     const size_t N2 = 12 * M, b = B, ms = states ? max_samples : 0;
-    int rc;
-    for (int pass = 0; pass < 2; pass++) {
-        Carver c{pass ? (char *)h->bufs[4].p : nullptr};
-        double *d_c = c.take<double>(b * N2), *d_ts = c.take<double>(b * M), *d_s = c.take<double>(b * ms * 6 + 1);
-        int32_t *d_cnt = c.take<int32_t>(b);
-        if (!pass) {
-            void *p;
-            if ((rc = dev_buf(h, 4, c.off + 256, &p))) return rc;
-            continue;
-        }
-        cudaStream_t st = h->stream;
-        CK(cudaMemcpyAsync(d_c, coeffs, sizeof(double) * b * N2, cudaMemcpyHostToDevice, st));
-        CK(cudaMemcpyAsync(d_ts, ts, sizeof(double) * b * M, cudaMemcpyHostToDevice, st));
-        if (states) CK(cudaMemcpyAsync(d_s, states, sizeof(double) * b * ms * 6, cudaMemcpyHostToDevice, st));
-        dim3 grid(states ? (max_samples + 127) / 128 : 1, B < 65535 ? B : 65535);
-        k_sample<<<grid, 128, 0, st>>>(B, M, d_c, d_ts, hz, max_samples, states ? d_s : nullptr, d_cnt);
-        h->launches++;
-        CK(cudaGetLastError());
-        CK(cudaMemcpyAsync(count, d_cnt, sizeof(int32_t) * b, cudaMemcpyDeviceToHost, st));
-        if (states) CK(cudaMemcpyAsync(states, d_s, sizeof(double) * b * ms * 6, cudaMemcpyDeviceToHost, st));
-        CK(cudaStreamSynchronize(st));
-        if (states) for (size_t i = 0; i < b; i++) if (count[i] > max_samples) return fail(h, "neo_sample: max_samples too small");
-    }
+    Layout L;
+    const size_t o_c = L.add(sizeof(double) * b * N2), o_ts = L.add(sizeof(double) * b * M),
+                 o_s = L.add(sizeof(double) * b * ms * 6), o_cnt = L.add(sizeof(int32_t) * b);
+    char *d;
+    int rc = grow(h, h->stage, L.end, &d);
+    if (rc) return rc;
+    cudaStream_t st = h->stream;
+    CK(cudaMemcpyAsync(d + o_c, coeffs, sizeof(double) * b * N2, cudaMemcpyHostToDevice, st));
+    CK(cudaMemcpyAsync(d + o_ts, ts, sizeof(double) * b * M, cudaMemcpyHostToDevice, st));
+    if (states) CK(cudaMemcpyAsync(d + o_s, states, sizeof(double) * b * ms * 6, cudaMemcpyHostToDevice, st));
+    dim3 grid(states ? (max_samples + 127) / 128 : 1, B < 65535 ? B : 65535);
+    k_sample<<<grid, 128, 0, st>>>(B, M, (const double *)(d + o_c), (const double *)(d + o_ts), hz, max_samples,
+                                   states ? (double *)(d + o_s) : nullptr, (int32_t *)(d + o_cnt));
+    h->launches++;
+    CK(cudaGetLastError());
+    CK(cudaMemcpyAsync(count, d + o_cnt, sizeof(int32_t) * b, cudaMemcpyDeviceToHost, st));
+    if (states) CK(cudaMemcpyAsync(states, d + o_s, sizeof(double) * b * ms * 6, cudaMemcpyDeviceToHost, st));
+    CK(cudaStreamSynchronize(st));
+    if (states) for (size_t i = 0; i < b; i++) if (count[i] > max_samples) return fail(h, "neo_sample: max_samples too small");
     return NEO_OK;
 }
 
@@ -1541,9 +1513,9 @@ static int astar_launch(neo_handle *h, int B, const double *start, const double 
         CK(cudaFuncSetAttribute(k_astar, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)ASTAR_SMEM_BYTES));
         h->astar_cap = cap; h->astar_warps = (int)warps; h->astar_laid_icap = icap;
     }
-    int rc;
-    int32_t *overflow;
-    if ((rc = dev_buf(h, 9, sizeof(int32_t) * (size_t)B + 256, (void **)&overflow))) return rc;
+    char *overflow;
+    const int rc = grow(h, h->astar_overflow, sizeof(int32_t) * (size_t)B, &overflow);
+    if (rc) return rc;
     AstarArgs a;
     a.maps = h->d_maps; a.map_ids = map_ids; a.start = start; a.target = target;
     a.B = B; a.max_closed = max_closed; a.max_path = max_path;
@@ -1554,7 +1526,7 @@ static int astar_launch(neo_handle *h, int B, const double *start, const double 
     char *p1 = p0 + list0 * laid;
     a.nodes = (AstarNode *)h->astar.p;
     a.cap = cap;
-    a.overflow = overflow;
+    a.overflow = (int32_t *)overflow;
     a.overflow_count = h->d_counter + 18;
     CK(cudaMemsetAsync(h->d_counter + 16, 0, 3 * sizeof(unsigned int), st));
     // pass 0
@@ -1606,45 +1578,36 @@ extern "C" int neo_astar(neo_handle *h, int B, const double *start, const double
     if (!h) return NEO_ERR_INVALID;
     std::lock_guard<std::mutex> g(h->mu);
     int rc = astar_check(h, B, start, target, max_closed, max_path, path, path_len, pruned, status, closed);
-    if (rc) return rc;
-    if (B == 0) return NEO_OK;
+    if (rc || B == 0) return rc;
     for (int i = 0; i < 2 * B; i++)
         if (!isfinite(start[i]) || !isfinite(target[i])) return fail(h, "neo_astar: start/target must be finite");
-    if (map_ids)
-        for (int i = 0; i < B; i++)
-            if (map_ids[i] < 0 || map_ids[i] >= (int)h->slots.size() || !h->slots[map_ids[i]].cells)
-                return fail(h, "neo_astar: map id refers to an empty slot");
-    if (!map_ids && !h->slots[0].cells) return fail(h, "neo_astar: slot 0 is empty");
+    if ((rc = check_map_ids(h, B, map_ids, "neo_astar"))) return rc;
     CK(cudaSetDevice(h->device));
     const size_t b = B, np = path ? (size_t)max_path : 0;
-    for (int pass = 0; pass < 2; pass++) {
-        Carver c{pass ? (char *)h->bufs[7].p : nullptr};
-        double *d_s = c.take<double>(2 * b), *d_t = c.take<double>(2 * b), *d_pr = c.take<double>(8 * b),
-               *d_path = c.take<double>(2 * b * np + 1);
-        int32_t *d_ids = c.take<int32_t>(b), *d_len = c.take<int32_t>(b), *d_st = c.take<int32_t>(b),
-                *d_cl = c.take<int32_t>(b);
-        if (!pass) {
-            void *p;
-            if ((rc = dev_buf(h, 7, c.off + 256, &p))) return rc;
-            continue;
-        }
-        cudaStream_t st = h->stream;
-        CK(cudaMemcpyAsync(d_s, start, sizeof(double) * 2 * b, cudaMemcpyHostToDevice, st));
-        CK(cudaMemcpyAsync(d_t, target, sizeof(double) * 2 * b, cudaMemcpyHostToDevice, st));
-        if (map_ids) CK(cudaMemcpyAsync(d_ids, map_ids, sizeof(int32_t) * b, cudaMemcpyHostToDevice, st));
-        CK(cudaEventRecord(h->ev0, st));
-        rc = astar_launch(h, B, d_s, d_t, map_ids ? d_ids : nullptr, max_closed, max_path, path ? d_path : nullptr, d_len,
-                          d_pr, d_st, d_cl, st);
-        if (rc) return rc;
-        CK(cudaEventRecord(h->ev1, st));
-        CK(cudaMemcpyAsync(path_len, d_len, sizeof(int32_t) * b, cudaMemcpyDeviceToHost, st));
-        CK(cudaMemcpyAsync(status, d_st, sizeof(int32_t) * b, cudaMemcpyDeviceToHost, st));
-        CK(cudaMemcpyAsync(closed, d_cl, sizeof(int32_t) * b, cudaMemcpyDeviceToHost, st));
-        CK(cudaMemcpyAsync(pruned, d_pr, sizeof(double) * 8 * b, cudaMemcpyDeviceToHost, st));
-        if (path) CK(cudaMemcpyAsync(path, d_path, sizeof(double) * 2 * b * np, cudaMemcpyDeviceToHost, st));
-        CK(cudaStreamSynchronize(st));
-        CK(cudaEventElapsedTime(&h->last_ms, h->ev0, h->ev1));
-    }
+    Layout L;
+    const size_t o_s = L.add(sizeof(double) * 2 * b), o_t = L.add(sizeof(double) * 2 * b),
+                 o_pr = L.add(sizeof(double) * 8 * b), o_path = L.add(sizeof(double) * 2 * b * np),
+                 o_ids = L.add(sizeof(int32_t) * b), o_len = L.add(sizeof(int32_t) * b), o_st = L.add(sizeof(int32_t) * b),
+                 o_cl = L.add(sizeof(int32_t) * b);
+    char *d;
+    if ((rc = grow(h, h->stage, L.end, &d))) return rc;
+    cudaStream_t st = h->stream;
+    CK(cudaMemcpyAsync(d + o_s, start, sizeof(double) * 2 * b, cudaMemcpyHostToDevice, st));
+    CK(cudaMemcpyAsync(d + o_t, target, sizeof(double) * 2 * b, cudaMemcpyHostToDevice, st));
+    if (map_ids) CK(cudaMemcpyAsync(d + o_ids, map_ids, sizeof(int32_t) * b, cudaMemcpyHostToDevice, st));
+    CK(cudaEventRecord(h->ev0, st));
+    rc = astar_launch(h, B, (const double *)(d + o_s), (const double *)(d + o_t), map_ids ? (const int32_t *)(d + o_ids) : nullptr,
+                      max_closed, max_path, path ? (double *)(d + o_path) : nullptr, (int32_t *)(d + o_len),
+                      (double *)(d + o_pr), (int32_t *)(d + o_st), (int32_t *)(d + o_cl), st);
+    if (rc) return rc;
+    CK(cudaEventRecord(h->ev1, st));
+    CK(cudaMemcpyAsync(path_len, d + o_len, sizeof(int32_t) * b, cudaMemcpyDeviceToHost, st));
+    CK(cudaMemcpyAsync(status, d + o_st, sizeof(int32_t) * b, cudaMemcpyDeviceToHost, st));
+    CK(cudaMemcpyAsync(closed, d + o_cl, sizeof(int32_t) * b, cudaMemcpyDeviceToHost, st));
+    CK(cudaMemcpyAsync(pruned, d + o_pr, sizeof(double) * 8 * b, cudaMemcpyDeviceToHost, st));
+    if (path) CK(cudaMemcpyAsync(path, d + o_path, sizeof(double) * 2 * b * np, cudaMemcpyDeviceToHost, st));
+    CK(cudaStreamSynchronize(st));
+    CK(cudaEventElapsedTime(&h->last_ms, h->ev0, h->ev1));
     return NEO_OK;
 }
 
@@ -1671,13 +1634,13 @@ extern "C" int neo_fp64_peak(neo_handle *h, double *tflops)
     std::lock_guard<std::mutex> g(h->mu);
     CK(cudaSetDevice(h->device));
     const int threads = 256, blocks = h->sm_count * 8, iters = 1 << 16;
-    double *d;
-    int rc = dev_buf(h, 5, sizeof(double) * threads * blocks, (void **)&d);
+    char *d;
+    const int rc = grow(h, h->stage, sizeof(double) * threads * blocks, &d);
     if (rc) return rc;
     float best = 1e30f;
     for (int rep = 0; rep < 4; rep++) {
         CK(cudaEventRecord(h->ev0, h->stream));
-        k_fp64_peak<<<blocks, threads, 0, h->stream>>>(d, iters);
+        k_fp64_peak<<<blocks, threads, 0, h->stream>>>((double *)d, iters);
         CK(cudaEventRecord(h->ev1, h->stream));
         CK(cudaStreamSynchronize(h->stream));
         float ms;
@@ -1696,14 +1659,16 @@ extern "C" int neo_test_exp_dev(neo_handle *h, int n, const double *x, double *y
     std::lock_guard<std::mutex> g(h->mu);
     if (n == 0) return NEO_OK;
     CK(cudaSetDevice(h->device));
-    double *d;
-    int rc = dev_buf(h, 5, sizeof(double) * 2 * n, (void **)&d);
+    Layout L;
+    const size_t o_x = L.add(sizeof(double) * n), o_y = L.add(sizeof(double) * n);
+    char *d;
+    const int rc = grow(h, h->stage, L.end, &d);
     if (rc) return rc;
-    CK(cudaMemcpyAsync(d, x, sizeof(double) * n, cudaMemcpyHostToDevice, h->stream));
-    k_exp_dd<<<(n + 255) / 256, 256, 0, h->stream>>>(n, d, d + n);
+    CK(cudaMemcpyAsync(d + o_x, x, sizeof(double) * n, cudaMemcpyHostToDevice, h->stream));
+    k_exp_dd<<<(n + 255) / 256, 256, 0, h->stream>>>(n, (const double *)(d + o_x), (double *)(d + o_y));
     h->launches++;
     CK(cudaGetLastError());
-    CK(cudaMemcpyAsync(y, d + n, sizeof(double) * n, cudaMemcpyDeviceToHost, h->stream));
+    CK(cudaMemcpyAsync(y, d + o_y, sizeof(double) * n, cudaMemcpyDeviceToHost, h->stream));
     CK(cudaStreamSynchronize(h->stream));
     return NEO_OK;
 }
@@ -1714,16 +1679,19 @@ static int test_blas_prims(neo_handle *h, int count, int n, const double *a, con
     std::lock_guard<std::mutex> g(h->mu);
     if (count == 0 || n == 0) { for (size_t i = 0; i < 3 * (size_t)count; i++) out[i] = 0.0; return NEO_OK; }
     CK(cudaSetDevice(h->device));
-    double *d;
     const size_t len = (size_t)count * n;
-    int rc = dev_buf(h, 5, sizeof(double) * (2 * len + 3 * (size_t)count), (void **)&d);
+    Layout L;
+    const size_t o_a = L.add(sizeof(double) * len), o_b = L.add(sizeof(double) * len),
+                 o_out = L.add(sizeof(double) * 3 * (size_t)count);
+    char *d;
+    const int rc = grow(h, h->stage, L.end, &d);
     if (rc) return rc;
-    CK(cudaMemcpyAsync(d, a, sizeof(double) * len, cudaMemcpyHostToDevice, h->stream));
-    CK(cudaMemcpyAsync(d + len, b ? b : a, sizeof(double) * len, cudaMemcpyHostToDevice, h->stream));
-    launch_blas_prims(count, n, d, d + len, d + 2 * len, h->stream);
+    CK(cudaMemcpyAsync(d + o_a, a, sizeof(double) * len, cudaMemcpyHostToDevice, h->stream));
+    CK(cudaMemcpyAsync(d + o_b, b ? b : a, sizeof(double) * len, cudaMemcpyHostToDevice, h->stream));
+    launch_blas_prims(count, n, (const double *)(d + o_a), (const double *)(d + o_b), (double *)(d + o_out), h->stream);
     h->launches++;
     CK(cudaGetLastError());
-    CK(cudaMemcpyAsync(out, d + 2 * len, sizeof(double) * 3 * count, cudaMemcpyDeviceToHost, h->stream));
+    CK(cudaMemcpyAsync(out, d + o_out, sizeof(double) * 3 * count, cudaMemcpyDeviceToHost, h->stream));
     CK(cudaStreamSynchronize(h->stream));
     return NEO_OK;
 }

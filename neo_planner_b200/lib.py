@@ -225,7 +225,9 @@ class Handle:
             setattr(r, k, None if out.get(k) is None else out[k].ctypes.data)
         return r
 
-    def optimize(self, M, q0, ts0, head, tail, map_ids=None, retry_q=None, retry_ts=None, max_attempts=1, out=None):
+    @staticmethod
+    def _plan_inputs(M, q0, ts0, head, tail, map_ids, retry_q, retry_ts, max_attempts):
+        """Contiguous arrays of the shapes neo_optimize reads: (B, q0, ts0, head, tail, map_ids, retry_q, retry_ts)."""
         q0 = f64(q0); B = q0.shape[0]
         q0 = f64(q0, (B, 2, M - 1)); ts0 = f64(ts0, (B, M))
         head = f64(pad_state(head), (B, 3, 2)); tail = f64(pad_state(tail), (B, 3, 2))
@@ -234,32 +236,28 @@ class Handle:
             retry_q = f64(retry_q, (B, max_attempts - 1, 2, M - 1)); retry_ts = f64(retry_ts, (M,))
         else:
             retry_q = retry_ts = None
+        return B, q0, ts0, head, tail, ids, retry_q, retry_ts
+
+    def optimize(self, M, q0, ts0, head, tail, map_ids=None, retry_q=None, retry_ts=None, max_attempts=1, out=None):
+        B, *args = self._plan_inputs(M, q0, ts0, head, tail, map_ids, retry_q, retry_ts, max_attempts)
         if out is None:
             out = self.alloc_result(B, M)
         r = self.result_struct(out)
-        self._ck(self.lib.neo_optimize(self.h, B, M, ptr(q0), ptr(ts0), ptr(head), ptr(tail), ptr(ids), ptr(retry_q),
-                                       ptr(retry_ts), max_attempts, C.byref(r)))
+        self._ck(self.lib.neo_optimize(self.h, B, M, *map(ptr, args), max_attempts, C.byref(r)))
         return out
 
     def optimize_trace(self, M, q0, ts0, head, tail, map_ids=None, retry_q=None, retry_ts=None, max_attempts=1, cap=512):
         """neo_optimize_trace: optimize() plus, per task (attempt * B + problem), the first `cap` evaluations the device
         made: dict(x (A*B, cap, n), f, g, costs, status, len (A*B)). For the lockstep tests."""
-        q0 = f64(q0); B = q0.shape[0]; n = 3 * M - 2
-        q0 = f64(q0, (B, 2, M - 1)); ts0 = f64(ts0, (B, M))
-        head = f64(pad_state(head), (B, 3, 2)); tail = f64(pad_state(tail), (B, 3, 2))
-        ids = None if map_ids is None else np.ascontiguousarray(map_ids, dtype=np.int32)
-        if max_attempts > 1:
-            retry_q = f64(retry_q, (B, max_attempts - 1, 2, M - 1)); retry_ts = f64(retry_ts, (M,))
-        else:
-            retry_q = retry_ts = None
+        B, *args = self._plan_inputs(M, q0, ts0, head, tail, map_ids, retry_q, retry_ts, max_attempts)
+        n = 3 * M - 2
         out = self.alloc_result(B, M)
         r = self.result_struct(out)
         T = B * max_attempts
         tr = dict(x=np.zeros((T, cap, n)), f=np.zeros((T, cap)), g=np.zeros((T, cap, n)), costs=np.zeros((T, cap, 4)),
                   status=np.zeros((T, cap), np.int32), len=np.zeros(T, np.int32))
-        self._ck(self.lib.neo_optimize_trace(self.h, B, M, ptr(q0), ptr(ts0), ptr(head), ptr(tail), ptr(ids), ptr(retry_q),
-                                             ptr(retry_ts), max_attempts, C.byref(r), cap, ptr(tr['x']), ptr(tr['f']),
-                                             ptr(tr['g']), ptr(tr['costs']), ptr(tr['status']), ptr(tr['len'])))
+        self._ck(self.lib.neo_optimize_trace(self.h, B, M, *map(ptr, args), max_attempts, C.byref(r), cap, ptr(tr['x']),
+                                             ptr(tr['f']), ptr(tr['g']), ptr(tr['costs']), ptr(tr['status']), ptr(tr['len'])))
         return out, tr
 
     def T2tau(self, ts):
