@@ -28,16 +28,6 @@
 
 namespace neo {
 
-// Development probe (-DNEO_OPT_TICKS, devtools/README.md): cycles spent in each phase of the optimizer, summed over all
-// tiles by their first lane. Compiled out of the shipped library.
-#ifdef NEO_OPT_TICKS
-#define OT_BEGIN long long ot_last = clock64()
-#define OT(i) do { const long long ot_now = clock64(); if (T.tl == 0) { atomicAdd((unsigned long long *)&g_opt_ticks[i], (unsigned long long)(ot_now - ot_last)); atomicAdd((unsigned long long *)&g_opt_ticks[32 + (i)], 1ull); } ot_last = clock64(); } while (0)
-#else
-#define OT_BEGIN do { } while (0)
-#define OT(i) do { } while (0)
-#endif
-
 // ---- exactly rounded, never contracted -----------------------------------------------------------------------------
 __device__ __forceinline__ double xmul(double a, double b) { return __dmul_rn(a, b); }
 __device__ __forceinline__ double xadd(double a, double b) { return __dadd_rn(a, b); }
@@ -219,7 +209,7 @@ __device__ __noinline__ double loop_dot(int n, const double *a, const double *b)
 template <int N>
 __device__ __forceinline__ double loop_dot_n(const double *a, const double *b, int n = N)
 {
-    if constexpr (N > 0 && N <= 10) {
+    if constexpr (N <= 10) {
         double s = 0.0;
 #pragma unroll
         for (int i = 0; i < N; i++) s = xadd(s, xmul(a[i], b[i]));
@@ -229,7 +219,7 @@ __device__ __forceinline__ double loop_dot_n(const double *a, const double *b, i
 template <int N>
 __device__ __forceinline__ double blas_ddot_n(const double *a, const double *b, int n = N)
 {
-    if constexpr (N > 0 && N <= 10) {
+    if constexpr (N <= 10) {
         double s = 0.0;
 #pragma unroll
         for (int i = 0; i < N; i++) s = xfma(a[i], b[i], s);
@@ -302,7 +292,6 @@ __device__ __forceinline__ int lb_slot(const LbMem &L, int k) { const int s = L.
 template <int TL, int NC>
 __device__ __forceinline__ void lb_update(const Tile<TL> &T, const TileMem &m, int n, LbMem &L, double s, double y, double rr, double dr)
 {
-    OT_BEGIN;
     L.iupdat++;
     if (L.iupdat <= HIST) L.col = L.iupdat;
     else L.head = L.head + 1 == HIST ? 0 : L.head + 1;                // the oldest pair's slot is reused
@@ -324,7 +313,6 @@ __device__ __forceinline__ void lb_update(const Tile<TL> &T, const TileMem &m, i
         }
     }
     T.sync();
-    OT(2);
 }
 
 // formk: assemble the middle matrix and factor it. false: a Cholesky factorisation failed (scipy drops the memory).
@@ -332,7 +320,6 @@ template <int TL>
 __device__ __forceinline__ bool lb_factor(const Tile<TL> &T, const TileMem &m, const LbMem &L)
 {
     const int col = L.col;
-    OT_BEGIN;
     const double theta = L.theta, rtheta = xrcp(theta);
     double *wn = m.wn, *rd = m.wn + wn_col(LBW) + LBW;
 #pragma unroll 1
@@ -357,9 +344,7 @@ __device__ __forceinline__ bool lb_factor(const Tile<TL> &T, const TileMem &m, c
     }
     // NOTE the transposition: formk fills wn(jy, is) = R_z(iy, jy) for jy >= iy -- column `is`, rows jy: c2[jy] above.
     T.sync();
-    OT(3);
     if (!lb_potf2(T.tl, TL, T.mask, wn, rd, 0, col)) return false;
-    OT(4);
     if (col == 1) {                                                    // one right-hand side: trsv, a true division
         if (T.tl == 0) wn[wn_col(1)] = xdiv_r(wn[wn_col(1)], wn[0], rd[0]);
     } else {                                                           // blocked trsm kernel: 8, 4, 2, 1 rows
@@ -390,7 +375,6 @@ __device__ __forceinline__ bool lb_factor(const Tile<TL> &T, const TileMem &m, c
         }
     }
     T.sync();
-    OT(5);
     // (2,2) block: every entry (is <= js) gets its own inner product over the first col rows -- one lane each
 #pragma unroll 1
     for (int e = T.tl; e < col * (col + 1) / 2; e += TL) {
@@ -400,9 +384,7 @@ __device__ __forceinline__ bool lb_factor(const Tile<TL> &T, const TileMem &m, c
         wn[wn_col(js) + is] = xadd(wn[wn_col(js) + is], blas_ddot(col, wn + wn_col(is), wn + wn_col(js)));
     }
     T.sync();
-    OT(6);
     const bool pd = lb_potf2(T.tl, TL, T.mask, wn, rd, col, col);
-    OT(7);
     return pd;
 }
 
@@ -411,7 +393,6 @@ template <int TL, int NC>
 __device__ __forceinline__ double lb_step(const Tile<TL> &T, const TileMem &m, int n, const LbMem &L, double g)
 {
     const int col = L.col, m2 = 2 * col;
-    OT_BEGIN;
     const double theta = L.theta, rtheta = xrcp(theta);
     double *wn = m.wn, *wv = m.wn + wn_col(LBW), *rd = wv + LBW;
     double d = -g;
@@ -421,7 +402,6 @@ __device__ __forceinline__ double lb_step(const Tile<TL> &T, const TileMem &m, i
     for (int e = T.tl; e < m2; e += TL)
         wv[e] = e < col ? loop_dot_n<NC>(m.wy + lb_slot(L, e) * n, m.dv, n) : xmul(theta, loop_dot_n<NC>(m.ws + lb_slot(L, e - col) * n, m.dv, n));
     T.sync();
-    OT(8);
     // trsv, transposed: b_i = (b_i - ddot(i, u(0:i, i), b)) / u_ii. Every row's inner product is a chain of fused
     // multiply-adds in index order, so all rows advance together as each b_k becomes final.
     {
@@ -455,7 +435,6 @@ __device__ __forceinline__ double lb_step(const Tile<TL> &T, const TileMem &m, i
         }
     }
     T.sync();
-    OT(9);
 #pragma unroll 1
     for (int i = T.tl; i < col; i += TL) wv[i] = -wv[i];
     T.sync();
@@ -470,7 +449,6 @@ __device__ __forceinline__ double lb_step(const Tile<TL> &T, const TileMem &m, i
         for (int k = T.tl; k < i; k += TL) wv[k] = xfma(t, ui[k], wv[k]);
         T.sync();
     }
-    OT(10);
     if (T.tl < n) {
 #pragma unroll 1
         for (int jy = 0; jy < col; jy++) {
@@ -480,7 +458,6 @@ __device__ __forceinline__ double lb_step(const Tile<TL> &T, const TileMem &m, i
         d = xmul(d, rtheta);
     }
     T.sync();
-    OT(11);
     return d;
 }
 
@@ -556,7 +533,6 @@ __device__ __forceinline__ void opt_advance(const Tile<TL> &T, const TileMem &m,
     const double tol = (ftol / epsmch) * epsmch;
     const int maxls = 20, maxiter = 15000, maxfun = 15000;
     bool new_dir;
-    OT_BEGIN;
     if (o.first) {
         o.first = false;
         if (T.dmax(mine ? fabs(o.g) : 0.0) <= pgtol) { o.status = 1; return; }
@@ -567,7 +543,6 @@ __device__ __forceinline__ void opt_advance(const Tile<TL> &T, const TileMem &m,
         ls_load(T, m.ls, ls);
         const int ls_task = dcsrch_step(ls, o.stp, o.f, o.gd);
         if (ls_task == 0) ls_store(T, m.ls, ls);
-        OT(0);
         if (ls_task == 0) new_dir = false;                                       // FG: another trial point
         else {
             // ---- the line search accepted the last evaluated point -------------------------------------------------
@@ -585,10 +560,8 @@ __device__ __forceinline__ void opt_advance(const Tile<TL> &T, const TileMem &m,
             T.sync();
             if (mine) m.dv[T.tl] = y;
             T.sync();
-            OT(12);
             const double nr = nrm2_x87(n, m.dv);
             const double rr = xmul(nr, nr);
-            OT(1);
             double dr, ddum, s;
             if (o.stp == 1.0) { dr = xsub(o.gd, gdold); ddum = -gdold; s = o.d; }
             else { dr = xmul(xsub(o.gd, gdold), o.stp); s = xmul(o.d, o.stp); ddum = xmul(-gdold, o.stp); }
@@ -599,7 +572,6 @@ __device__ __forceinline__ void opt_advance(const Tile<TL> &T, const TileMem &m,
     for (;;) {      // (re)start a line search; loops only when a failed search drops the memory
         if (new_dir) {
             // ---- direction: Cauchy point x - g with an empty memory (theta = 1), else the subspace step; d = z - x ---
-            OT(15);
             if (o.L.col > 0 && !lb_factor(T, m, o.L)) { o.L.col = 0; o.L.head = 0; o.L.iupdat = 0; o.L.theta = 1.0; }
             if (o.L.col == 0) o.z = xsub(o.x, o.g);
             else o.z = xadd(o.x, lb_step<TL, NC>(T, m, n, o.L, o.g));
@@ -608,9 +580,7 @@ __device__ __forceinline__ void opt_advance(const Tile<TL> &T, const TileMem &m,
             T.sync();
             if (mine) m.dv[T.tl] = o.d;
             T.sync();
-            OT(13);
             const double dnorm = nrm2_x87(n, m.dv);
-            OT(1);
             o.stp = (o.nit == 0) ? fmin(xdiv(1.0, dnorm), LS_STPMAX) : 1.0;
             o.t = o.x; o.r = o.g;
             o.gd = opt_gd<TL, NC>(T, m, n, o.g, o.d);
@@ -619,7 +589,6 @@ __device__ __forceinline__ void opt_advance(const Tile<TL> &T, const TileMem &m,
             o.ifun = 0;
             if (o.gd >= 0.0) o.ifun = maxls + 1;                                // not a descent direction: fail
             else { Dcsrch ls; dcsrch_start(ls, o.stp, o.f, o.gd); ls_store(T, m.ls, ls); }
-            OT(14);
         }
         o.ifun++;
         if (o.ifun - 1 < maxls) break;                                          // evaluate the trial point

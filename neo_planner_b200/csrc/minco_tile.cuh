@@ -31,21 +31,8 @@
 #include "dd_exp.h"
 
 namespace neo {
-#ifdef NEO_OPT_TICKS
-__device__ long long g_opt_ticks[64];      // development probe: cycles [0..32) and calls [32..64) per phase
-#endif
-
 constexpr unsigned FULL = 0xffffffffu;
 
-// Phase cycles of the evaluator for the development probe (-DNEO_OPT_TICKS, scripts/gpu_opt_ticks.py: counters 17..25 of
-// g_opt_ticks, summed over tiles by their first lane); compiled out everywhere else.
-#ifdef NEO_OPT_TICKS
-#define NEO_TICK(i) do { const long long et_now = clock64(); if ((i) > 0 && T.tl == 0) { atomicAdd((unsigned long long *)&g_opt_ticks[16 + (i)], (unsigned long long)(et_now - et_last)); atomicAdd((unsigned long long *)&g_opt_ticks[48 + (i)], 1ull); } et_last = clock64(); } while (0)
-#define NEO_TICK_DECL long long et_last = 0
-#else
-#define NEO_TICK(i) do { } while (0)
-#define NEO_TICK_DECL do { } while (0)
-#endif
 constexpr int HIST = 10;        // L-BFGS memory (maxcor, EP:220)
 constexpr int LBW = 2 * HIST;   // order of the middle matrix of the compact representation
 constexpr int WN_DOUBLES = LBW * (LBW + 1) / 2 + 2 * LBW + 2;    // packed upper triangle + the subspace vector wv + 1/diagonal
@@ -132,12 +119,34 @@ struct TileMem {
     double *asg;   // [32]     cached lane assignment: piece + 16 * width + 1024 * rank
 };
 
+// Schedules of the evaluator's sample loop (eval_fg). The piece count and the tile width fix which one runs, and the
+// tile's shared-memory layout below depends on it: sample_schedule is the one place that decides.
+constexpr int SAMPLE_BY_PIECE = 0;          // M <= 4, one problem per warp
+constexpr int SAMPLE_ALL_PIECES = 1;        // M >= 5 (always 32 lanes)
+constexpr int SAMPLE_BY_PIECE_STAGED = 2;   // M <= 4, tiles narrower than a warp: one staging block, reduced after every
+                                            // piece (4 KB instead of 4 M KB of shared memory per warp -> more L1 for the map)
+__host__ __device__ constexpr int sample_schedule(int M, int TL)
+{
+    return M > 4 ? SAMPLE_ALL_PIECES : (TL < 32 ? SAMPLE_BY_PIECE_STAGED : SAMPLE_BY_PIECE);
+}
+
 // staging rows of the sample loop's partial sums: one block of 15 rows per piece when all pieces are parked before the
 // owners add them (by-piece schedule, latency-optimised), one block otherwise (see eval_fg)
 // rows are padded to TL + 1 for a full warp (conflict-free owner reads); narrow tiles are not padded (their shared memory
 // decides how many problems an SM holds)
 __host__ __device__ constexpr int red_stride(int TL) { return TL == 32 ? 33 : TL; }
-__host__ __device__ inline int red_doubles(int M, int TL, bool one_block) { return (M > 4 || one_block) ? 15 * red_stride(TL) : 15 * red_stride(TL) * M; }
+// (the one-block schedules are named rather than tested as != SAMPLE_BY_PIECE: for k_coeffs, whose M is not a constant,
+// the compiler then shares one M > 4 test with lane_cache_doubles)
+__host__ __device__ inline int red_doubles(int M, int TL)
+{
+    const int s = sample_schedule(M, TL);
+    return (s == SAMPLE_ALL_PIECES || s == SAMPLE_BY_PIECE_STAGED) ? 15 * red_stride(TL) : 15 * red_stride(TL) * M;
+}
+// the all-pieces schedule's cached lane assignment: lw [2M], nsprev [M], asg [32]
+__host__ __device__ inline int lane_cache_doubles(int M, int TL)
+{
+    return sample_schedule(M, TL) == SAMPLE_ALL_PIECES ? 2 * M + M + 32 : 0;
+}
 
 // Layout of a tile's slice. Shared memory is what limits the number of problems in flight per SM, so regions whose
 // lifetimes do not overlap share storage:
@@ -154,32 +163,32 @@ __host__ __device__ inline int scratch_a_doubles(int M)
     const int n = 3 * M - 2, M1 = M + 1;
     return M + M + 5 * M + M + 2 * M1 + 4 * M1 + 12 * (M - 1) + 12 * M + 12 * M + 2 * M + 2 * M + n + 2 * M;
 }
-__host__ __device__ inline int scratch_b_doubles(int M, int TL, bool one_block)
+__host__ __device__ inline int scratch_b_doubles(int M, int TL)
 {
-    const int M1 = M + 1, adj = 4 * M1 + 4 * M1 + 12 * M + 10 * M1, red = red_doubles(M, TL, one_block);
+    const int M1 = M + 1, adj = 4 * M1 + 4 * M1 + 12 * M + 10 * M1, red = red_doubles(M, TL);
     return red > adj ? red : adj;
 }
-__host__ __device__ inline int scratch_doubles(int M, int TL, bool one_block)
+__host__ __device__ inline int scratch_doubles(int M, int TL)
 {
-    const int ab = scratch_a_doubles(M) + scratch_b_doubles(M, TL, one_block);
+    const int ab = scratch_a_doubles(M) + scratch_b_doubles(M, TL);
     return ab > WN_DOUBLES ? ab : WN_DOUBLES;
 }
 
-__host__ __device__ inline int tile_mem_doubles(int M, int TL = 32, bool one_block = false)
+__host__ __device__ inline int tile_mem_doubles(int M, int TL = 32)
 {
     const int n = 3 * M - 2;
-    int tot = 12 + scratch_doubles(M, TL, one_block) + 2 * HIST * n + HIST * HIST + 2 * HIST + 2 * n + 16 + 7 + (M > 4 ? 2 * M + M + 32 : 0);
+    int tot = 12 + scratch_doubles(M, TL) + 2 * HIST * n + HIST * HIST + 2 * HIST + 2 * n + 16 + 7 + lane_cache_doubles(M, TL);
     return (tot + 1) & ~1;
 }
 
-// evaluator only (k_eval, k_coeffs): no optimizer state behind the scratch regions
-__host__ __device__ inline int eval_mem_doubles(int M, int TL = 32, bool one_block = false)
+// evaluator only (k_eval): no optimizer state behind the scratch regions
+__host__ __device__ inline int eval_mem_doubles(int M, int TL)
 {
-    const int tot = 12 + scratch_a_doubles(M) + scratch_b_doubles(M, TL, one_block) + (M > 4 ? 2 * M + M + 32 : 0);
+    const int tot = 12 + scratch_a_doubles(M) + scratch_b_doubles(M, TL) + lane_cache_doubles(M, TL);
     return (tot + 1) & ~1;
 }
 
-__device__ inline TileMem carve(double *base, int M, int TL = 32, bool one_block = false, bool eval_only = false)
+__device__ inline TileMem carve(double *base, int M, int TL = 32, bool eval_only = false)
 {
     const int n = 3 * M - 2, M1 = M + 1;
     TileMem m;
@@ -205,12 +214,12 @@ __device__ inline TileMem carve(double *base, int M, int TL = 32, bool one_block
     m.h = m.lam + 4 * M1;
     m.Gs = m.h + 12 * M;
     if (eval_only) {
-        base = scratch + scratch_a_doubles(M) + scratch_b_doubles(M, TL, one_block);
+        base = scratch + scratch_a_doubles(M) + scratch_b_doubles(M, TL);
         m.ws = m.wy = m.yr = m.rzd = m.dr = m.gv = m.dv = m.ls = m.oc = nullptr;
         m.lw = base; m.nsprev = base + 2 * M; m.asg = base + 3 * M;
         return m;
     }
-    base = scratch + scratch_doubles(M, TL, one_block);
+    base = scratch + scratch_doubles(M, TL);
     m.ws = base; base += HIST * n;
     m.wy = base; base += HIST * n;
     m.yr = base; base += HIST * HIST;
@@ -220,7 +229,7 @@ __device__ inline TileMem carve(double *base, int M, int TL = 32, bool one_block
     m.dv = base; base += n;
     m.ls = base; base += 16;
     m.oc = base; base += 7;
-    m.lw = base; m.nsprev = base + 2 * M; m.asg = base + 3 * M;      // only carved for M > 4 (see tile_mem_doubles)
+    m.lw = base; m.nsprev = base + 2 * M; m.asg = base + 3 * M;      // sized by lane_cache_doubles
     return m;
 }
 
@@ -230,7 +239,10 @@ __device__ __forceinline__ void begin_problem(const Tile<TL> &T, const TileMem &
 {
     const int lane = T.tl;
     if (lane < 6) { m.ht[lane] = head[lane]; m.ht[6 + lane] = tail[lane]; }
-    if (lane < M) { if (M > 4) m.nsprev[lane] = -1.0; m.pc[2 * lane] = 0.0; m.pc[2 * lane + 1] = 0.0; }
+    if (lane < M) {
+        if (sample_schedule(M, TL) == SAMPLE_ALL_PIECES) m.nsprev[lane] = -1.0;
+        m.pc[2 * lane] = 0.0; m.pc[2 * lane + 1] = 0.0;
+    }
     T.sync();
 }
 
@@ -349,11 +361,6 @@ struct EvalOut {
     unsigned ns, nv, nc;   // samples, velocity-violating samples, colliding samples (work accounting)
 };
 
-constexpr int SAMPLE_BY_PIECE = 0;   // M <= 4
-constexpr int SAMPLE_ALL_PIECES = 1; // M >= 5
-constexpr int SAMPLE_BY_PIECE_STAGED = 2;   // M <= 4, throughput variant: one staging block, reduced after every piece
-                                            // (4 KB instead of 4 M KB of shared memory per warp -> more L1 for the map)
-
 // Exact quotient (p - origin)/res (ESDF:61-62) for the rare sample whose reciprocal estimate lies within 1e-9 of an
 // integer; kept out of line so the fp64 division sequence does not sit in the hot loop's instruction stream.
 __device__ __noinline__ double exact_quotient(double num, double res) { return num / res; }
@@ -364,8 +371,8 @@ __device__ __noinline__ double exact_quotient(double num, double res) { return n
 // while the load is in flight. Polynomials are evaluated in Estrin form (three independent FMAs, then two dependent
 // ones) instead of a six-deep chain (DFMA latency is 12 cycles on this part).
 __device__ __forceinline__ void sample_point(const DevParams &P, const MapView &map, const double (&cx)[6],
-                                             const double (&cy)[6], int j, int ns, double inv_ns, bool want_grad,
-                                             double (&acc)[16], EvalOut &out, int &bad)
+                                             const double (&cy)[6], int j, int ns, double inv_ns, double (&acc)[16],
+                                             EvalOut &out, int &bad)
 {
     const double t = (double)j * P.dt;               // np.arange(0, T_max, dt)[j] (EP:251)
     const double t2 = t * t, t4 = t2 * t2;
@@ -401,33 +408,29 @@ __device__ __forceinline__ void sample_point(const DevParams &P, const MapView &
     if (vv > 0.0) {       // feasibility (EP:409-413, EP:441-451)
         const double vv2 = vv * vv, vv3 = vv2 * vv;
         acc[13] += (omg * P.dt) * vv3;
-        if (want_grad) {
-            const double K = (3.0 * P.dt * omg) * vv2;
-            const double ax = fma(20.0 * t3, cx[5], 12.0 * t2 * cx[4]) + fma(6.0 * t, cx[3], 2.0 * cx[2]);
-            const double ay = fma(20.0 * t3, cy[5], 12.0 * t2 * cy[4]) + fma(6.0 * t, cy[3], 2.0 * cy[2]);
-            const double v2t = 2.0 * (ax * vx + ay * vy);
-            const double kx = (P.w2 * K) * (2.0 * vx), ky = (P.w2 * K) * (2.0 * vy);
+        const double K = (3.0 * P.dt * omg) * vv2;
+        const double ax = fma(20.0 * t3, cx[5], 12.0 * t2 * cx[4]) + fma(6.0 * t, cx[3], 2.0 * cx[2]);
+        const double ay = fma(20.0 * t3, cy[5], 12.0 * t2 * cy[4]) + fma(6.0 * t, cy[3], 2.0 * cy[2]);
+        const double v2t = 2.0 * (ax * vx + ay * vy);
+        const double kx = (P.w2 * K) * (2.0 * vx), ky = (P.w2 * K) * (2.0 * vy);
 #pragma unroll
-            for (int k = 1; k < 6; k++) { acc[2 * k] += b1[k] * kx; acc[2 * k + 1] += b1[k] * ky; }
-            acc[12] += P.w2 * ((omg * vv3 + K * v2t * (double)j) * inv_ns);
-        }
+        for (int k = 1; k < 6; k++) { acc[2 * k] += b1[k] * kx; acc[2 * k + 1] += b1[k] * ky; }
+        acc[12] += P.w2 * ((omg * vv3 + K * v2t * (double)j) * inv_ns);
         out.nv++;
     }
     const double vd = P.safe_dis - dis;
     if (vd > 0.0) {       // collision (EP:418-422, EP:453-466); outside the map dis = 10000 never violates
         const double vd2 = vd * vd, vd3 = vd2 * vd;
         acc[14] += (omg * P.dt) * vd3;
-        if (want_grad) {
-            const double2 g = __ldg(reinterpret_cast<const double2 *>(cell));
-            const double K = (3.0 * P.dt * omg) * vd2;
-            const double p2t = -(g.x * vx + g.y * vy);
-            const double kx = -(P.w3 * K) * g.x, ky = -(P.w3 * K) * g.y;
-            const double t5 = t4 * t;
-            const double b0[6] = {1.0, t, t2, t3, t4, t5};
+        const double2 g = __ldg(reinterpret_cast<const double2 *>(cell));
+        const double K = (3.0 * P.dt * omg) * vd2;
+        const double p2t = -(g.x * vx + g.y * vy);
+        const double kx = -(P.w3 * K) * g.x, ky = -(P.w3 * K) * g.y;
+        const double t5 = t4 * t;
+        const double b0[6] = {1.0, t, t2, t3, t4, t5};
 #pragma unroll
-            for (int k = 0; k < 6; k++) { acc[2 * k] += b0[k] * kx; acc[2 * k + 1] += b0[k] * ky; }
-            acc[12] += P.w3 * ((omg * vd3 + K * p2t * (double)j) * inv_ns);
-        }
+        for (int k = 0; k < 6; k++) { acc[2 * k] += b0[k] * kx; acc[2 * k + 1] += b0[k] * ky; }
+        acc[12] += P.w3 * ((omg * vd3 + K * p2t * (double)j) * inv_ns);
         out.nc++;
     }
 }
@@ -469,14 +472,14 @@ __device__ __forceinline__ int times_from_tau(const Tile<TL> &T, const DevParams
 // before the sample loop every lane walks its samples once, forming only position -> cell address, and issues an L2
 // prefetch for each, so that the misses overlap instead of being taken one per loop trip (k_eval is bound by exactly
 // that latency: long-scoreboard stalls 43 %). The optimizer's evaluations re-read the same cells ~70 times: not worth it.
-template <int MODE, int TL, bool COLD = false>
+// MC: the piece count the kernel is compiled for (M == MC); with TL it fixes the sampling schedule.
+template <int MC, int TL, bool COLD = false>
 __device__ __forceinline__ void eval_fg(const Tile<TL> &T, const DevParams &P, const MapView &map, const TileMem &m, int M,
-                                        double xl, bool want_grad, EvalOut &out, long long *ticks = nullptr)
+                                        double xl, EvalOut &out)
 {
-    static_assert(MODE != SAMPLE_ALL_PIECES || TL == 32, "the all-pieces schedule assigns the 32 lanes of a warp");
+    static_assert(TL == 32 || MC <= 4, "the all-pieces schedule (M > 4) assigns the 32 lanes of a warp");
+    constexpr int SCHEDULE = sample_schedule(MC, TL);
     const int lane = T.tl;
-    NEO_TICK_DECL;
-    NEO_TICK(0);
     const int nq = 2 * (M - 1);
     out.status = 0; out.ns = out.nv = out.nc = 0;
     out.g = 0.0;
@@ -486,12 +489,9 @@ __device__ __forceinline__ void eval_fg(const Tile<TL> &T, const DevParams &P, c
     if (bad) { out.status = bad; out.f = 0.0; out.costs[0] = out.costs[1] = out.costs[2] = out.costs[3] = 0.0; return; }
 
     // ---- coefficients (EP:261-336) ----------------------------------------------------------------
-    NEO_TICK(1);
     load_nodes(T, m, M, xl);
     solve_nodes(T, m, M);
-    NEO_TICK(2);
     hermite_coeffs(T, m, M);
-    NEO_TICK(3);
 
     // ---- energy + time (EP:345-390): lane (piece i, dim d) -------------------------------------------
     if (lane < 2 * M) {
@@ -518,7 +518,6 @@ __device__ __forceinline__ void eval_fg(const Tile<TL> &T, const DevParams &P, c
         costs1 += m.ts[i];
     }
 
-    NEO_TICK(4);
     if constexpr (COLD) {
         for (int i = 0; i < M; i++) {
             const int ns = (int)m.nsd[2 * i];
@@ -538,14 +537,14 @@ __device__ __forceinline__ void eval_fg(const Tile<TL> &T, const DevParams &P, c
     }
     // ---- sampled penalties (EP:392-466) -----------------------------------------------------------------
     double costs2 = 0.0, costs3 = 0.0;
-    if constexpr (MODE == SAMPLE_BY_PIECE || MODE == SAMPLE_BY_PIECE_STAGED) {
+    if constexpr (SCHEDULE == SAMPLE_BY_PIECE || SCHEDULE == SAMPLE_BY_PIECE_STAGED) {
         // few pieces (M <= 4): one piece at a time, lanes over its samples; every lane parks its 15 partial sums of the
         // piece in shared memory (row = (piece, slot), padded to TL + 1 so that the owners below read conflict-free).
         // Owner (piece, slot) adds the TL per-lane partial sums in lane order (four interleaved chains): uniform trip
         // counts, no shuffles, deterministic. SAMPLE_BY_PIECE parks all pieces first and lets 15 M owners work at once
         // (shortest dependent chain); SAMPLE_BY_PIECE_STAGED re-uses one block and reduces after every piece (same
         // additions in the same order, a third of the shared memory).
-        constexpr bool STAGED = MODE == SAMPLE_BY_PIECE_STAGED;
+        constexpr bool STAGED = SCHEDULE == SAMPLE_BY_PIECE_STAGED;
 #pragma unroll 1
         for (int i = 0; i < M; i++) {            // not unrolled: ONE copy of the sample body in the instruction stream
             const int ns = (int)m.nsd[2 * i];                    // int(T/delta_t) (EP:401)
@@ -557,7 +556,7 @@ __device__ __forceinline__ void eval_fg(const Tile<TL> &T, const DevParams &P, c
             double acc[16];
 #pragma unroll
             for (int s2 = 0; s2 < 16; s2++) acc[s2] = 0.0;
-            for (int j = lane; j < ns; j += TL) sample_point(P, map, cx, cy, j, ns, inv_ns, want_grad, acc, out, bad);
+            for (int j = lane; j < ns; j += TL) sample_point(P, map, cx, cy, j, ns, inv_ns, acc, out, bad);
             double *row = m.red + (STAGED ? 0 : 15 * i) * red_stride(TL) + lane;
 #pragma unroll
             for (int s2 = 0; s2 < 15; s2++) row[s2 * red_stride(TL)] = acc[s2];
@@ -639,7 +638,7 @@ __device__ __forceinline__ void eval_fg(const Tile<TL> &T, const DevParams &P, c
             double acc[16];
 #pragma unroll
             for (int s2 = 0; s2 < 16; s2++) acc[s2] = 0.0;
-            for (int j = my_rank; j < ns; j += my_width) sample_point(P, map, cx, cy, j, ns, inv_ns, want_grad, acc, out, bad);
+            for (int j = my_rank; j < ns; j += my_width) sample_point(P, map, cx, cy, j, ns, inv_ns, acc, out, bad);
 #pragma unroll
             for (int s2 = 0; s2 < 15; s2++) m.red[s2 * 33 + lane] = acc[s2];
         }
@@ -672,10 +671,8 @@ __device__ __forceinline__ void eval_fg(const Tile<TL> &T, const DevParams &P, c
     out.costs[0] = costs0; out.costs[1] = costs1; out.costs[2] = costs2; out.costs[3] = costs3;
     out.f = costs0 * P.w0 + costs1 * P.w1 + costs2 * P.w2 + costs3 * P.w3;
     if (bad) { out.status = bad; return; }
-    if (!want_grad) return;
     T.sync();
 
-    NEO_TICK(5);
     // ---- adjoint (EP:494-537) ------------------------------------------------------------------------
     // h_i = H(T_i)^T dW/dc_i: gradient w.r.t. the boundary states of piece i, lane (i, d)
     if (lane < 2 * M) {
@@ -693,7 +690,6 @@ __device__ __forceinline__ void eval_fg(const Tile<TL> &T, const DevParams &P, c
         h[10] = 0.5 * a * g3 - a2 * g4 + 0.5 * a3 * g5;
     }
     T.sync();
-    NEO_TICK(6);
     // eta_j = dW/d(v_j, a_j) at the interior nodes, then K^T lam = eta by block elimination (lanes 0/1 per dim);
     // the Schur complements of K^T are the transposes of those of K, so D'^-1 from the forward solve is reused.
     {
@@ -729,7 +725,6 @@ __device__ __forceinline__ void eval_fg(const Tile<TL> &T, const DevParams &P, c
         if (lane < 2) { m.lam[d] = 0.0; m.lam[2 + d] = 0.0; m.lam[4 * M + d] = 0.0; m.lam[4 * M + 2 + d] = 0.0; }
     }
     T.sync();
-    NEO_TICK(7);
     // G rows of interior node j (reference rows 6(j-1)+3 .. 6(j-1)+8), lane (j, d): grad_q and the T-gradient inputs
     if (lane >= 2 && lane < 2 * M) {
         const int j = lane >> 1, d = lane & 1;
@@ -750,7 +745,6 @@ __device__ __forceinline__ void eval_fg(const Tile<TL> &T, const DevParams &P, c
         m.gout[d * (M - 1) + (j - 1)] = Gq;              // grad_q[d][j-1] = G[6(j-1)+3][d] (EP:506-508)
     }
     T.sync();
-    NEO_TICK(8);
     // grad_T (EP:511-533): piece i < M-1 uses T_i; the last piece re-uses the loop variable T = ts[M-2]
     if (lane < M) {
         const int i = lane;
@@ -785,7 +779,6 @@ __device__ __forceinline__ void eval_fg(const Tile<TL> &T, const DevParams &P, c
     T.sync();
     out.g = (lane < nq + M) ? m.gout[lane] : 0.0;
     T.sync();
-    NEO_TICK(9);
 }
 
 }  // namespace neo

@@ -98,19 +98,15 @@ __device__ __forceinline__ bool resolved(unsigned st, int A)
 // the stall samples `no_instruction`). Warps that walk the code TOGETHER share every fetched line (devtools/
 // icache_share.cu: 12 warps in step run a 96 KB body at 3.6 IPC per SM, spread out at 2.5), but a barrier over all 12
 // warps waits for the slowest search direction every round (40 % barrier stalls). Groups of nine are the measured optimum.
-#ifdef NEO_ROUND_TRACE
-__device__ long long g_round_trace[12 * 2048 * 4];      // development probe: per warp of CTA 0, per round: arrive, go, evaluated, advanced
-#endif
-template <int MODE, int MC, int TL, int MINB, int WPC = WARPS_PER_CTA>
+template <int MC, int TL, int MINB, int WPC = WARPS_PER_CTA>
 __global__ void __launch_bounds__(WPC * 32, MINB) k_optimize(const DevParams P, const OptArgs a)
 {
     extern __shared__ double smem[];
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
     const Tile<TL> T(lane);
     constexpr int TPW = 32 / TL;
-    const int M = MC > 0 ? MC : a.M, n = 3 * M - 2, nq = 2 * (M - 1), N = 6 * M, A = a.max_attempts;
-    constexpr bool ONE_BLOCK = MODE == SAMPLE_BY_PIECE_STAGED;
-    const TileMem m = carve(smem + (size_t)(warp * TPW + lane / TL) * tile_mem_doubles(M, TL, ONE_BLOCK), M, TL, ONE_BLOCK);
+    const int M = MC, n = 3 * M - 2, nq = 2 * (M - 1), N = 6 * M, A = a.max_attempts;
+    const TileMem m = carve(smem + (size_t)(warp * TPW + lane / TL) * tile_mem_doubles(M, TL), M, TL);
     const unsigned total = (unsigned)A * (unsigned)a.B;
     const bool mine = T.tl < n;
     OptState o;
@@ -128,13 +124,7 @@ __global__ void __launch_bounds__(WPC * 32, MINB) k_optimize(const DevParams P, 
         if (threadIdx.x == 0) s_arrivals = 0;
         __syncthreads();
     }
-#ifdef NEO_ROUND_TRACE
-    int rt_round = 0;
-#endif
     for (;;) {
-#ifdef NEO_ROUND_TRACE
-        if (blockIdx.x == 0 && lane == 0 && rt_round < 2048) g_round_trace[(warp * 2048 + rt_round) * 4 + 0] = clock64();
-#endif
         if constexpr (WPC > WARPS_PER_CTA) {
             // departures in groups: a warp arriving at the evaluation site takes a ticket and waits on a hardware
             // barrier until the bus_q warps of its group have gathered, so that the group walks the evaluator's code
@@ -149,10 +139,6 @@ __global__ void __launch_bounds__(WPC * 32, MINB) k_optimize(const DevParams P, 
                 else asm volatile("bar.sync %0, %1;" ::"r"(1 + (int)((k / (unsigned)a.bus_q) & 7u)), "r"(a.bus_q * 32) : "memory");
             }
         }
-#ifdef NEO_ROUND_TRACE
-        if (blockIdx.x == 0 && lane == 0 && rt_round < 2048) g_round_trace[(warp * 2048 + rt_round) * 4 + 1] = clock64();
-        const int rt_now = rt_round++;
-#endif
         if (__all_sync(FULL, retired)) {
             if constexpr (WPC > WARPS_PER_CTA) {
                 if (!drained) {
@@ -210,12 +196,7 @@ __global__ void __launch_bounds__(WPC * 32, MINB) k_optimize(const DevParams P, 
             if (!opt_same_point(T, o, n)) {
                 // ---- the evaluation site: f, g at x --------------------------------------------------------------
                 EvalOut ev;
-                OT_BEGIN;
-                eval_fg<MODE, TL>(T, P, a.maps[map_id], m, M, o.x, true, ev);
-                OT(16);
-#ifdef NEO_ROUND_TRACE
-                if (blockIdx.x == 0 && lane == 0 && rt_now < 2048) g_round_trace[(warp * 2048 + rt_now) * 4 + 2] = clock64();
-#endif
+                eval_fg<MC, TL>(T, P, a.maps[map_id], m, M, o.x, ev);
                 if (T.tl == 0) { m.oc[4] += (double)ev.ns; m.oc[5] += (double)ev.nv; m.oc[6] += (double)ev.nc; }   // exact below 2^53
                 if (a.tr_x && o.nfev < a.trace_cap) {
                     const size_t k = (size_t)tid * a.trace_cap + o.nfev;
@@ -230,14 +211,10 @@ __global__ void __launch_bounds__(WPC * 32, MINB) k_optimize(const DevParams P, 
                 }
             }
             if (running) {
-                opt_advance<TL, (MC > 0 ? 3 * MC - 2 : 0)>(T, m, n, o, a.p_state + b, lower_ok);
+                opt_advance<TL, 3 * MC - 2>(T, m, n, o, a.p_state + b, lower_ok);
                 if (o.status != ST_RUNNING) { running = false; ended = true; report = true; }
             }
         }
-#ifdef NEO_ROUND_TRACE
-        __syncwarp();
-        if (blockIdx.x == 0 && lane == 0 && rt_now < 2048) g_round_trace[(warp * 2048 + rt_now) * 4 + 3] = clock64();
-#endif
         if (!ended) continue;
 
         // ---- the task ended: record it, mark it in the problem's state word -------------------------------------
@@ -319,23 +296,22 @@ struct EvalArgs {
 };
 
 // get_cost + get_grad (EP:539-585) fused, one tile per problem
-template <int MODE, int MC, int TL>
+template <int MC, int TL>
 __global__ void __launch_bounds__(WARPS_PER_CTA * 32, 3) k_eval(const DevParams P, const EvalArgs a)
 {
     extern __shared__ double smem[];
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
     const Tile<TL> T(lane);
     constexpr int TPW = 32 / TL, TPC = WARPS_PER_CTA * TPW;
-    const int M = MC > 0 ? MC : a.M, n = 3 * M - 2, N = 6 * M;
+    const int M = MC, n = 3 * M - 2, N = 6 * M;
     const int tile = warp * TPW + lane / TL;
-    constexpr bool ONE_BLOCK = MODE == SAMPLE_BY_PIECE_STAGED;
-    const TileMem m = carve(smem + (size_t)tile * eval_mem_doubles(M, TL, ONE_BLOCK), M, TL, ONE_BLOCK, true);
+    const TileMem m = carve(smem + (size_t)tile * eval_mem_doubles(M, TL), M, TL, true);
     for (size_t b = (size_t)blockIdx.x * TPC + tile; b < (size_t)a.B; b += (size_t)gridDim.x * TPC) {
         begin_problem(T, m, M, a.head + b * 6, a.tail + b * 6);
         const MapView map = a.maps[a.map_ids ? a.map_ids[b] : 0];
         const double xl = T.tl < n ? a.x[b * n + T.tl] : 0.0;
         EvalOut ev;
-        eval_fg<MODE, TL, true>(T, P, map, m, M, xl, true, ev);
+        eval_fg<MC, TL, true>(T, P, map, m, M, xl, ev);
         if (T.tl < n) a.grad[b * n + T.tl] = ev.status ? 0.0 : ev.g;
         if (T.tl < 4) a.costs[b * 4 + T.tl] = ev.costs[T.tl];
         if (T.tl == 0) a.status[b] = ev.status;
@@ -964,9 +940,9 @@ static int check_map_ids(neo_handle *h, int B, const int32_t *map_ids, const cha
     return NEO_OK;
 }
 
-static size_t smem_bytes(int M, int TL = 32, bool one_block = false, int wpc = WARPS_PER_CTA)
+static size_t smem_bytes(int M, int TL = 32, int wpc = WARPS_PER_CTA)
 {
-    return sizeof(double) * (size_t)tile_mem_doubles(M, TL, one_block) * wpc * (32 / TL);
+    return sizeof(double) * (size_t)tile_mem_doubles(M, TL) * wpc * (32 / TL);
 }
 
 // sets the kernel's dynamic shared memory and returns in *grid the CTAs for `items` work items at per_cta a CTA, no
@@ -996,7 +972,7 @@ static int tile_lanes(const neo_handle *h, int B, int M)
 }
 
 // The kernels of one piece count and lane count. One instantiation per supported piece count (loops over pieces/nodes
-// unroll: 1.27x); sampling schedule (minco_tile.cuh) by trajectory length. Every k_optimize variant is sized for 12
+// unroll: 1.27x); sampling schedule by sample_schedule (minco_tile.cuh). Every k_optimize variant is sized for 12
 // warps per SM (168 registers, no spills: config 5 38.7 -> 33.2 ms against 8 warps) and exists twice: three CTAs of 4
 // warps per SM (small batches: spread over all SMs, nobody waits) and ONE CTA of 12 warps whose warps leave the
 // evaluation site in groups of nine, sharing their instruction fetches (config 4 33.9 -> 26.4 ms, config 5 33.2 -> 30.5
@@ -1007,22 +983,23 @@ struct Variant {
     void (*eval)(const DevParams, const EvalArgs) = nullptr;
 };
 
-template <int MODE, int MC, int TL>
+template <int MC, int TL>
 static Variant kernels(bool grouped)
 {
     Variant v;
-    v.eval = k_eval<MODE, MC, TL>;
-    if (grouped) { v.opt = k_optimize<MODE, MC, TL, 1, 3 * WARPS_PER_CTA>; v.opt_wpc = 3 * WARPS_PER_CTA; }
-    else v.opt = k_optimize<MODE, MC, TL, 3, WARPS_PER_CTA>;
+    v.eval = k_eval<MC, TL>;
+    if (grouped) { v.opt = k_optimize<MC, TL, 1, 3 * WARPS_PER_CTA>; v.opt_wpc = 3 * WARPS_PER_CTA; }
+    else v.opt = k_optimize<MC, TL, 3, WARPS_PER_CTA>;
     return v;
 }
 
-// TL: tile_lanes; only M <= 4 has shared-tile kernels (one staging block per tile)
+// TL: tile_lanes; only M <= 4 has shared-tile kernels
 template <int MC>
 static Variant variant(int TL, bool grouped)
 {
-    if constexpr (MC > 4) return kernels<SAMPLE_ALL_PIECES, MC, 32>(grouped);
-    else return TL < 32 ? kernels<SAMPLE_BY_PIECE_STAGED, MC, shared_lanes(MC)>(grouped) : kernels<SAMPLE_BY_PIECE, MC, 32>(grouped);
+    if constexpr (MC <= 4)
+        if (TL < 32) return kernels<MC, shared_lanes(MC)>(grouped);
+    return kernels<MC, 32>(grouped);
 }
 
 static Variant pick_variant(int M, int TL, bool grouped)
@@ -1053,8 +1030,7 @@ static int launch_optimize(neo_handle *h, OptArgs a, cudaStream_t st)
     const int wpc = v.opt_wpc;
     a.bus_q = h->group_warps > 0 ? h->group_warps : 3 * wpc / 4;        // 12 warps: 9 (26.4 ms; 8: 26.5, 10: 26.9, 6: 27.9, 12: 30.2)
     if (a.bus_q > wpc) a.bus_q = wpc;
-    // shared tiles: one staging block per tile (shared memory is what limits occupancy)
-    const size_t smem = smem_bytes(a.M, TL, TL < 32, wpc);
+    const size_t smem = smem_bytes(a.M, TL, wpc);
     const size_t tasks = (size_t)a.B * a.max_attempts, n = 3 * a.M - 2;
     int grid;
     int rc = launch_grid(h, v.opt, smem, wpc, tasks, (size_t)wpc * (32 / TL), &grid);
@@ -1084,7 +1060,7 @@ static int launch_eval(neo_handle *h, EvalArgs a, cudaStream_t st)
     const auto kern = pick_variant(a.M, TL, false).eval;
     if (!kern) return fail(h, "M must be in [2, NEO_MAX_PIECES]");
     // evaluator-only shared memory (no optimizer state): half of k_optimize's per tile, so registers decide the occupancy
-    const size_t smem = sizeof(double) * (size_t)eval_mem_doubles(a.M, TL, TL < 32) * WARPS_PER_CTA * (32 / TL);
+    const size_t smem = sizeof(double) * (size_t)eval_mem_doubles(a.M, TL) * WARPS_PER_CTA * (32 / TL);
     int grid;
     int rc = launch_grid(h, kern, smem, WARPS_PER_CTA, a.B, WARPS_PER_CTA * (32 / TL), &grid);
     if (rc) return rc;
@@ -1715,27 +1691,6 @@ extern "C" int neo_test_ddot_dev(neo_handle *h, int count, int n, const double *
     for (int i = 0; i < count; i++) { blas[i] = out[3 * (size_t)i + 1]; loop[i] = out[3 * (size_t)i + 2]; }
     return NEO_OK;
 }
-
-#ifdef NEO_ROUND_TRACE
-extern "C" int neo_test_round_trace(long long *out)
-{
-    cudaDeviceSynchronize();
-    cudaMemcpyFromSymbol(out, g_round_trace, sizeof(long long) * 12 * 2048 * 4);
-    return NEO_OK;
-}
-#endif
-
-#ifdef NEO_OPT_TICKS
-// development probe: read and clear the optimizer's phase counters (cycles [0..32), calls [32..64))
-extern "C" int neo_test_opt_ticks(long long *out)
-{
-    cudaDeviceSynchronize();
-    cudaMemcpyFromSymbol(out, g_opt_ticks, sizeof(long long) * 64);
-    long long z[64] = {0};
-    cudaMemcpyToSymbol(g_opt_ticks, z, sizeof(z));
-    return NEO_OK;
-}
-#endif
 
 // test hook (no GPU needed): `calls` runs of the host worker pool over [0, count); every index must be visited exactly once
 // per run. Returns the number of indices whose visit count is wrong.
