@@ -374,6 +374,12 @@ __device__ __forceinline__ void sample_point(const DevParams &P, const MapView &
                                              const double (&cy)[6], int j, int ns, double inv_ns, double (&acc)[16],
                                              EvalOut &out, int &bad)
 {
+    // The map's size and cell base are read here, with its origin and 1/res, not where they are used: k_optimize passes
+    // the map by reference into global memory, and reads after the out-of-line exact_quotient call could not be issued
+    // before it, so they would wait for the position and then for each other -- three dependent L1/L2 round trips per
+    // sample instead of one ahead of the distance load.
+    const Cell *const cells = map.cells;
+    const int H = map.H, W = map.W;
     const double t = (double)j * P.dt;               // np.arange(0, T_max, dt)[j] (EP:251)
     const double t2 = t * t, t4 = t2 * t2;
     const double px = fma(t4, fma(cx[5], t, cx[4]), fma(t2, fma(cx[3], t, cx[2]), fma(cx[1], t, cx[0])));
@@ -391,11 +397,11 @@ __device__ __forceinline__ void sample_point(const DevParams &P, const MapView &
         if (ec < 1e-9 || ec > 1.0 - 1e-9) { fc = exact_quotient(dx, map.res); tc = trunc(fc); }
     }
     if (fr != fr || fc != fc) bad = 6;                 // int(nan) raises ValueError
-    const bool inside = tr >= 0.0 && tr < (double)map.H && tc >= 0.0 && tc < (double)map.W;
+    const bool inside = tr >= 0.0 && tr < (double)H && tc >= 0.0 && tc < (double)W;
     double dis = 10000.0;
-    const Cell *cell = map.cells;
+    const Cell *cell = cells;
     if (inside) {
-        cell = map.cells + ((size_t)(int)tr * map.W + (int)tc);
+        cell = cells + ((size_t)(int)tr * W + (int)tc);
         dis = __ldg(&cell->d);
     }
     const double t3 = t2 * t;
