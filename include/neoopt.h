@@ -19,7 +19,7 @@
  *   reported in `status` arrays (NEO_ST_*), never as a failing return code.
  *   Thread safety: calls on one handle are serialised by an internal mutex; handles are independent.
  *   Functions ending in _dev take DEVICE pointers and enqueue on `stream` (a cudaStream_t passed as
- *   void*; NULL = the handle's own stream) without synchronising. A handle owns ONE set of scratch buffers
+ *   void*; NULL = the handle's own stream, cudaStreamLegacy = the legacy default stream) without synchronising. A handle owns ONE set of scratch buffers
  *   (work-queue counter, per-attempt records): consecutive _dev launches on the same handle must be ordered on the
  *   same stream, and maps must not be re-uploaded while a launch is in flight. Use one handle per concurrent stream.
  *   map_ids passed to host-pointer entry points are validated (every id must name a slot that holds a map, else
@@ -156,8 +156,8 @@ int neo_optimize_trace(neo_handle *h, int B, int M, const double *q0, const doub
                        double *tr_costs, int32_t *tr_status, int32_t *tr_len);
 
 /* Device-pointer variant: every pointer (inputs, retry_*, and all non-NULL members of *out) is a DEVICE
- * pointer; the launch is enqueued on `stream` and not synchronised. Inputs are in tau form because
- * map_T2tau (EP:468-475) has to run on the host libm to match CPython's math.log bit for bit:
+ * pointer; the launch is enqueued on `stream` and not synchronised. Inputs are in tau form (neo_prepare_dev
+ * builds them on the device, neo_T2tau on the host):
  *   x0 (B,n) = [q0, neo_T2tau(ts0)], x0_status (B) or NULL = its per-problem status,
  *   retry_tau (M) = neo_T2tau(retry_ts), retry_status = its status (0 or NEO_ST_DOMAIN). */
 int neo_optimize_dev(neo_handle *h, int B, int M, const double *x0, const int32_t *x0_status, const double *head,
@@ -166,6 +166,29 @@ int neo_optimize_dev(neo_handle *h, int B, int M, const double *x0, const int32_
 int neo_eval_dev(neo_handle *h, int B, int M, const double *x, const double *head, const double *tail,
                  const int32_t *map_ids, double *costs, double *grad, int32_t *status, double *coeffs, double *ts,
                  void *stream);
+
+/* Device-resident inputs: the same values the host-pointer path assembles, computed on the device. DEVICE pointers,
+ * enqueued on `stream` (NULL = the handle's own) without synchronising, like the _dev calls above.
+ * neo_T2tau_dev: neo_T2tau for n device values -- glibc's log is restated on the device (csrc/libm_log.h), so tau and
+ *   status equal neo_T2tau's bit for bit on a host whose C library is glibc on an x86-64 CPU with FMA. status may be NULL.
+ * neo_prepare_dev: the inputs of neo_optimize_dev for B problems, as neo_optimize builds them from (q0, ts0):
+ *   x0 (B,n) = [q0, T2tau(ts0)] (tau = 0 where the status is set), x0_status (B) = the last nonzero status of the row;
+ *   q0 (B,2,M-1) or NULL = the straight line of guesses.straight_line_guess (head pos -> tail pos, M-1 waypoints);
+ *   ts0 (B,M) or NULL = the HOST vector init_ts (M) for every problem;
+ *   retry_q (B,count,2,M-1) = that straight line + noise (B,count,M-1,2) (guesses.retry_guesses); count in [0, 7];
+ *   map_ids_host (B) or NULL: HOST ids, checked like neo_optimize's (NEO_ERR_INVALID before anything is enqueued),
+ *   then copied to the device array map_ids_dev (B) that neo_optimize_dev reads.
+ *   head, tail (B,3,2) are device arrays. The retry durations are host data: pass neo_T2tau(init_ts) as retry_tau. */
+int neo_T2tau_dev(neo_handle *h, int n, const double *ts, double *tau, int32_t *status, void *stream);
+int neo_prepare_dev(neo_handle *h, int B, int M, const double *head, const double *tail, const double *q0,
+                    const double *ts0, const double *init_ts, int count, const double *noise, const int32_t *map_ids_host,
+                    double *x0, int32_t *x0_status, double *retry_q, int32_t *map_ids_dev, void *stream);
+/* neo_get_coeffs / neo_sample on device arrays. neo_sample_dev always writes count (the full count, which may exceed
+ * max_samples) and never writes a row at or past max_samples; states may be NULL (counts only). */
+int neo_get_coeffs_dev(neo_handle *h, int B, int M, const double *q, const double *ts, const double *head,
+                       const double *tail, double *coeffs, void *stream);
+int neo_sample_dev(neo_handle *h, int B, int M, const double *coeffs, const double *ts, double hz, int max_samples,
+                   double *states, int32_t *count, void *stream);
 
 /* host helpers with the reference's libm semantics --------------------------------------------- */
 /* map_T2tau (EP:468-475) for n values using the C library's log(), i.e. the same function CPython's

@@ -13,8 +13,8 @@ import sys
 HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, 'csrc')
 SO = os.path.join(HERE, 'libneoopt.so')
-SOURCES = ['neoopt.cu', 'test_prims.cu']
-DEPS = ['neoopt.cu', 'test_prims.cu', 'minco_tile.cuh', 'lbfgsb_tile.cuh', 'x87_nrm2.h', 'map_kernels.cuh', 'astar_warp.cuh', 'dd_exp.h', '../../include/neoopt.h']
+SOURCES = ['neoopt.cu', 'test_prims.cu', 'device_api.cu']
+DEPS = ['neoopt.cu', 'test_prims.cu', 'device_api.cu', 'libm_log.h', 'minco_tile.cuh', 'lbfgsb_tile.cuh', 'x87_nrm2.h', 'map_kernels.cuh', 'astar_warp.cuh', 'dd_exp.h', '../../include/neoopt.h']
 NVCC_FLAGS = ['-gencode', 'arch=compute_100a,code=sm_100a', '-lineinfo', '-O3', '-std=c++17',
               '-Xcompiler', '-fPIC', '-Xcompiler', '-Wno-format-truncation', '-shared']
 

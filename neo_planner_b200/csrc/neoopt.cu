@@ -406,6 +406,11 @@ __global__ void k_exp_dd(int n, const double *x, double *y)
 // test_prims.cu: the optimizer's vector primitives on the device, in a translation unit of their own so that a second
 // caller does not change how k_optimize is compiled
 void launch_blas_prims(int count, int n, const double *a, const double *b, double *out, cudaStream_t stream);
+// device_api.cu: map_T2tau with glibc's log and the initial guesses on the device (neo_T2tau_dev, neo_prepare_dev)
+cudaError_t launch_T2tau(int n, double T_min, double T_max, const double *ts, double *tau, int32_t *status, cudaStream_t st);
+cudaError_t launch_prepare(int B, int M, double T_min, double T_max, const double *head, const double *tail,
+                           const double *q0, const double *ts0, const double *init_ts, int count, const double *noise,
+                           double *x0, int32_t *x0_status, double *retry_q, cudaStream_t st);
 
 // ---------------------------------------------------------------------------------------------------------
 // handle
@@ -1162,6 +1167,47 @@ extern "C" int neo_T2tau(const neo_config *cfg, int n, const double *ts, double 
     return NEO_OK;
 }
 
+// neo_T2tau on the device: glibc's log restated (libm_log.h), so the results equal the host's bit for bit
+extern "C" int neo_T2tau_dev(neo_handle *h, int n, const double *ts, double *tau, int32_t *status, void *stream)
+{
+    if (!h) return NEO_ERR_INVALID;
+    std::lock_guard<std::mutex> g(h->mu);
+    if (n < 0) return fail(h, "neo_T2tau_dev: n must be >= 0");
+    if (!ts || !tau) return fail(h, "neo_T2tau_dev: null pointer");
+    if (n == 0) return NEO_OK;
+    CK(cudaSetDevice(h->device));
+    CK(launch_T2tau(n, h->cfg.T_min, h->cfg.T_max, ts, tau, status, stream ? (cudaStream_t)stream : h->stream));
+    h->launches++;
+    return NEO_OK;
+}
+
+// The device inputs of neo_optimize_dev, built as optimize_host builds them: x0 = [q0, T2tau(ts0)] with its status,
+// the straight-line guess where q0 is NULL, init_ts where ts0 is NULL, and the retry guesses line + noise. The map ids
+// are host data: checked like every host-pointer entry point's, then copied to map_ids_dev.
+extern "C" int neo_prepare_dev(neo_handle *h, int B, int M, const double *head, const double *tail, const double *q0,
+                               const double *ts0, const double *init_ts, int count, const double *noise,
+                               const int32_t *map_ids_host, double *x0, int32_t *x0_status, double *retry_q,
+                               int32_t *map_ids_dev, void *stream)
+{
+    if (!h) return NEO_ERR_INVALID;
+    std::lock_guard<std::mutex> g(h->mu);
+    int rc = check_problem(h, B, M);
+    if (rc) return rc;
+    if (count < 0 || count > NEO_MAX_ATTEMPTS - 1) return fail(h, "neo_prepare_dev: count out of range");
+    if (!head || !tail || !x0 || !x0_status || (!ts0 && !init_ts) || (count > 0 && (!noise || !retry_q)) ||
+        (map_ids_host && !map_ids_dev))
+        return fail(h, "neo_prepare_dev: null pointer");
+    if (B == 0) return NEO_OK;
+    if ((rc = check_map_ids(h, B, map_ids_host, "neo_prepare_dev"))) return rc;
+    CK(cudaSetDevice(h->device));
+    cudaStream_t st = stream ? (cudaStream_t)stream : h->stream;
+    if (map_ids_host) CK(cudaMemcpyAsync(map_ids_dev, map_ids_host, sizeof(int32_t) * B, cudaMemcpyHostToDevice, st));
+    CK(launch_prepare(B, M, h->cfg.T_min, h->cfg.T_max, head, tail, q0, ts0, init_ts, count, noise, x0, x0_status,
+                      retry_q, st));
+    h->launches++;
+    return NEO_OK;
+}
+
 // internal: device pointers, tau-form inputs
 // the arrays of a neo_result, each with its bytes per problem of M pieces
 template <typename F>
@@ -1203,8 +1249,8 @@ static OptArgs opt_args(int B, int M, const double *x0, const int32_t *x0_status
     return a;
 }
 
-// Device-pointer entry. Inputs are in tau form (x0 = [q0, map_T2tau(ts0)], retry_tau = map_T2tau(retry_ts))
-// because map_T2tau must run on the host libm to match the reference bit for bit (see neo_T2tau).
+// Device-pointer entry. Inputs are in tau form (x0 = [q0, map_T2tau(ts0)], retry_tau = map_T2tau(retry_ts)): neo_prepare_dev
+// builds them on the device, neo_T2tau on the host.
 extern "C" int neo_optimize_dev(neo_handle *h, int B, int M, const double *x0, const int32_t *x0_status,
                                 const double *head, const double *tail, const int32_t *map_ids, const double *retry_q,
                                 const double *retry_tau, int retry_status, int max_attempts, const neo_result *out,
@@ -1376,14 +1422,43 @@ extern "C" int neo_optimize_trace(neo_handle *h, int B, int M, const double *q0,
 // ---------------------------------------------------------------------------------------------------------
 // coefficients / sampling
 // ---------------------------------------------------------------------------------------------------------
+static int coeffs_check(neo_handle *h, const char *who, int B, int M, bool arrays)
+{
+    if (B < 0 || M < 2 || M > NEO_MAX_PIECES) return fail(h, std::string(who) + ": B or M out of range");
+    if (!arrays) return fail(h, std::string(who) + ": null pointer");
+    return NEO_OK;
+}
+
+static int launch_coeffs(neo_handle *h, int B, int M, const double *q, const double *ts, const double *head,
+                         const double *tail, double *coeffs, cudaStream_t st)
+{
+    int grid;
+    const int rc = launch_grid(h, k_coeffs, smem_bytes(M), WARPS_PER_CTA, B, WARPS_PER_CTA, &grid);
+    if (rc) return rc;
+    k_coeffs<<<grid, WARPS_PER_CTA * 32, smem_bytes(M), st>>>(B, M, q, ts, head, tail, coeffs);
+    h->launches++;
+    CK(cudaGetLastError());
+    return NEO_OK;
+}
+
+extern "C" int neo_get_coeffs_dev(neo_handle *h, int B, int M, const double *q, const double *ts, const double *head,
+                                  const double *tail, double *coeffs, void *stream)
+{
+    if (!h) return NEO_ERR_INVALID;
+    std::lock_guard<std::mutex> g(h->mu);
+    const int rc = coeffs_check(h, "neo_get_coeffs_dev", B, M, q && ts && head && tail && coeffs);
+    if (rc || B == 0) return rc;
+    CK(cudaSetDevice(h->device));
+    return launch_coeffs(h, B, M, q, ts, head, tail, coeffs, stream ? (cudaStream_t)stream : h->stream);
+}
+
 extern "C" int neo_get_coeffs(neo_handle *h, int B, int M, const double *q, const double *ts, const double *head,
                               const double *tail, double *coeffs)
 {
     if (!h) return NEO_ERR_INVALID;
     std::lock_guard<std::mutex> g(h->mu);
-    if (B < 0 || M < 2 || M > NEO_MAX_PIECES) return fail(h, "neo_get_coeffs: B or M out of range");
-    if (!q || !ts || !head || !tail || !coeffs) return fail(h, "neo_get_coeffs: null pointer");
-    if (B == 0) return NEO_OK;
+    int rc = coeffs_check(h, "neo_get_coeffs", B, M, q && ts && head && tail && coeffs);
+    if (rc || B == 0) return rc;
     CK(cudaSetDevice(h->device));
     const size_t nq = 2 * (M - 1), N2 = 12 * M, b = B;
     Layout L;
@@ -1391,23 +1466,47 @@ extern "C" int neo_get_coeffs(neo_handle *h, int B, int M, const double *q, cons
                  o_head = L.add(sizeof(double) * b * 6), o_tail = L.add(sizeof(double) * b * 6),
                  o_c = L.add(sizeof(double) * b * N2);
     char *d;
-    int rc = grow(h, h->stage, L.end, &d);
-    if (rc) return rc;
+    if ((rc = grow(h, h->stage, L.end, &d))) return rc;
     cudaStream_t st = h->stream;
     CK(cudaMemcpyAsync(d + o_q, q, sizeof(double) * b * nq, cudaMemcpyHostToDevice, st));
     CK(cudaMemcpyAsync(d + o_ts, ts, sizeof(double) * b * M, cudaMemcpyHostToDevice, st));
     CK(cudaMemcpyAsync(d + o_head, head, sizeof(double) * b * 6, cudaMemcpyHostToDevice, st));
     CK(cudaMemcpyAsync(d + o_tail, tail, sizeof(double) * b * 6, cudaMemcpyHostToDevice, st));
-    int grid;
-    if ((rc = launch_grid(h, k_coeffs, smem_bytes(M), WARPS_PER_CTA, b, WARPS_PER_CTA, &grid))) return rc;
-    k_coeffs<<<grid, WARPS_PER_CTA * 32, smem_bytes(M), st>>>(B, M, (const double *)(d + o_q), (const double *)(d + o_ts),
-                                                              (const double *)(d + o_head), (const double *)(d + o_tail),
-                                                              (double *)(d + o_c));
-    h->launches++;
-    CK(cudaGetLastError());
+    if ((rc = launch_coeffs(h, B, M, (const double *)(d + o_q), (const double *)(d + o_ts), (const double *)(d + o_head),
+                            (const double *)(d + o_tail), (double *)(d + o_c), st)))
+        return rc;
     CK(cudaMemcpyAsync(coeffs, d + o_c, sizeof(double) * b * N2, cudaMemcpyDeviceToHost, st));
     CK(cudaStreamSynchronize(st));
     return NEO_OK;
+}
+
+static int sample_check(neo_handle *h, const char *who, int B, int M, double hz, bool arrays, const double *states,
+                        int max_samples)
+{
+    if (B < 0 || M < 1 || M > 64 || !(hz > 0.0)) return fail(h, std::string(who) + ": invalid argument");
+    if (!arrays || (states && max_samples < 1)) return fail(h, std::string(who) + ": null pointer");
+    return NEO_OK;
+}
+
+static int launch_sample(neo_handle *h, int B, int M, const double *coeffs, const double *ts, double hz, int max_samples,
+                         double *states, int32_t *count, cudaStream_t st)
+{
+    dim3 grid(states ? (max_samples + 127) / 128 : 1, B < 65535 ? B : 65535);
+    k_sample<<<grid, 128, 0, st>>>(B, M, coeffs, ts, hz, max_samples, states, count);
+    h->launches++;
+    CK(cudaGetLastError());
+    return NEO_OK;
+}
+
+extern "C" int neo_sample_dev(neo_handle *h, int B, int M, const double *coeffs, const double *ts, double hz,
+                              int max_samples, double *states, int32_t *count, void *stream)
+{
+    if (!h) return NEO_ERR_INVALID;
+    std::lock_guard<std::mutex> g(h->mu);
+    const int rc = sample_check(h, "neo_sample_dev", B, M, hz, coeffs && ts && count, states, max_samples);
+    if (rc || B == 0) return rc;
+    CK(cudaSetDevice(h->device));
+    return launch_sample(h, B, M, coeffs, ts, hz, max_samples, states, count, stream ? (cudaStream_t)stream : h->stream);
 }
 
 extern "C" int neo_sample(neo_handle *h, int B, int M, const double *coeffs, const double *ts, double hz, int max_samples,
@@ -1415,26 +1514,22 @@ extern "C" int neo_sample(neo_handle *h, int B, int M, const double *coeffs, con
 {
     if (!h) return NEO_ERR_INVALID;
     std::lock_guard<std::mutex> g(h->mu);
-    if (B < 0 || M < 1 || M > 64 || !(hz > 0.0)) return fail(h, "neo_sample: invalid argument");
-    if (!coeffs || !ts || !count || (states && max_samples < 1)) return fail(h, "neo_sample: null pointer");
-    if (B == 0) return NEO_OK;
+    int rc = sample_check(h, "neo_sample", B, M, hz, coeffs && ts && count, states, max_samples);
+    if (rc || B == 0) return rc;
     CK(cudaSetDevice(h->device));
     const size_t N2 = 12 * M, b = B, ms = states ? max_samples : 0;
     Layout L;
     const size_t o_c = L.add(sizeof(double) * b * N2), o_ts = L.add(sizeof(double) * b * M),
                  o_s = L.add(sizeof(double) * b * ms * 6), o_cnt = L.add(sizeof(int32_t) * b);
     char *d;
-    int rc = grow(h, h->stage, L.end, &d);
-    if (rc) return rc;
+    if ((rc = grow(h, h->stage, L.end, &d))) return rc;
     cudaStream_t st = h->stream;
     CK(cudaMemcpyAsync(d + o_c, coeffs, sizeof(double) * b * N2, cudaMemcpyHostToDevice, st));
     CK(cudaMemcpyAsync(d + o_ts, ts, sizeof(double) * b * M, cudaMemcpyHostToDevice, st));
     if (states) CK(cudaMemcpyAsync(d + o_s, states, sizeof(double) * b * ms * 6, cudaMemcpyHostToDevice, st));
-    dim3 grid(states ? (max_samples + 127) / 128 : 1, B < 65535 ? B : 65535);
-    k_sample<<<grid, 128, 0, st>>>(B, M, (const double *)(d + o_c), (const double *)(d + o_ts), hz, max_samples,
-                                   states ? (double *)(d + o_s) : nullptr, (int32_t *)(d + o_cnt));
-    h->launches++;
-    CK(cudaGetLastError());
+    if ((rc = launch_sample(h, B, M, (const double *)(d + o_c), (const double *)(d + o_ts), hz, max_samples,
+                            states ? (double *)(d + o_s) : nullptr, (int32_t *)(d + o_cnt), st)))
+        return rc;
     CK(cudaMemcpyAsync(count, d + o_cnt, sizeof(int32_t) * b, cudaMemcpyDeviceToHost, st));
     if (states) CK(cudaMemcpyAsync(states, d + o_s, sizeof(double) * b * ms * 6, cudaMemcpyDeviceToHost, st));
     CK(cudaStreamSynchronize(st));

@@ -104,3 +104,42 @@ def clamp_durations(ts, T_min, T_max, margin=1e-3):
     lo, hi = T_min + margin * (T_max - T_min), T_max - margin * (T_max - T_min)
     out = np.clip(np.where(np.isfinite(ts), ts, lo), lo, hi)
     return out, np.any(out != ts, axis=-1)
+
+
+# ---- the same transforms on CUDA tensors (float64), bit-identical to the NumPy functions above -----------------------
+# Every product and sum is its own elementwise operation (no fused multiply-add) and the sums run in NumPy 2.x's order
+# for these shapes: np.linalg.norm over 4 components adds them left to right, and einsum('...ij,...j->...i') with a
+# broadcast (B,1,3,3) matrix forms (R[i,0] v0 + R[i,2] v2) + R[i,1] v1. tests/test_frames_dev_order.py pins both.
+def rotation_matrix_dev(q):
+    """rotation_matrix for a (..., 4) float64 tensor."""
+    s = q * q
+    q = q / (((s[..., 0:1] + s[..., 1:2]) + s[..., 2:3]) + s[..., 3:4]).sqrt()
+    w, x, y, z = q[..., 0], q[..., 1], q[..., 2], q[..., 3]
+    rows = [[1 - 2 * (y * y + z * z), 2 * (x * y - z * w), 2 * (x * z + y * w)],
+            [2 * (x * y + z * w), 1 - 2 * (x * x + z * z), 2 * (y * z - x * w)],
+            [2 * (x * z - y * w), 2 * (y * z + x * w), 1 - 2 * (x * x + y * y)]]
+    import torch
+    return torch.stack([torch.stack(r, dim=-1) for r in rows], dim=-2)
+
+
+def rotate_dev(q, v):
+    """rotate for tensors: q (..., 4), v (..., 3) broadcast against it."""
+    R = rotation_matrix_dev(q)
+    p = [R[..., :, j] * v[..., None, j] for j in range(3)]
+    return (p[0] + p[2]) + p[1]
+
+
+def wpts_world_dev(attitude, global_pos, net_out, M=3):
+    """wpts_world on the device: attitude (B,4), global_pos (B,3), net_out (B, 3(M-1)+M) float64 CUDA tensors ->
+    int_wpts (B,2,M-1), ts (B,M), both contiguous."""
+    B = net_out.shape[0]
+    local = net_out[:, :3 * (M - 1)].reshape(B, M - 1, 3)
+    world = rotate_dev(attitude[:, None, :], local) + global_pos[:, None, :]
+    return world[:, :, :2].transpose(1, 2).contiguous(), net_out[:, 3 * (M - 1):].contiguous()
+
+
+def clamp_durations_dev(ts, T_min, T_max, margin=1e-3):
+    """clamp_durations for a float64 tensor: (ts_clamped, touched (B,) bool)."""
+    lo, hi = T_min + margin * (T_max - T_min), T_max - margin * (T_max - T_min)
+    out = ts.where(ts.isfinite(), ts.new_tensor(lo)).clamp(lo, hi)
+    return out, (out != ts).any(dim=-1)

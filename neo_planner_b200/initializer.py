@@ -92,12 +92,14 @@ class NeoBatchPlanner:
     @torch.no_grad()
     def normalize_depth(self, depth_img, chunk=512):
         """record_planner.py:15 on the device: (depth / max(depth) * 255).astype(uint8), evaluated in fp64 like NumPy
-        does, so the truncation to uint8 is the reference's. depth_img: (B,H,W) array (any real dtype). Returns a uint8
-        CUDA tensor (B,H,W)."""
-        depth_img = np.asarray(depth_img)
-        out = torch.empty(depth_img.shape, dtype=torch.uint8, device=self.device)
+        does, so the truncation to uint8 is the reference's. depth_img: (B,H,W) array (any real dtype) or tensor. Returns
+        a uint8 CUDA tensor (B,H,W)."""
+        if not torch.is_tensor(depth_img):
+            depth_img = np.asarray(depth_img)
+        out = torch.empty(tuple(depth_img.shape), dtype=torch.uint8, device=self.device)
         for i in range(0, len(depth_img), chunk):
-            d = torch.from_numpy(np.ascontiguousarray(depth_img[i:i + chunk])).to(self.device, non_blocking=True).double()
+            d = depth_img[i:i + chunk]
+            d = (d if torch.is_tensor(d) else torch.from_numpy(np.ascontiguousarray(d))).to(self.device, non_blocking=True).double()
             mx = d.amax(dim=(1, 2), keepdim=True)
             out[i:i + chunk] = (d / mx * 255).to(torch.uint8)
         return out
@@ -106,9 +108,14 @@ class NeoBatchPlanner:
     def predict(self, depth_norm, motion_info, chunk=512):
         """Network forward for B samples. depth_norm: (B,H,W) uint8, NumPy or CUDA tensor (images travel as uint8 and
         are widened on the device; the flattened float vector of nn_trainer.py:51-58 is formed there). Returns (B,9)."""
+        return self.predict_dev(depth_norm, motion_info, chunk).cpu().numpy()
+
+    @torch.no_grad()
+    def predict_dev(self, depth_norm, motion_info, chunk=512):
+        """predict, leaving the (B,9) float64 output on the device."""
         if not torch.is_tensor(depth_norm):
             depth_norm = torch.from_numpy(np.ascontiguousarray(depth_norm))
-        motion = torch.from_numpy(np.asarray(motion_info, dtype=np.float32)).to(self.device)
+        motion = torch.from_numpy(np.asarray(motion_info, dtype=np.float32)).to(self.device, non_blocking=True)
         B = depth_norm.shape[0]
         outs = []
         for i in range(0, B, chunk):
@@ -117,7 +124,7 @@ class NeoBatchPlanner:
                 lowp = self.dtype if self.device.type == 'cuda' else torch.float32      # 0..255 is exact in bf16
                 x = torch.cat([img.to(lowp), motion[i:i + chunk].to(lowp)], dim=1)
                 outs.append(self.net(x).float())
-        return torch.cat(outs).double().cpu().numpy()
+        return torch.cat(outs).double()
 
     def enhanced_traj_plan(self, depth_img, local_vel, attitude, global_pos, global_vel, init_pos, init_vel, target_state,
                            map_ids=None, rng=None):
@@ -130,6 +137,26 @@ class NeoBatchPlanner:
         ts_used = frames.clamp_durations(ts, cfg.T_min, cfg.T_max)[0] if self.clamp_ts else ts
         head = np.stack([np.asarray(init_pos)[:, :2], np.asarray(init_vel)[:, :2]], axis=1)
         res = self.planner.warm_start_plan(head, target_state, int_wpts, ts_used, map_ids, rng)
+        res['nn_int_wpts'], res['nn_ts'], res['nn_ts_outside_bounds'] = int_wpts, ts, outside
+        return res
+
+    def enhanced_traj_plan_dev(self, depth_img, local_vel, attitude, global_pos, global_vel, init_pos, init_vel,
+                               target_state, map_ids=None, noise=None, generator=None):
+        """enhanced_traj_plan with the network output kept on the device: the waypoint transform, the duration clamp,
+        the initial guesses and the optimizer all run there, and nothing waits for the GPU. depth_img may be a CUDA
+        tensor; the per-sample states are host arrays (they also form the motion vector). Retry noise as in
+        BatchPlanner.warm_start_plan_dev (`noise` tensor, else N(0, 0.5) from the torch `generator`, not np.random).
+        Returns the keys of enhanced_traj_plan as CUDA tensors, bit-identical to it for the same network and noise."""
+        motion = frames.motion_info(local_vel, attitude, global_pos, global_vel, self.des_pos_z, init_pos, init_vel,
+                                    target_state)
+        out = self.predict_dev(self.normalize_depth(depth_img), motion)
+        up = lambda a: torch.from_numpy(np.ascontiguousarray(a, dtype=np.float64)).to(self.device, non_blocking=True)  # noqa: E731
+        int_wpts, ts = frames.wpts_world_dev(up(attitude), up(global_pos), out, M=3)
+        cfg = self.planner.cfg
+        outside = ~((ts > cfg.T_min) & (ts < cfg.T_max)).all(dim=1)
+        ts_used = frames.clamp_durations_dev(ts, cfg.T_min, cfg.T_max)[0] if self.clamp_ts else ts
+        head = np.stack([np.asarray(init_pos)[:, :2], np.asarray(init_vel)[:, :2]], axis=1)
+        res = self.planner.warm_start_plan_dev(head, target_state, int_wpts, ts_used, map_ids, noise, generator)
         res['nn_int_wpts'], res['nn_ts'], res['nn_ts_outside_bounds'] = int_wpts, ts, outside
         return res
 

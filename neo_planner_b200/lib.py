@@ -46,7 +46,8 @@ class Result(C.Structure):
 EXPORTS = ['neo_create', 'neo_destroy', 'neo_set_config', 'neo_last_error', 'neo_device_info', 'neo_set_map_esdf',
            'neo_set_map_occupancy', 'neo_set_maps_occupancy', 'neo_set_map_points', 'neo_get_occupancy', 'neo_get_map', 'neo_query_map', 'neo_eval', 'neo_eval_dev', 'neo_optimize',
            'neo_optimize_dev', 'neo_optimize_trace', 'neo_T2tau', 'neo_get_coeffs', 'neo_sample', 'neo_last_kernel_ms', 'neo_fp64_peak',
-           'neo_launch_count', 'neo_test_exp_dev', 'neo_test_exp_host', 'neo_test_nrm2_dev', 'neo_test_ddot_dev', 'neo_test_host_pool', 'neo_astar', 'neo_astar_dev']
+           'neo_launch_count', 'neo_test_exp_dev', 'neo_test_exp_host', 'neo_test_nrm2_dev', 'neo_test_ddot_dev', 'neo_test_host_pool', 'neo_astar', 'neo_astar_dev',
+           'neo_T2tau_dev', 'neo_prepare_dev', 'neo_get_coeffs_dev', 'neo_sample_dev']
 
 _lib = None
 
@@ -90,6 +91,10 @@ def load():
         lib.neo_test_ddot_dev.argtypes = [V, I, I, V, V, V, V]
         lib.neo_astar.argtypes = [V, I, V, V, V, I, I, V, V, V, V, V]
         lib.neo_astar_dev.argtypes = [V, I, V, V, V, I, I, V, V, V, V, V, V]
+        lib.neo_T2tau_dev.argtypes = [V, I, V, V, V, V]
+        lib.neo_prepare_dev.argtypes = [V, I, I, V, V, V, V, V, I, V, V, V, V, V, V, V]
+        lib.neo_get_coeffs_dev.argtypes = [V, I, I, V, V, V, V, V, V]
+        lib.neo_sample_dev.argtypes = [V, I, I, V, V, D, I, V, V, V]
         _lib = lib
     return _lib
 
@@ -282,6 +287,127 @@ class Handle:
         mx = max(int(count.max()), 1)
         states = np.zeros((B, mx, 3, 2))
         self._ck(self.lib.neo_sample(self.h, B, M, ptr(coeffs), ptr(ts), float(hz), mx, ptr(states), ptr(count)))
+        return states, count
+
+    # ---- device tensors ----------------------------------------------------------------------------------
+    # The _dev methods take and return torch CUDA tensors on this handle's device, enqueue their work on the current
+    # torch stream of that device and do not synchronise. They compute what the host methods above compute.
+    def _stream(self):
+        import torch
+        s = torch.cuda.current_stream(self.device).cuda_stream
+        # torch's default stream is the legacy default stream, handle 0, which the C API would read as "the handle's own
+        # stream" (a non-blocking one, unordered with torch's work); cudaStreamLegacy (1) names it instead
+        return C.c_void_p(s if s else 1)
+
+    def _dev(self, name, t, dtype, shape, optional=False):
+        """Device pointer of tensor t after checking its dtype, shape, contiguity and device (None stays None when
+        optional)."""
+        import torch
+        if t is None and optional:
+            return None
+        if not torch.is_tensor(t):
+            raise TypeError(f'{name}: expected a torch tensor, got {type(t).__name__}')
+        if t.dtype != dtype:
+            raise ValueError(f'{name}: expected dtype {dtype}, got {t.dtype}')
+        if tuple(t.shape) != tuple(shape):
+            raise ValueError(f'{name}: expected shape {tuple(shape)}, got {tuple(t.shape)}')
+        if t.device != torch.device('cuda', self.device):
+            raise ValueError(f'{name}: expected a tensor on cuda:{self.device}, got {t.device}')
+        if not t.is_contiguous():
+            raise ValueError(f'{name}: tensor must be contiguous')
+        return t.data_ptr()
+
+    def _empty(self, shape, dtype=None, zero=False):
+        import torch
+        dtype = torch.float64 if dtype is None else dtype
+        return (torch.zeros if zero else torch.empty)(shape, dtype=dtype, device=torch.device('cuda', self.device))
+
+    def T2tau_dev(self, ts):
+        """neo_T2tau_dev: T2tau of a float64 CUDA tensor (any shape) -> (tau, status int32), equal to T2tau's bits."""
+        import torch
+        p = self._dev('ts', ts, torch.float64, ts.shape)
+        tau = self._empty(ts.shape); st = self._empty(ts.shape, torch.int32)
+        self._ck(self.lib.neo_T2tau_dev(self.h, ts.numel(), p, tau.data_ptr(), st.data_ptr(), self._stream()))
+        return tau, st
+
+    def prepare_dev(self, M, head, tail, q0=None, ts0=None, init_ts=None, noise=None, map_ids=None):
+        """neo_prepare_dev: the inputs of optimize_dev, built on the device as optimize() builds them on the host.
+        head, tail (B,3,2); q0 (B,2,M-1) or None = straight line; ts0 (B,M) or None = init_ts, a HOST array (M);
+        noise (B,count,M-1,2) or None; map_ids: HOST array-like (B) or None. Returns dict(x0 (B,n), x0_status (B),
+        retry_q (B,count,2,M-1) or None, map_ids (B) int32 CUDA tensor or None)."""
+        import torch
+        B, n, K = len(head), 3 * M - 2, M - 1
+        f = torch.float64
+        ph = self._dev('head', head, f, (B, 3, 2)); pt = self._dev('tail', tail, f, (B, 3, 2))
+        pq = self._dev('q0', q0, f, (B, 2, K), optional=True); pts = self._dev('ts0', ts0, f, (B, M), optional=True)
+        count = 0 if noise is None else noise.shape[1] if noise.dim() == 4 else -1
+        pn = self._dev('noise', noise, f, (B, count, K, 2), optional=True)
+        its = None if init_ts is None else f64(init_ts, (M,))
+        ids = None if map_ids is None else np.ascontiguousarray(map_ids, dtype=np.int32).reshape(-1)
+        if ids is not None and ids.size != B:
+            raise ValueError(f'map_ids: expected {B} ids, got {ids.size}')
+        out = dict(x0=self._empty((B, n)), x0_status=self._empty(B, torch.int32),
+                   retry_q=self._empty((B, count, 2, K)) if count > 0 else None,
+                   map_ids=self._empty(B, torch.int32) if ids is not None else None)
+        self._ck(self.lib.neo_prepare_dev(self.h, B, M, ph, pt, pq, pts, ptr(its), count, pn, ptr(ids),
+                                          out['x0'].data_ptr(), out['x0_status'].data_ptr(),
+                                          None if out['retry_q'] is None else out['retry_q'].data_ptr(),
+                                          None if ids is None else out['map_ids'].data_ptr(), self._stream()))
+        return out
+
+    def alloc_result_dev(self, B, M, work=True):
+        """alloc_result's fields as CUDA tensors on this handle's device."""
+        import torch
+        n, i32 = 3 * M - 2, torch.int32
+        out = dict(x=self._empty((B, n), zero=True), ts=self._empty((B, M), zero=True),
+                   coeffs=self._empty((B, 6 * M, 2), zero=True), costs=self._empty((B, 4), zero=True))
+        for k in ('status', 'ok', 'attempt', 'nit', 'runs', 'nfev'):
+            out[k] = self._empty(B, i32, zero=True)
+        out['work'] = self._empty((B, 4), torch.int64, zero=True) if work else None
+        return out
+
+    def optimize_dev(self, M, x0, head, tail, x0_status=None, map_ids=None, retry_q=None, retry_tau=None, retry_status=0,
+                     max_attempts=1, out=None):
+        """neo_optimize_dev on CUDA tensors: x0 (B,n) in tau form, x0_status (B) int32 or None, head/tail (B,3,2),
+        map_ids (B) int32 CUDA tensor or None (a precondition: every id names a slot holding a map -- prepare_dev checks
+        them), retry_q (B,A-1,2,M-1), retry_tau (M) and the host int retry_status when max_attempts > 1. Returns the
+        result dict of alloc_result_dev (or `out`)."""
+        import torch
+        B, n, f, i32 = x0.shape[0], 3 * M - 2, torch.float64, torch.int32
+        args = [self._dev('x0', x0, f, (B, n)), self._dev('x0_status', x0_status, i32, (B,), True),
+                self._dev('head', head, f, (B, 3, 2)), self._dev('tail', tail, f, (B, 3, 2)),
+                self._dev('map_ids', map_ids, i32, (B,), True),
+                self._dev('retry_q', retry_q, f, (B, max_attempts - 1, 2, M - 1), True),
+                self._dev('retry_tau', retry_tau, f, (M,), True)]
+        out = self.alloc_result_dev(B, M) if out is None else out
+        r = Result()
+        shapes = dict(x=(B, n), ts=(B, M), coeffs=(B, 6 * M, 2), costs=(B, 4), work=(B, 4))
+        for k, _ in Result._fields_:
+            dt = f if k in ('x', 'ts', 'coeffs', 'costs') else torch.int64 if k == 'work' else i32
+            setattr(r, k, self._dev(k, out.get(k), dt, shapes.get(k, (B,)), optional=k == 'work'))
+        self._ck(self.lib.neo_optimize_dev(self.h, B, M, *args, int(retry_status), int(max_attempts), C.byref(r),
+                                           self._stream()))
+        return out
+
+    def get_coeffs_dev(self, M, q, ts, head, tail):
+        """neo_get_coeffs_dev: q (B,2,M-1), ts (B,M), head/tail (B,3,2) CUDA tensors -> coeffs (B,6M,2)."""
+        import torch
+        B, f = q.shape[0], torch.float64
+        out = self._empty((B, 6 * M, 2))
+        self._ck(self.lib.neo_get_coeffs_dev(self.h, B, M, self._dev('q', q, f, (B, 2, M - 1)), self._dev('ts', ts, f, (B, M)),
+                                             self._dev('head', head, f, (B, 3, 2)), self._dev('tail', tail, f, (B, 3, 2)),
+                                             out.data_ptr(), self._stream()))
+        return out
+
+    def sample_dev(self, M, coeffs, ts, hz, max_samples):
+        """neo_sample_dev: states (B, max_samples, 3, 2) (zero past each count) and count (B) int32, the full sample
+        count even where it exceeds max_samples (those trajectories are cut at max_samples rows)."""
+        import torch
+        B, f = coeffs.shape[0], torch.float64
+        states = self._empty((B, max_samples, 3, 2), zero=True); count = self._empty(B, torch.int32)
+        self._ck(self.lib.neo_sample_dev(self.h, B, M, self._dev('coeffs', coeffs, f, (B, 6 * M, 2)),
+                                         self._dev('ts', ts, f, (B, M)), float(hz), int(max_samples), states.data_ptr(),
+                                         count.data_ptr(), self._stream()))
         return states, count
 
     # ---- geometric initializer -------------------------------------------------------------------------

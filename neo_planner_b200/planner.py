@@ -407,3 +407,66 @@ class BatchPlanner:
     def get_full_state_cmd(self, coeffs, ts, hz=300):
         """TU:181-195 for B trajectories: states (B, Nmax, 3, 2), count (B)."""
         return self.handle.sample(np.asarray(ts).shape[1], coeffs, ts, hz)
+
+    # ---- device-resident variants ------------------------------------------------------------------------------
+    # The same operations on torch CUDA tensors: inputs stay on the device, results come back as CUDA tensors on the
+    # handle's device, and the work is enqueued on the current torch stream without a host synchronisation. Results are
+    # bit-identical to the host methods given the same inputs and retry noise.
+    def _dev_states(self, s):
+        """(B, k<=3, 2) tensor or array-like -> (B, 3, 2) contiguous float64 tensor on the handle's device, zero padded."""
+        import torch
+        dev = torch.device('cuda', self.handle.device)
+        s = s.to(dev, torch.float64) if torch.is_tensor(s) else torch.from_numpy(np.asarray(s, dtype=np.float64)).to(dev, non_blocking=True)
+        if s.shape[-1] != 2:
+            raise ValueError('only planar problems (D = 2) are supported, as in the reference node (NODE:593-595)')
+        if s.shape[-2] == 3:
+            return s.contiguous()
+        out = torch.zeros(s.shape[:-2] + (3, 2), dtype=torch.float64, device=dev)
+        out[..., :min(3, s.shape[-2]), :] = s[..., :3, :]
+        return out
+
+    def plan_dev(self, head, tail, map_ids=None, noise=None, generator=None, max_attempts=5, M=None):
+        """plan on the device: straight-line guess, up to max_attempts attempts. See warm_start_plan_dev."""
+        return self.warm_start_plan_dev(head, tail, None, None, map_ids, noise, generator, max_attempts,
+                                        M=self.M if M is None else M)
+
+    def warm_start_plan_dev(self, head, tail, int_wpts, ts, map_ids=None, noise=None, generator=None, max_attempts=5,
+                            M=None):
+        """warm_start_plan on the device. head/tail (B,k,2), int_wpts (B,2,M-1) and ts (B,M) are CUDA tensors (or
+        array-likes, uploaded); int_wpts = None starts from the straight line, ts = None from the init_T durations.
+        map_ids is HOST array-like (B) (checked before anything is enqueued). Retry noise (B, max_attempts-1, M-1, 2) is
+        `noise` (a float64 CUDA tensor) or, when None, drawn on the device as N(0, 0.5) with the torch.Generator
+        `generator` (None: torch's default CUDA generator). That is not the np.random stream the host method draws
+        from: pass the same `noise` to compare the two. Returns the result dict of warm_start_plan as CUDA tensors."""
+        import torch
+        h = self.handle
+        dev = torch.device('cuda', h.device)
+        head, tail = self._dev_states(head), self._dev_states(tail)
+        B = head.shape[0]
+        if M is None:
+            M = ts.shape[1] if ts is not None else int_wpts.shape[2] + 1
+        up = lambda a: None if a is None else (a if torch.is_tensor(a) else torch.from_numpy(np.ascontiguousarray(a, dtype=np.float64)).to(dev, non_blocking=True))  # noqa: E731
+        init = guesses.init_ts(self.cfg, M)
+        count = max_attempts - 1
+        if count > 0 and noise is None:
+            noise = torch.normal(0.0, 0.5, (B, count, M - 1, 2), generator=generator, dtype=torch.float64, device=dev)
+        prep = h.prepare_dev(M, head, tail, up(int_wpts), up(ts), init, noise if count > 0 else None, map_ids)
+        rtau, rst = None, 0
+        if count > 0:
+            tau, st = h.T2tau(init)                  # host data: the host's log, as neo_optimize computes it
+            rtau, rst = torch.from_numpy(tau).to(dev, non_blocking=True), int(st.max())
+        return h.optimize_dev(M, prep['x0'], head, tail, prep['x0_status'], prep['map_ids'], prep['retry_q'], rtau, rst,
+                              max_attempts)
+
+    def get_coeffs_dev(self, int_wpts, ts, head, tail):
+        """get_coeffs (EP:261-336) on the device for B problems: int_wpts (B,2,M-1), ts (B,M) -> coeffs (B,6M,2)."""
+        return self.handle.get_coeffs_dev(ts.shape[1], int_wpts, ts, self._dev_states(head), self._dev_states(tail))
+
+    def get_full_state_cmd_dev(self, coeffs, ts, hz=300, max_samples=None):
+        """get_full_state_cmd on the device: states (B, max_samples, 3, 2), count (B) int32. max_samples defaults to
+        ceil(M T_max hz) + 1, which holds every trajectory the optimizer returns; count is the full sample count, and a
+        trajectory with more samples than max_samples is cut at max_samples rows."""
+        M = ts.shape[1]
+        if max_samples is None:
+            max_samples = math.ceil(M * self.cfg.T_max * hz) + 1
+        return self.handle.sample_dev(M, coeffs, ts, hz, max_samples)
