@@ -100,10 +100,15 @@ int neo_set_maps_occupancy(neo_handle *h, int K, const int32_t *slots, int H, in
  * then the same exact EDT + gradient as neo_set_map_occupancy. */
 int neo_set_map_points(neo_handle *h, int slot, int n_points, const float *xyz, double z_min, double z_max,
                        int H, int W, double res, double ox, double oy);
-/* The binarised (0 / 100) grid the last neo_set_map_occupancy / neo_set_map_points call on this slot used: occ (H, W). */
-int neo_get_occupancy(neo_handle *h, int slot, int8_t *occ);
-/* Read a slot back (for checks / for filling a reference ESDF object): each out array (H, W) or NULL. */
-int neo_get_map(neo_handle *h, int slot, double *esdf, double *gx, double *gy);
+/* The occupancy grid the map in this slot was built from: occ (H, W), the values neo_set_map_occupancy /
+ * neo_set_maps_occupancy received (100 = occupied, any other value free) or the 0 / 100 grid neo_set_map_points
+ * projected. A slot whose map came from neo_set_map_esdf has none (NEO_ERR_INVALID) until the next
+ * neo_set_map_occupancy / neo_set_maps_occupancy / neo_set_map_points on it. (H, W) is the size of the caller's array
+ * and must be the slot's shape, else NEO_ERR_INVALID and nothing is written. */
+int neo_get_occupancy(neo_handle *h, int slot, int H, int W, int8_t *occ);
+/* Read a slot back (for checks / for filling a reference ESDF object): each out array (H, W) or NULL; (H, W) must be the
+ * slot's shape, as for neo_get_occupancy. */
+int neo_get_map(neo_handle *h, int slot, int H, int W, double *esdf, double *gx, double *gy);
 /* ESDF.get_edt_dis / get_edt_grad (ESDF:53-82) for n points xy (n,2): idx (n,2) = row, col (-1,-1 when
  * outside), dis (n) (10000 outside), grad (n,2) = [grad_x, grad_y] ([0,0] outside). */
 int neo_query_map(neo_handle *h, int slot, int n, const double *xy, int32_t *idx, double *dis, double *grad);

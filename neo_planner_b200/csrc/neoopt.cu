@@ -417,8 +417,9 @@ cudaError_t launch_prepare(int B, int M, double T_min, double T_max, const doubl
 // ---------------------------------------------------------------------------------------------------------
 struct MapSlot {
     Cell *cells = nullptr;
-    int8_t *occ = nullptr;       // binarised grid of the last occupancy / point-cloud build
+    int8_t *occ = nullptr;       // occupancy grid of the last occupancy / point-cloud build
     size_t occ_cap = 0;
+    bool has_occ = false;        // occ holds the grid of the map now in the slot (an ESDF upload has none)
     unsigned char *blocked = nullptr;   // has_collision over the enlarged A* grid (astar_warp.cuh), rebuilt with the map
     size_t blocked_cap = 0;
     int H = 0, W = 0;
@@ -684,6 +685,7 @@ static int slot_prepare(neo_handle *h, int slot, int H, int W, double res, doubl
     if (s.cells && (size_t)s.H * s.W != (size_t)H * W) { CK(cudaFree(s.cells)); s.cells = nullptr; }
     if (!s.cells) CK(cudaMalloc(&s.cells, sizeof(Cell) * (size_t)H * W));
     s.H = H; s.W = W; s.res = res; s.ox = ox; s.oy = oy;
+    s.has_occ = false;                  // until an occupancy build of this shape completes (build_from_occ)
     return NEO_OK;
 }
 
@@ -760,6 +762,7 @@ static int build_from_occ(neo_handle *h, int slot, int H, int W, double res, cha
     if (s.occ && s.occ_cap < n) { CK(cudaFree(s.occ)); s.occ = nullptr; }
     if (!s.occ) { CK(cudaMalloc(&s.occ, n)); s.occ_cap = n; }
     CK(cudaMemcpyAsync(s.occ, d_occ, n, cudaMemcpyDeviceToDevice, h->stream));
+    s.has_occ = true;
     CK(cudaMemsetAsync(d_any, 0, sizeof(int), h->stream));
     k_edt_rows<<<(H + 7) / 8, 256, 0, h->stream>>>(d_occ, H, W, d_g, d_any);                 // one warp per row
     dim3 grid((W + 127) / 128, H);
@@ -853,31 +856,42 @@ extern "C" int neo_set_map_points(neo_handle *h, int slot, int n_points, const f
     return build_from_occ(h, slot, H, W, res, d, o);
 }
 
-extern "C" int neo_get_occupancy(neo_handle *h, int slot, int8_t *occ)
+// the caller's (H, W) must be the slot's: read-back writes exactly H * W elements into caller-sized arrays
+static int check_shape(neo_handle *h, const MapSlot &s, int H, int W, const char *who)
+{
+    if (H == s.H && W == s.W) return NEO_OK;
+    return fail(h, std::string(who) + ": the slot holds a " + std::to_string(s.H) + " x " + std::to_string(s.W) + " map, not " +
+                       std::to_string(H) + " x " + std::to_string(W));
+}
+
+extern "C" int neo_get_occupancy(neo_handle *h, int slot, int H, int W, int8_t *occ)
 {
     if (!h) return NEO_ERR_INVALID;
     std::lock_guard<std::mutex> g(h->mu);
-    if (slot < 0 || slot >= (int)h->slots.size() || !h->slots[slot].occ || !occ) return fail(h, "neo_get_occupancy: no occupancy in this slot");
-    CK(cudaSetDevice(h->device));
+    if (slot < 0 || slot >= (int)h->slots.size() || !h->slots[slot].has_occ || !occ) return fail(h, "neo_get_occupancy: no occupancy in this slot");
     const MapSlot &s = h->slots[slot];
+    int rc = check_shape(h, s, H, W, "neo_get_occupancy");
+    if (rc) return rc;
+    CK(cudaSetDevice(h->device));
     CK(cudaMemcpyAsync(occ, s.occ, (size_t)s.H * s.W, cudaMemcpyDeviceToHost, h->stream));
     CK(cudaStreamSynchronize(h->stream));
     return NEO_OK;
 }
 
-extern "C" int neo_get_map(neo_handle *h, int slot, double *esdf, double *gx, double *gy)
+extern "C" int neo_get_map(neo_handle *h, int slot, int H, int W, double *esdf, double *gx, double *gy)
 {
     if (!h) return NEO_ERR_INVALID;
     std::lock_guard<std::mutex> g(h->mu);
     if (slot < 0 || slot >= (int)h->slots.size() || !h->slots[slot].cells) return fail(h, "neo_get_map: empty slot");
-    CK(cudaSetDevice(h->device));
     const MapSlot &s = h->slots[slot];
+    int rc = check_shape(h, s, H, W, "neo_get_map");
+    if (rc) return rc;
+    CK(cudaSetDevice(h->device));
     const size_t n = (size_t)s.H * s.W;
     Layout L;
     const size_t o_e = L.add(sizeof(double) * n), o_gx = L.add(sizeof(double) * n), o_gy = L.add(sizeof(double) * n);
     char *d;
-    int rc = grow(h, h->stage, L.end, &d);
-    if (rc) return rc;
+    if ((rc = grow(h, h->stage, L.end, &d))) return rc;
     k_unpack_cells<<<(unsigned)((n + 255) / 256), 256, 0, h->stream>>>(s.cells, n, (double *)(d + o_e), (double *)(d + o_gx),
                                                                        (double *)(d + o_gy));
     h->launches++;

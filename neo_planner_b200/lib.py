@@ -70,9 +70,9 @@ def load():
         lib.neo_set_map_esdf.argtypes = [V, I, I, I, D, D, D, V, V, V]
         lib.neo_set_map_occupancy.argtypes = [V, I, I, I, D, D, D, V]
         lib.neo_set_maps_occupancy.argtypes = [V, I, V, I, I, D, V, V, V]
-        lib.neo_get_map.argtypes = [V, I, V, V, V]
+        lib.neo_get_map.argtypes = [V, I, I, I, V, V, V]
         lib.neo_set_map_points.argtypes = [V, I, I, V, D, D, I, I, D, D, D]
-        lib.neo_get_occupancy.argtypes = [V, I, V]
+        lib.neo_get_occupancy.argtypes = [V, I, I, I, V]
         lib.neo_query_map.argtypes = [V, I, I, V, V, V, V]
         lib.neo_eval.argtypes = [V, I, I, V, V, V, V, V, V, V, V, V]
         lib.neo_eval_dev.argtypes = [V, I, I, V, V, V, V, V, V, V, V, V, V]
@@ -184,13 +184,16 @@ class Handle:
         self._ck(self.lib.neo_set_map_points(self.h, slot, xyz.shape[0], ptr(xyz), z_min, z_max, H, W, res, ox, oy))
 
     def get_occupancy(self, slot, H, W):
+        """The (H, W) grid the slot's map was built from; raises NeoError if (H, W) is not the slot's shape or the map
+        came from set_map_esdf."""
         occ = np.empty((H, W), np.int8)
-        self._ck(self.lib.neo_get_occupancy(self.h, slot, ptr(occ)))
+        self._ck(self.lib.neo_get_occupancy(self.h, slot, H, W, ptr(occ)))
         return occ
 
     def get_map(self, slot, H, W):
+        """(esdf, gx, gy) of the slot, each (H, W); raises NeoError if (H, W) is not the slot's shape."""
         e = np.empty((H, W)); gx = np.empty((H, W)); gy = np.empty((H, W))
-        self._ck(self.lib.neo_get_map(self.h, slot, ptr(e), ptr(gx), ptr(gy)))
+        self._ck(self.lib.neo_get_map(self.h, slot, H, W, ptr(e), ptr(gx), ptr(gy)))
         return e, gx, gy
 
     def query_map(self, slot, xy):

@@ -197,6 +197,59 @@ def test_sample_rejects_too_small_max_samples(ctx):
     ctx.eval_unchanged()
 
 
+def test_map_read_back_checks_the_shape(ctx):
+    """neo_get_map / neo_get_occupancy write H x W elements into the caller's arrays: a shape other than the slot's is
+    rejected before anything is copied, and after an ESDF upload the slot has no occupancy grid until the next
+    occupancy build -- whether the new map is larger, smaller or of the same shape."""
+    w = make_world(0)
+    h = lib.Handle(YamlConfig(), 0, 1)
+    h.set_map_occupancy(0, w.H, w.W, w.res, w.ox, w.oy, w.occ)
+    occ_want = np.where(w.occ == 100, 100, 0).astype(np.int8)
+    n = (w.H + 1) * (w.W + 1)                         # room for every shape tried below
+    bufs = [np.full(n, 7.0) for _ in range(3)]
+    obuf = np.full(n, 7, np.int8)
+
+    def rejected(H, W, what):
+        before = h.launch_count()
+        assert h.lib.neo_get_map(h.h, 0, H, W, *map(lib.ptr, bufs)) == INVALID, ('get_map', H, W)
+        assert what in h.lib.neo_last_error(h.h), h.lib.neo_last_error(h.h)
+        assert h.lib.neo_get_occupancy(h.h, 0, H, W, lib.ptr(obuf)) == INVALID, ('get_occupancy', H, W)
+        assert h.launch_count() == before
+        assert all((b == 7.0).all() for b in bufs) and (obuf == 7).all()
+
+    for H, W in ((w.H, w.W - 1), (w.H + 1, w.W), (150, 600), (0, 0), (-1, w.W)):
+        rejected(H, W, b'300 x 300')
+        if H >= 0:
+            with pytest.raises(lib.NeoError):
+                h.get_map(0, H, W)
+            with pytest.raises(lib.NeoError):
+                h.get_occupancy(0, H, W)
+    assert np.array_equal(h.get_occupancy(0, w.H, w.W), occ_want)
+    e, gx, gy = h.get_map(0, w.H, w.W)
+    # ESDF uploads: smaller, then the same shape as the occupancy build, then larger
+    for H, W in ((9, 11), (w.H, w.W), (w.H + 20, w.W + 7)):
+        rng = np.random.default_rng(H)
+        arrays = [rng.normal(size=(H, W)) for _ in range(3)]
+        h.set_map_esdf(0, 0.1, 1.0, -2.0, *arrays)
+        before = h.launch_count()
+        for args in ((H, W), (w.H, w.W)):
+            assert h.lib.neo_get_occupancy(h.h, 0, *args, lib.ptr(obuf)) == INVALID
+            assert b'no occupancy' in h.lib.neo_last_error(h.h)
+        assert h.launch_count() == before and (obuf == 7).all()
+        with pytest.raises(lib.NeoError, match='no occupancy'):
+            h.get_occupancy(0, H, W)
+        back = h.get_map(0, H, W)
+        assert all(np.array_equal(a, b) for a, b in zip(back, arrays))
+        if (H, W) != (w.H, w.W):
+            rejected(w.H, w.W, f'{H} x {W}'.encode())
+    # the next occupancy build brings the grid back
+    h.set_map_occupancy(0, w.H, w.W, w.res, w.ox, w.oy, w.occ)
+    assert np.array_equal(h.get_occupancy(0, w.H, w.W), occ_want)
+    assert all(np.array_equal(a, b) for a, b in zip(h.get_map(0, w.H, w.W), (e, gx, gy)))
+    h.close()
+    ctx.eval_unchanged()
+
+
 def test_set_maps_occupancy_argument_checks(ctx):
     H = W = 8
     occ = np.zeros((2, H, W), np.int8)
